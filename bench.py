@@ -2,6 +2,7 @@
 """Benchmark of the outfit-scoring hot path on B200 (contract: see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--skip cir,cir3,large,fp32]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One JSON line on rank 0.  Primary metric: CP outfits/s on BASELINE.json configs[1]
@@ -19,6 +20,10 @@ collective).  The same line carries one object per remaining config, each with i
 `--impl reference` times the reference's CPU path (oracle/torch_port.py: the stock torch modules the
 reference itself is built from -- the reference is pure Python and cannot travel to the GPU box) on the host
 cores for the same metric.
+
+`--dump-outputs DIR` writes what the primary step returned in its last timed step on rank 0 (CP probabilities,
+FITB argmin, FITB distances, CIR query embeddings) as DIR/<name>.npy, so that two builds can be compared output for
+output: the inputs are seeded, identical from run to run for the same arguments.
 """
 from __future__ import annotations
 
@@ -215,6 +220,28 @@ def make_cp_inputs(batch, dev, seed):
     cand = torch.randn(batch, N_CAND, 2, DPM, device=dev, generator=g)
     cand = torch.nn.functional.normalize(cand, dim=-1).reshape(batch, N_CAND, 2 * DPM).contiguous()
     return img, txt, mask, text, cand, lengths
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, seed=0):
+    """Writes `arrays` (name -> tensor with one row per outfit) as DIR/<name>.npy, float64 where the tensor is
+    float64 and float32 otherwise.  Above DUMP_BYTES in all, every array keeps the same fixed, seeded sample of
+    rows (ascending), and their row numbers are written as rows.npy."""
+    host = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    host = {k: v.astype(np.float64 if v.dtype == np.float64 else np.float32) for k, v in host.items()}
+    n = len(next(iter(host.values())))
+    row_bytes = sum(v.nbytes // max(n, 1) for v in host.values())
+    budget = DUMP_BYTES - 4096                  # room for the .npy headers
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(seed).choice(n, keep, replace=False))
+        host = {k: v[rows] for k, v in host.items()}
+        host["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in host.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def make_model(dev, d_model=D_MODEL, precision="bf16"):
@@ -496,6 +523,8 @@ def main():
     ap.add_argument("--cpu-sample", type=int, default=512)
     ap.add_argument("--e2e-chunk", type=int, default=2048, help="outfits per device chunk of the host pipeline")
     ap.add_argument("--sweep-out", default="", help="also append the configs[4] sweep points to this .jsonl file")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write the primary step's outputs of its last timed step (rank 0) to DIR/<name>.npy")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     skip = set(x for x in args.skip.split(",") if x)
@@ -542,6 +571,10 @@ def main():
     sampler = ClockSampler(local) if rank == 0 else None
     cp_ms = timed(cp_step, args.steps, args.warmup, dist_ok, dev, sampler)
     launches_cp = (L.ofx_launch_count() - n0) * args.steps // (args.steps + args.warmup)
+    if args.dump_outputs and rank == 0:
+        pred, dists, query = state["fitb"]
+        dump_outputs(args.dump_outputs, {"cp_probs": state["probs"], "fitb_pred": pred, "fitb_dists": dists,
+                                         "cir_query": query})
     cp_value = world * B * args.steps / (cp_ms * 1e-3)
     flops_step = float(flops_alg(lengths, task="cp").sum() + flops_alg(lengths, task="fitb").sum())
     cp_tflops = flops_step * args.steps / (cp_ms * 1e-3) / 1e12     # per GPU (every rank does B outfits)
