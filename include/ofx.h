@@ -191,6 +191,44 @@ OFX_API int ofx_exact_search(const float* gallery_f32, int64_t n_rows, int32_t d
 OFX_API int ofx_topk_merge(const double* scores, const int64_t* idx, int32_t n_lists, int32_t n_query,
                    int32_t k, double* out_score, int64_t* out_idx, void* stream);
 
+/* ---- category-restricted search over a whole gallery shard: the reference ranks a CIR query only against
+ * the items of its target category (compute_recall_metrics, complementary_item_retrieval_trainer.py:192-249;
+ * demo/app.py:182-190).  Same arithmetic, ranking, exactness certificate and sharding as ofx_topk_search, but
+ * the exact top-k of each query is taken over the shard's rows of the query's category only.
+ *
+ * Packing: categories (n_rows) int32 ids in [0, n_categories), n_categories <= 65536 (empty categories are
+ * fine; a row with an id outside the range belongs to no category and is never returned).  The shard is sorted
+ * stably by category: packed row p holds gallery row perm[p], category c is packed rows
+ * [seg_off[c], seg_off[c+1]), so within a category packed order is the original order.  Outputs: packed
+ * (ofx_category_gallery_packed_bytes: the bf16 rows of ofx_gallery_pack in packed order, then scratch of the
+ * sort), perm (n_rows) int32, seg_off (n_categories + 1) int64, cat_max_half_sqnorm (n_categories) fp32 =
+ * max 0.5|g|^2 of each category, for the certificate.  The fp32 rows stay in the caller's order: the re-rank
+ * and the fallback read them through perm. */
+OFX_API size_t ofx_category_gallery_packed_bytes(int64_t n_rows, int32_t dim, int32_t n_categories);
+OFX_API int ofx_category_gallery_pack(const float* gallery, const int32_t* categories, int64_t n_rows, int32_t dim,
+                              int32_t n_categories, void* packed, int32_t* perm, int64_t* seg_off,
+                              float* cat_max_half_sqnorm, void* stream);
+/* workspace for any distribution of the n_query query categories */
+OFX_API size_t ofx_category_search_workspace_bytes(int32_t dim, int32_t n_categories, int32_t n_query, int32_t k);
+/* Exact top-k of every query over this shard's rows of category query_category[q] (n_query int32, device).
+ * Outputs as ofx_topk_search: GLOBAL ids id_offset + perm[p], ties to the lowest id, idx -1 / score -inf past
+ * the category's rows; a query whose category has no row here, or is out of range, gets padding only (and
+ * out_certified 1).  out_certified 0: run ofx_category_exact_search on those queries.  The work list is built
+ * on the device: no synchronisation, capturable in a CUDA graph. */
+OFX_API int ofx_category_search(const void* packed, const int32_t* perm, const int64_t* seg_off,
+                        const float* cat_max_half_sqnorm, int32_t n_categories, const float* gallery_f32,
+                        int64_t n_rows, int32_t dim, int64_t id_offset, const float* queries,
+                        const int32_t* query_category, int32_t n_query, int32_t k, int32_t metric,
+                        double* out_score, int64_t* out_idx, uint8_t* out_certified, void* workspace,
+                        size_t workspace_bytes, void* stream);
+/* ofx_exact_search restricted to each selected query's category segment (cost proportional to the segment);
+ * workspace: ofx_exact_search_workspace_bytes(n_rows, n_sel, k). */
+OFX_API int ofx_category_exact_search(const float* gallery_f32, const int32_t* perm, const int64_t* seg_off,
+                              int32_t n_categories, int64_t n_rows, int32_t dim, int64_t id_offset,
+                              const float* queries, const int32_t* query_category, const int32_t* sel,
+                              int32_t n_sel, int32_t k, int32_t metric, double* out_score, int64_t* out_idx,
+                              uint8_t* out_certified, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ---- per-category candidate pools (SURVEY.md N1): the retrieval evaluation of
  * complementary_item_retrieval_trainer.py:192-249 ranks every query against the pool of its target
  * category only (<= 3000 items, polyvore_complementary_item_retrieval_dataset.py:111-153) with

@@ -74,6 +74,18 @@ _SIGNATURES = {
                                    C.c_void_p, C.c_size_t, C.c_void_p]),
     "ofx_topk_merge": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                  C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ofx_category_gallery_packed_bytes": (C.c_size_t, [C.c_int64, C.c_int32, C.c_int32]),
+    "ofx_category_gallery_pack": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_int32, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    "ofx_category_search_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "ofx_category_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
+                                      C.c_int64, C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_int32,
+                                      C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                      C.c_size_t, C.c_void_p]),
+    "ofx_category_exact_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int32,
+                                            C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32,
+                                            C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                            C.c_void_p]),
     "ofx_pool_search": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                   C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ofx_loss_workspace_bytes": (C.c_size_t, [C.c_int64]),

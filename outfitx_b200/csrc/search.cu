@@ -179,6 +179,63 @@ struct SchedSearch {
         n0 = (seg_lo + sub_lo + t) * kSearchBN;
         return true;
     }
+    // query rows >= m_end and gallery rows >= n_end are not part of the unit (EpiTopK)
+    __device__ __forceinline__ int m_end(int n_query) const { return n_query; }
+    __device__ __forceinline__ long long n_end(long long n_rows) const { return n_rows; }
+};
+
+// ---------------------------------------------------------------------------------------
+// Category schedule (ofx_category_search).  The shard's rows are sorted by category, so category c
+// is the packed rows [seg_off[c], seg_off[c+1]); its queries are gathered into groups of cl
+// consecutive 128-row query blocks.  A unit = (group of category c, tile range inside c's segment),
+// read from the work list cat_plan_kernel writes on the device: {m0 = the group's first query row,
+// m_end = end of c's live query rows, n_lo, n_hi = the range's packed rows}.  Tiles start at
+// n_lo + 256 it (TMA takes any row coordinate, so segments need no padding) and the epilogue masks
+// columns >= n_hi: no row of another category is ever admitted.  CTA c runs units c, c + P, ... as
+// in SchedSearch; both CTAs of a pair take the same unit (same category, same tiles).
+// ---------------------------------------------------------------------------------------
+struct SchedCat {
+    struct Params {
+        const int4* units;    // [n_units] {m0, m_end, n_lo, n_hi}
+        const int* n_units;   // written by cat_plan_kernel
+        int cl;
+    };
+    static constexpr bool kPrefetch = false;
+    static constexpr bool kThrottle = false;
+    int m0, n0, unit, step, rank, it, n_it, total, n_lo, row_end, col_end;
+    bool first, last;
+    Params p;
+    __device__ SchedCat(const Params& pp, int cta, int n_cta) : p(pp) {
+        rank = cta % pp.cl;
+        step = n_cta / pp.cl;
+        unit = cta / pp.cl - step;
+        it = n_it = 0;
+        m0 = n0 = n_lo = row_end = col_end = 0;
+        first = last = false;
+        total = *pp.n_units;
+    }
+    __device__ bool next() {
+        if (it + 1 < n_it) {
+            ++it;
+            first = false;
+        } else {
+            unit += step;
+            if (unit >= total) return false;
+            const int4 w = p.units[unit];
+            m0 = w.x + rank * kBM;
+            row_end = w.y;
+            n_lo = w.z;
+            col_end = w.w;
+            n_it = (w.w - w.z + kSearchBN - 1) / kSearchBN;
+            it = 0;
+            first = true;
+        }
+        last = it + 1 == n_it;
+        n0 = n_lo + it * kSearchBN;
+        return true;
+    }
+    __device__ __forceinline__ int m_end(int) const { return row_end; }
+    __device__ __forceinline__ long long n_end(long long) const { return col_end; }
 };
 
 struct SearchPlan {
@@ -267,9 +324,10 @@ static __device__ __noinline__ float hist_bound(const uint32_t* __restrict__ h, 
 
 // ---------------------------------------------------------------------------------------
 // Fused top-K' epilogue.  Thread <-> accumulator row <-> query.  List slot j of thread t is
-// ls[j * 128 + t] / li[j * 128 + t] (conflict-free across a warp).
+// ls[j * 128 + t] / li[j * 128 + t] (conflict-free across a warp).  Sched = SchedSearch (flat
+// shard) or SchedCat (category segments); the unit's live query rows and gallery rows come from it.
 // ---------------------------------------------------------------------------------------
-template <int KCAP>
+template <int KCAP, class Sched = SchedSearch>
 struct EpiTopK {
     struct Params {
         long long n_rows;
@@ -293,7 +351,7 @@ struct EpiTopK {
     float gthr;       // the shared bound: thr_enc / counting bound as last read
     bool full;
 
-    __device__ void begin(const Params&, const SchedSearch&, int quarter, int lane, uint8_t* smem) {
+    __device__ void begin(const Params&, const Sched&, int quarter, int lane, uint8_t* smem) {
         const int t = quarter * 32 + lane;
         ls = reinterpret_cast<float*>(smem) + t;
         li = reinterpret_cast<int*>(smem + KCAP * 128 * 4) + t;
@@ -301,7 +359,7 @@ struct EpiTopK {
     }
 
     __device__ void end(const Params&, int) {}
-    __device__ void pre_tile(const Params&, const SchedSearch&, int, int, uint8_t*) {}
+    __device__ void pre_tile(const Params&, const Sched&, int, int, uint8_t*) {}
 
     // evict candidate = lowest score, highest index among equal scores.  Static + by-value so
     // the per-thread state stays in registers (no `this` escaping into local memory).
@@ -351,10 +409,10 @@ struct EpiTopK {
         return (i & 16) ? d1 : d0;
     }
 
-    __device__ void tile(const Params& p, const SchedSearch& s, uint32_t t_acc, int quarter,
+    __device__ void tile(const Params& p, const Sched& s, uint32_t t_acc, int quarter,
                          int lane, uint8_t*) {
         const int row = s.m0 + quarter * 32 + lane;
-        const bool live = row < p.n_query;
+        const bool live = row < s.m_end(p.n_query);
         uint32_t* const hrow = p.hist ? p.hist + static_cast<size_t>(row) * kHistBuckets : nullptr;
         float* const hp = reinterpret_cast<float*>(li + KCAP * 128);      // [2][128]: lo, inv_w of this thread's query
         if (s.first) {
@@ -378,7 +436,7 @@ struct EpiTopK {
             gthr = fmaxf(gthr, fmaxf(t, g));
             thr = fmaxf(thr, gthr);
         }
-        const long long col_lim = p.n_rows - s.n0;  // columns >= col_lim are padding
+        const long long col_lim = s.n_end(p.n_rows) - s.n0;  // columns >= col_lim are padding or another category
 #pragma unroll 1
         for (int c = 0; c < kSearchBN; c += 32) {
             uint32_t raw[32];
@@ -519,17 +577,23 @@ to_bf16_kernel(const float* __restrict__ in, int n_query, int dim, float aug, __
     *reinterpret_cast<uint2*>(out + i) = u;
 }
 
+// CAT: packed row `row` is gallery row perm[row] (category order), and the maximum of 0.5|g|^2 is kept per
+// category (max_hs_bits[n_cat]); rows whose id is outside [0, n_cat) belong to no category and count nowhere.
+template <bool CAT>
 __global__ void __launch_bounds__(256)
 gallery_pack_kernel(const float* __restrict__ g, long long n_rows, int dim,
                     __nv_bfloat16* __restrict__ out, float* __restrict__ half_sqnorm,
-                    unsigned int* __restrict__ max_hs_bits) {
+                    unsigned int* __restrict__ max_hs_bits, const int* __restrict__ perm = nullptr,
+                    const int* __restrict__ cat = nullptr, int n_cat = 0) {
     const long long row = static_cast<long long>(blockIdx.x) * 8 + (threadIdx.x >> 5);
     if (row >= n_rows) return;
     const int lane = threadIdx.x & 31;
     const int pitch = dim + kAugCols;
+    long long src = row;
+    if constexpr (CAT) src = perm[row];
     float ss = 0.f;
     for (int e = lane * 4; e < dim; e += 128) {
-        const float4 v = *reinterpret_cast<const float4*>(g + row * dim + e);
+        const float4 v = *reinterpret_cast<const float4*>(g + src * dim + e);
         ss += v.x * v.x + v.y * v.y + v.z * v.z + v.w * v.w;
         __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
         uint2 u;
@@ -540,8 +604,13 @@ gallery_pack_kernel(const float* __restrict__ g, long long n_rows, int dim,
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, o);
     if (lane == 0) {
-        half_sqnorm[row] = 0.5f * ss;
-        atomicMax(max_hs_bits, __float_as_uint(0.5f * ss));     // non-negative floats order like their bit patterns
+        if constexpr (CAT) {
+            const int c = cat[src];
+            if (static_cast<unsigned>(c) < static_cast<unsigned>(n_cat)) atomicMax(max_hs_bits + c, __float_as_uint(0.5f * ss));
+        } else {
+            half_sqnorm[row] = 0.5f * ss;
+            atomicMax(max_hs_bits, __float_as_uint(0.5f * ss));     // non-negative floats order like their bit patterns
+        }
     }
     // bias columns: -0.5|g|^2 = hi + lo in bf16, then zeros (2 x 4 bytes per lane = 64 columns)
     const float bias = -0.5f * ss;
@@ -572,6 +641,11 @@ struct MergeArgs {
     const float* max_half_sqnorm;   // max over the shard of 0.5|g|^2 (tail of the packed gallery), for the certificate
     unsigned char* certified;   // (nq) or nullptr: 1 = the returned top-k is PROVEN equal to the exhaustive fp64 result
     unsigned long long* prof;   // OFX_MERGE_PROF=1: [0..3] summed cycles of gather / sort / re-score / rank, [4] CTAs that sorted all keys
+    // category search only (merge_rerank_kernel<true>): candidate ids are packed rows
+    const int* qpos;            // (nq) query row in the category-grouped query blocks, -1 = no row of its category here
+    const int* grp;             // [groups][3] {first unit, unit stride, units} of a group of cl query blocks
+    const int* perm;            // packed row -> shard-local row (fp32 rows and returned ids)
+    const int* q_cat;           // (nq) category of each query; max_half_sqnorm is per category
 };
 
 constexpr int kMergeThreads = 256;
@@ -645,6 +719,10 @@ seed_finish_kernel(const float* __restrict__ queries, int n_query, int dim, int 
     hq[q] = r;
 }
 
+// CAT: the query's lists are those of its group's units (a.grp), not one per gallery segment; candidate ids are
+// packed rows, mapped through a.perm to read the fp32 row and to emit the id.  Within a category packed order is
+// the original order, so ranking by (score, packed row) is ranking by (score, id).
+template <bool CAT>
 __global__ void __launch_bounds__(kMergeThreads)
 merge_rerank_kernel(const MergeArgs a) {
     extern __shared__ unsigned long long keys[];
@@ -654,7 +732,25 @@ merge_rerank_kernel(const MergeArgs a) {
     __shared__ int n_ext;
     __shared__ double s_kth, s_qq;
     const int q = blockIdx.x, tid = threadIdx.x;
-    const int qb = q / kBM, r = q % kBM;
+    int qb = q / kBM, r = q % kBM, trow = q, n_seg = a.n_seg, u0 = 0, ustride = 0;
+    if constexpr (CAT) {
+        const int pos = a.qpos[q];
+        if (pos < 0) {       // no row of the query's category in this shard: padding only, trivially exact
+            for (int j = tid; j < a.k; j += kMergeThreads) {
+                a.out_score[static_cast<long long>(q) * a.k + j] = -INFINITY;
+                a.out_idx[static_cast<long long>(q) * a.k + j] = -1;
+            }
+            if (tid == 0 && a.certified) a.certified[q] = a.gallery_f32 ? 1 : 0;
+            return;
+        }
+        qb = pos / kBM; r = pos % kBM; trow = pos;
+        const int* g = a.grp + 3 * (qb / a.cl);
+        u0 = g[0]; ustride = g[1]; n_seg = g[2];
+    }
+    auto src_row = [&](long long idx) -> long long {
+        if constexpr (CAT) return a.perm[idx];
+        return idx;
+    };
     __shared__ int n_small, sel_bin;
     __shared__ unsigned int es_lo, es_hi;
     __shared__ int hist[256];
@@ -668,8 +764,10 @@ merge_rerank_kernel(const MergeArgs a) {
     for (int e = tid; e < a.n_pad; e += kMergeThreads) {
         const int seg = e / a.kcap, j = e - seg * a.kcap;
         unsigned long long key = 0ull;
-        if (seg < a.n_seg) {
-            const long long slot = ((static_cast<long long>(seg) * a.n_qgroups + qb / a.cl) * a.cl + qb % a.cl) * 128 + r;
+        if (seg < n_seg) {
+            const long long unit = CAT ? static_cast<long long>(u0) + static_cast<long long>(seg) * ustride
+                                       : static_cast<long long>(seg) * a.n_qgroups + qb / a.cl;
+            const long long slot = (unit * a.cl + qb % a.cl) * 128 + r;
             if (j < a.cand_n[slot]) {
                 const float s = a.cand_s[slot * a.kcap + j];
                 const uint32_t idx = static_cast<uint32_t>(a.cand_i[slot * a.kcap + j]);
@@ -773,7 +871,7 @@ merge_rerank_kernel(const MergeArgs a) {
     if (a.gallery_f32) {
         for (int c = warp; c < n_r; c += kMergeThreads / 32) {
             const long long idx = 0xFFFFFFFFu - static_cast<uint32_t>(sk[c] & 0xFFFFFFFFull);
-            const float* g = a.gallery_f32 + idx * a.dim;
+            const float* g = a.gallery_f32 + src_row(idx) * a.dim;
             for (int d = lane * 32; d < a.dim; d += 1024)
                 asm volatile("prefetch.global.L2 [%0];" ::"l"(g + d));
         }
@@ -781,7 +879,7 @@ merge_rerank_kernel(const MergeArgs a) {
     // exact score of one candidate (whole warp), fp64 from the fp32 rows
     auto exact_score = [&](unsigned long long key, long long idx) -> double {
         if (!a.gallery_f32) return static_cast<double>(dec_score(static_cast<uint32_t>(key >> 32)));
-        const float* g = a.gallery_f32 + idx * a.dim;
+        const float* g = a.gallery_f32 + src_row(idx) * a.dim;
         const float* qv = a.queries + static_cast<long long>(q) * a.dim;
         double acc = 0.0, nn = 0.0;
         // eight gallery elements per lane in flight (the row is a cold 4 KB read from HBM; as a rolled loop
@@ -846,7 +944,7 @@ merge_rerank_kernel(const MergeArgs a) {
             if (rank < a.k) {
                 const long long o = static_cast<long long>(q) * a.k + rank;
                 a.out_score[o] = se;
-                a.out_idx[o] = a.id_offset + id;
+                a.out_idx[o] = a.id_offset + src_row(id);
                 if (rank == a.k - 1) s_kth = se;
             }
         }
@@ -863,8 +961,10 @@ merge_rerank_kernel(const MergeArgs a) {
     //    T_in, every listed row with bf16 score >= S_k - eps is re-scored too (the extension below).
     // eps = bf16_score_error_bound(|q|, max 0.5|g|^2).  No re-rank (bf16 ranking requested): nothing is claimed.
     if (!a.gallery_f32) { if (tid == 0) a.certified[q] = 0; return; }
-    const double eps = bf16_score_error_bound(sqrt(s_qq), static_cast<double>(__ldg(a.max_half_sqnorm)), a.dim, a.metric);
-    const uint32_t thr_e = a.thr_enc ? __ldcg(a.thr_enc + q) : 0u;
+    const float* hs_max = a.max_half_sqnorm;
+    if constexpr (CAT) hs_max += a.q_cat[q];        // the category's bound (tighter than the shard's)
+    const double eps = bf16_score_error_bound(sqrt(s_qq), static_cast<double>(__ldg(hs_max)), a.dim, a.metric);
+    const uint32_t thr_e = a.thr_enc ? __ldcg(a.thr_enc + trow) : 0u;
     const bool gated = thr_e != 0u;                  // some row may have been dropped without being listed
     const double t_out = gated ? static_cast<double>(dec_score(thr_e)) : -INFINITY;
     bool ok = true;
@@ -954,16 +1054,30 @@ topk_merge_kernel(const double* __restrict__ scores, const long long* __restrict
 constexpr int kExactQ = 8;
 constexpr int kExactWarps = 8;
 
+// CAT: one selected query per blockIdx.x, and the chunks (blockIdx.y) split the query's category segment
+// [seg_off[c], seg_off[c+1]) of packed rows, read through perm, so the cost follows the segment, not the shard.
+// Listed ids are packed rows (ascending within the category like the original ids).
+struct ExactCat {
+    const int* perm;
+    const long long* seg_off;
+    const int* q_cat;
+    int n_cat;
+};
+
+template <bool CAT>
 __global__ void __launch_bounds__(kExactWarps * 32)
 exact_scan_kernel(const float* __restrict__ gallery, long long n_rows, int dim, int metric,
                   const float* __restrict__ queries, const int* __restrict__ sel, int n_sel, int k,
-                  long long rows_per_chunk, double* __restrict__ part_s, long long* __restrict__ part_i) {
+                  long long rows_per_chunk, double* __restrict__ part_s, long long* __restrict__ part_i,
+                  const ExactCat xc) {
     extern __shared__ unsigned char sm_raw[];
     float* sq = reinterpret_cast<float*>(sm_raw);                                   // [kExactQ][dim]
     double* ls = reinterpret_cast<double*>(sm_raw + sizeof(float) * kExactQ * dim);  // [warps][kExactQ][k]
     long long* li = reinterpret_cast<long long*>(ls + kExactWarps * kExactQ * k);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int q0 = blockIdx.y * kExactQ, nq = min(kExactQ, n_sel - q0);
+    // CAT: x = selected query, y = chunk of its segment (grid x takes any number of queries)
+    const int chunk = CAT ? blockIdx.y : blockIdx.x, n_chunks = CAT ? gridDim.y : gridDim.x;
+    const int q0 = CAT ? blockIdx.x : blockIdx.y * kExactQ, nq = CAT ? 1 : min(kExactQ, n_sel - q0);
     for (int e = threadIdx.x; e < nq * dim; e += blockDim.x)
         sq[e] = queries[static_cast<long long>(sel[q0 + e / dim]) * dim + e % dim];
     for (int e = threadIdx.x; e < kExactWarps * kExactQ * k; e += blockDim.x) { ls[e] = -INFINITY; li[e] = -1; }
@@ -974,13 +1088,25 @@ exact_scan_kernel(const float* __restrict__ gallery, long long n_rows, int dim, 
     int worst_p[kExactQ];
 #pragma unroll
     for (int j = 0; j < kExactQ; ++j) { worst_s[j] = -INFINITY; worst_p[j] = 0; }
-    const long long lo = blockIdx.x * rows_per_chunk, hi = min(n_rows, lo + rows_per_chunk);
+    long long lo = chunk * rows_per_chunk, hi = min(n_rows, lo + rows_per_chunk);
+    if constexpr (CAT) {
+        const int c = xc.q_cat[sel[q0]];
+        lo = hi = 0;
+        if (static_cast<unsigned>(c) < static_cast<unsigned>(xc.n_cat)) {
+            const long long s_lo = xc.seg_off[c], s_hi = xc.seg_off[c + 1];
+            const long long per = (s_hi - s_lo + n_chunks - 1) / n_chunks;
+            lo = s_lo + chunk * per;
+            hi = min(s_hi, lo + per);
+        }
+    }
     for (long long row = lo + warp; row < hi; row += kExactWarps) {
         double acc[kExactQ], nn = 0.0;
 #pragma unroll
         for (int j = 0; j < kExactQ; ++j) acc[j] = 0.0;
+        long long src = row;
+        if constexpr (CAT) src = xc.perm[row];
         for (int d = lane * 4; d < dim; d += 128) {
-            const float4 g4 = __ldcs(reinterpret_cast<const float4*>(gallery + row * dim + d));
+            const float4 g4 = __ldcs(reinterpret_cast<const float4*>(gallery + src * dim + d));
             const double g[4] = {g4.x, g4.y, g4.z, g4.w};
 #pragma unroll
             for (int u = 0; u < 4; ++u) nn = fma(g[u], g[u], nn);
@@ -1040,20 +1166,249 @@ exact_scan_kernel(const float* __restrict__ gallery, long long n_rows, int dim, 
                 rank += (s2 > se) || (s2 == se && i2 < ie);
             }
         if (rank < k) {
-            const long long o = (static_cast<long long>(blockIdx.x) * n_sel + q0 + j) * k + rank;
+            const long long o = (static_cast<long long>(chunk) * n_sel + q0 + j) * k + rank;
             part_s[o] = se;
             part_i[o] = ie;
         }
     }
 }
 
+// CAT: the listed ids are packed rows; the returned id is offset + perm[row]
+template <bool CAT>
 __global__ void add_offset_kernel(long long* idx, const int* __restrict__ sel, int n_sel, int k, long long offset,
-                                  unsigned char* certified) {
+                                  unsigned char* certified, const int* __restrict__ perm) {
     const int e = blockIdx.x * blockDim.x + threadIdx.x;
     if (e >= n_sel * k) return;
     const long long o = static_cast<long long>(sel[e / k]) * k + e % k;
-    if (idx[o] >= 0) idx[o] += offset;
+    if constexpr (CAT) {
+        if (idx[o] >= 0) idx[o] = offset + perm[idx[o]];
+    } else {
+        if (idx[o] >= 0) idx[o] += offset;
+    }
     if (certified && e % k == 0) certified[sel[e / k]] = 1;
+}
+
+// ---------------------------------------------------------------------------------------
+// Category gallery (ofx_category_gallery_pack): a stable counting sort of the shard's rows by category.
+//   cat_count_kernel            rows per category; bin n_cat collects ids outside [0, n_cat) (in no segment)
+//   cat_scan_kernel             seg_off = exclusive prefix sums of the bins (one block)
+//   cat_sort_kernel             perm: chunks of 1024 rows, each sorted in shared memory by (category, row) and
+//                               then placed in chunk order -- a chunk waits until the previous one has advanced the
+//                               per-category cursors, so the rows of a category keep their original order.  Chunks
+//                               take tickets in the order they start, so the chunk waited on is always running.
+//   gallery_pack_kernel<true>   bf16 rows in packed order + per-category maximum of 0.5|g|^2
+// ---------------------------------------------------------------------------------------
+constexpr int kMaxCategories = 65536;
+constexpr int kSortChunk = 1024;
+constexpr int kMaxCatRanges = 64;     // units per query group: merge fan-in kMaxCatRanges * kcap <= 8192
+
+__global__ void __launch_bounds__(256)
+cat_count_kernel(const int* __restrict__ cat, long long n, int n_cat, int* __restrict__ cnt) {
+    const long long i = static_cast<long long>(blockIdx.x) * 256 + threadIdx.x;
+    int c = -1;
+    if (i < n) {
+        c = cat[i];
+        if (static_cast<unsigned>(c) >= static_cast<unsigned>(n_cat)) c = n_cat;
+    }
+    // one atomic per distinct category of a warp: a dominant category would otherwise serialise on one address
+    const unsigned same = __match_any_sync(0xffffffffu, c);
+    if (c >= 0 && static_cast<int>(threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(cnt + c, __popc(same));
+}
+
+// exclusive prefix sum over the 1024 threads of a block; *total = the sum of all v
+__device__ long long block_exscan(long long v, long long* sh, long long* total) {
+    const int t = threadIdx.x;
+    sh[t] = v;
+    __syncthreads();
+    for (int o = 1; o < 1024; o <<= 1) {
+        const long long x = t >= o ? sh[t - o] : 0;
+        __syncthreads();
+        sh[t] += x;
+        __syncthreads();
+    }
+    const long long incl = sh[t];
+    *total = sh[1023];
+    __syncthreads();
+    return incl - v;
+}
+
+__global__ void __launch_bounds__(1024)
+cat_scan_kernel(const int* __restrict__ cnt, int n_bins, long long* __restrict__ seg_off) {
+    __shared__ long long sh[1024];
+    const int per = (n_bins + 1023) / 1024;
+    const int b0 = min(n_bins, static_cast<int>(threadIdx.x) * per), b1 = min(n_bins, b0 + per);
+    long long s = 0, total;
+    for (int b = b0; b < b1; ++b) s += cnt[b];
+    long long o = block_exscan(s, sh, &total);
+    for (int b = b0; b < b1; ++b) { seg_off[b] = o; o += cnt[b]; }
+}
+
+__global__ void __launch_bounds__(512)
+cat_sort_kernel(const int* __restrict__ cat, long long n, int n_cat, const long long* __restrict__ seg_off,
+                int* cursor, int* chain, int* __restrict__ perm) {
+    __shared__ uint32_t key[kSortChunk];      // category << 10 | row within the chunk
+    __shared__ int run0[kSortChunk];          // sorted position where the element's category starts
+    __shared__ int s_chunk;
+    const int t = threadIdx.x;
+    if (t == 0) s_chunk = atomicAdd(chain, 1);
+    __syncthreads();
+    const int chunk = s_chunk;
+    const long long base = static_cast<long long>(chunk) * kSortChunk;
+    for (int e = t; e < kSortChunk; e += 512) {
+        const long long i = base + e;
+        uint32_t kk = 0xFFFFFFFFu;
+        if (i < n) {
+            int c = cat[i];
+            if (static_cast<unsigned>(c) >= static_cast<unsigned>(n_cat)) c = n_cat;
+            kk = (static_cast<uint32_t>(c) << 10) | static_cast<uint32_t>(e);
+        }
+        key[e] = kk;
+    }
+    __syncthreads();
+    for (int size = 2; size <= kSortChunk; size <<= 1) {      // bitonic sort, ascending
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            const int lo = 2 * t - (t & (stride - 1)), hi = lo + stride;
+            const bool up = (lo & size) == 0;
+            const uint32_t x = key[lo], y = key[hi];
+            if ((x > y) == up) { key[lo] = y; key[hi] = x; }
+            __syncthreads();
+        }
+    }
+    for (int e = t; e < kSortChunk; e += 512) run0[e] = (e == 0 || (key[e] >> 10) != (key[e - 1] >> 10)) ? e : 0;
+    __syncthreads();
+    for (int o = 1; o < kSortChunk; o <<= 1) {      // inclusive max-scan of the run heads
+        const int a = t >= o ? run0[t - o] : 0, b = run0[t + 512 - o];
+        __syncthreads();
+        run0[t] = max(run0[t], a);
+        run0[t + 512] = max(run0[t + 512], b);
+        __syncthreads();
+    }
+    if (t == 0) {
+        while (atomicAdd(chain + 1, 0) < chunk) __nanosleep(64);
+        __threadfence();
+    }
+    __syncthreads();
+    int tail_c[2] = {-1, -1}, tail_v[2] = {0, 0};
+#pragma unroll
+    for (int j = 0; j < 2; ++j) {
+        const int e = t + 512 * j;
+        const uint32_t kk = key[e];
+        if (kk == 0xFFFFFFFFu) continue;
+        const int c = static_cast<int>(kk >> 10);
+        const int rank = __ldcg(cursor + c) + (e - run0[e]);
+        perm[seg_off[c] + rank] = static_cast<int>(base + (kk & 1023u));
+        if (e == kSortChunk - 1 || (key[e + 1] >> 10) != (kk >> 10)) { tail_c[j] = c; tail_v[j] = rank + 1; }
+    }
+    __syncthreads();          // every read of a cursor precedes its update
+#pragma unroll
+    for (int j = 0; j < 2; ++j)
+        if (tail_c[j] >= 0) __stcg(cursor + tail_c[j], tail_v[j]);
+    __threadfence();
+    __syncthreads();
+    if (t == 0) atomicExch(chain + 1, chunk + 1);
+}
+
+// ---------------------------------------------------------------------------------------
+// Category search work list (ofx_category_search), built on the device so that the entry point never
+// synchronises and can be captured in a CUDA graph:
+//   cat_query_count_kernel   queries per category
+//   cat_plan_kernel          per category: groups of cl query blocks, tile ranges, units (one block)
+//   cat_query_pack_kernel    each query's row in its category's blocks, and its bf16 copy there
+// A range holds T = max(ceil(W / CTAs), 4) tiles, W = sum over categories of groups x tiles (the whole
+// tensor-core sweep), and a segment has at most kMaxCatRanges ranges: a category with a single query group
+// still spreads over ~tiles / T CTAs, and there are at most CTAs + groups units.  A category's units are
+// ordered range-major, so the groups that sweep the same range run side by side and share its tiles in L2.
+// ---------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+cat_query_count_kernel(const int* __restrict__ q_cat, int n_query, int n_cat, int* __restrict__ qcnt) {
+    const int i = blockIdx.x * 256 + threadIdx.x;
+    if (i >= n_query) return;
+    const int c = q_cat[i];
+    if (static_cast<unsigned>(c) < static_cast<unsigned>(n_cat)) atomicAdd(qcnt + c, 1);
+}
+
+__global__ void __launch_bounds__(1024)
+cat_plan_kernel(const long long* __restrict__ seg_off, int n_cat, const int* __restrict__ qcnt, int cl, int n_cta,
+                int* __restrict__ cat_g0, int4* __restrict__ units, int* __restrict__ grp, int* __restrict__ n_units) {
+    __shared__ long long sh[1024];
+    const int per = (n_cat + 1023) / 1024;
+    const int c0 = min(n_cat, static_cast<int>(threadIdx.x) * per), c1 = min(n_cat, c0 + per);
+    auto rows = [&](int c) { return seg_off[c + 1] - seg_off[c]; };
+    auto groups = [&](int c) { return rows(c) > 0 ? (qcnt[c] + kBM * cl - 1) / (kBM * cl) : 0; };
+    auto tiles = [&](int c) { return static_cast<int>((rows(c) + kSearchBN - 1) / kSearchBN); };
+    long long w = 0, total;
+    for (int c = c0; c < c1; ++c) w += static_cast<long long>(groups(c)) * tiles(c);
+    block_exscan(w, sh, &total);
+    const long long tpr = max((total + n_cta - 1) / n_cta, 4ll);
+    auto ranges = [&](int c, int* len) {         // -> number of ranges, *len = tiles per range
+        const int t = tiles(c);
+        const int r = static_cast<int>(min(static_cast<long long>(kMaxCatRanges), max(1ll, (t + tpr - 1) / tpr)));
+        *len = (t + r - 1) / r;
+        return (t + *len - 1) / *len;
+    };
+    long long gs = 0, us = 0;
+    for (int c = c0; c < c1; ++c) {
+        const int g = groups(c);
+        int len;
+        if (g) { gs += g; us += static_cast<long long>(g) * ranges(c, &len); }
+    }
+    long long g_tot, u_tot;
+    long long gb = block_exscan(gs, sh, &g_tot);
+    long long ub = block_exscan(us, sh, &u_tot);
+    for (int c = c0; c < c1; ++c) {
+        const int g = groups(c);
+        cat_g0[c] = g ? static_cast<int>(gb) : -1;
+        if (!g) continue;
+        int len;
+        const int r = ranges(c, &len);
+        const long long s_lo = seg_off[c], s_hi = seg_off[c + 1];
+        const int m_end = static_cast<int>(gb) * cl * kBM + qcnt[c];      // the category's live query rows end here
+        for (int j = 0; j < r; ++j) {
+            const long long n_lo = s_lo + static_cast<long long>(j) * len * kSearchBN;
+            const long long n_hi = min(s_hi, n_lo + static_cast<long long>(len) * kSearchBN);
+            for (int i = 0; i < g; ++i)
+                units[ub + static_cast<long long>(j) * g + i] =
+                    make_int4(static_cast<int>(gb + i) * cl * kBM, m_end, static_cast<int>(n_lo), static_cast<int>(n_hi));
+        }
+        for (int i = 0; i < g; ++i) {
+            grp[3 * (gb + i)] = static_cast<int>(ub + i);
+            grp[3 * (gb + i) + 1] = g;
+            grp[3 * (gb + i) + 2] = r;
+        }
+        gb += g;
+        ub += static_cast<long long>(g) * r;
+    }
+    if (threadIdx.x == 0) *n_units = static_cast<int>(u_tot);
+}
+
+// one warp per query: its row in the category's blocks (-1: no row of its category here, or an id out of range)
+// and the bf16 copy with the bias selector columns (as to_bf16_kernel)
+__global__ void __launch_bounds__(256)
+cat_query_pack_kernel(const float* __restrict__ queries, const int* __restrict__ q_cat, int n_query, int dim, int n_cat,
+                      float aug, const int* __restrict__ cat_g0, int cl, int* __restrict__ qfill, int* __restrict__ qpos,
+                      __nv_bfloat16* __restrict__ out) {
+    const int q = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (q >= n_query) return;
+    int pos = -1;
+    if (lane == 0) {
+        const int c = q_cat[q];
+        if (static_cast<unsigned>(c) < static_cast<unsigned>(n_cat) && cat_g0[c] >= 0)
+            pos = cat_g0[c] * cl * kBM + atomicAdd(qfill + c, 1);
+        qpos[q] = pos;
+    }
+    pos = __shfl_sync(0xffffffffu, pos, 0);
+    if (pos < 0) return;
+    const int pitch = dim + kAugCols;
+    for (int col = lane * 4; col < pitch; col += 128) {
+        float4 v;
+        if (col < dim) v = *reinterpret_cast<const float4*>(queries + static_cast<long long>(q) * dim + col);
+        else v = col == dim ? make_float4(aug, aug, 0.f, 0.f) : make_float4(0.f, 0.f, 0.f, 0.f);
+        __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+        uint2 u;
+        u.x = *reinterpret_cast<uint32_t*>(&a);
+        u.y = *reinterpret_cast<uint32_t*>(&b);
+        *reinterpret_cast<uint2*>(out + static_cast<long long>(pos) * pitch + col) = u;
+    }
 }
 
 // ---------------------------------------------------------------------------------------
@@ -1186,6 +1541,98 @@ static int launch_search_cl(const void* q_bf16, int n_query, const void* gallery
     return launch_search<Epi, STAGES, 1>(q_bf16, n_query, gallery, n_rows, pl, ep, dim, stream);
 }
 
+// ---------------------------------------------------------------------------------------
+// category search, host side
+// ---------------------------------------------------------------------------------------
+// packed category gallery: bf16 rows in category order, then the scratch of the counting sort
+struct CatGalleryLayout {
+    size_t rows_bytes, cnt, cursor, chain, total;
+};
+static CatGalleryLayout cat_gallery_layout(long long n_rows, int dim, int n_cat) {
+    CatGalleryLayout g{};
+    g.rows_bytes = align_up(static_cast<size_t>(n_rows) * (dim + kAugCols) * 2, 256);
+    g.cnt = g.rows_bytes;                                              // [n_cat + 1] rows per bin
+    g.cursor = g.cnt + align_up(static_cast<size_t>(n_cat + 1) * 4, 256);   // [n_cat + 1] rows placed per bin
+    g.chain = g.cursor + align_up(static_cast<size_t>(n_cat + 1) * 4, 256); // chunk ticket, chunks done
+    g.total = g.chain + 256;
+    return g;
+}
+
+// Workspace of ofx_category_search, sized for the worst case over the categories of the queries: a category
+// with q queries takes ceil(q / (128 cl)) groups of cl query blocks <= q / 128 + 1, so there are at most
+// ceil(n_query / 128) + min(n_query, n_cat) groups, and at most CTAs + groups units (cat_plan_kernel).
+struct CatWs {
+    size_t q_bf16, thr, cand_n, cand_s, cand_i, qcnt, cat_g0, qpos, units, grp, n_units, total;
+    int kcap, cl, n_cta, max_units;
+    long long q_rows;
+};
+static CatWs cat_ws(int dim, int n_cat, int n_query, int k) {
+    CatWs w{};
+    w.kcap = kcap_for(k);
+    w.cl = cluster_size();
+    w.n_cta = sm_count() / w.cl;
+    const long long groups = (n_query + kBM - 1) / kBM + (n_query < n_cat ? n_query : n_cat);
+    w.q_rows = groups * w.cl * kBM;
+    w.max_units = w.n_cta + static_cast<int>(groups);
+    size_t o = 0;
+    auto take = [&](size_t bytes) { size_t at = o; o = align_up(o + bytes, 256); return at; };
+    const size_t slots = static_cast<size_t>(w.max_units) * w.cl * 128;
+    w.q_bf16 = take(static_cast<size_t>(w.q_rows) * (dim + kAugCols) * 2);
+    w.thr = take(static_cast<size_t>(w.q_rows) * 4);
+    w.cand_n = take(slots * 4);
+    w.cand_s = take(slots * w.kcap * 4);
+    w.cand_i = take(slots * w.kcap * 4);
+    w.qcnt = take(static_cast<size_t>(n_cat) * 8);      // queries per category, then queries placed per category
+    w.cat_g0 = take(static_cast<size_t>(n_cat) * 4);
+    w.qpos = take(static_cast<size_t>(n_query) * 4);
+    w.units = take(static_cast<size_t>(w.max_units) * 16);
+    w.grp = take(static_cast<size_t>(groups) * 12);
+    w.n_units = take(4);
+    w.total = o;
+    return w;
+}
+
+// pass 1 of the category search: the same tcgen05 kernel as the flat search on the category schedule (CTA pairs,
+// or single CTAs with OFX_CLUSTER=1); CTAs past the last unit leave at once
+template <int KCAP, int STAGES, int CL, bool PAIR>
+static int launch_cat(const void* q_bf16, long long q_rows, const void* gallery, long long n_rows,
+                      const SchedCat::Params& sp, int grid, const typename EpiTopK<KCAP, SchedCat>::Params& ep, int dim,
+                      cudaStream_t stream) {
+    using Epi = EpiTopK<KCAP, SchedCat>;
+    CUtensorMap tm_q, tm_g;
+    const int kdim = dim + kAugCols;
+    OFX_TRY(make_tmap_bf16(&tm_q, q_bf16, static_cast<uint64_t>(q_rows), kdim, kdim, kBM));
+    OFX_TRY(make_tmap_bf16(&tm_g, gallery, static_cast<uint64_t>(n_rows), kdim, kdim, kSearchBN / CL));
+    auto kern = tc_kernel<kSearchBN, STAGES, CL, SchedCat, Epi, PAIR>;
+    constexpr int smem = tc_smem_bytes<kSearchBN, STAGES, Epi, PAIR>();
+    static_assert(smem <= 232448, "search kernel shared memory");
+    static DeviceOnce configured;
+    if (configured.need()) OFX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    cudaLaunchConfig_t cfg{};
+    cfg.gridDim = dim3(grid);
+    cfg.blockDim = dim3(tc_threads<Epi>());
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = CL;
+    attr[0].val.clusterDim.y = 1;
+    attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    count_launch();
+    OFX_CUDA(cudaLaunchKernelEx(&cfg, kern, tm_q, tm_g, sp, ep, kdim / kBK));
+    return OFX_OK;
+}
+
+template <int KCAP, int STAGES, int kPairStages>
+static int launch_cat_cl(int cl, const void* q_bf16, long long q_rows, const void* gallery, long long n_rows,
+                         const SchedCat::Params& sp, int grid, const typename EpiTopK<KCAP, SchedCat>::Params& ep,
+                         int dim, cudaStream_t stream) {
+    if (cl == 2) return launch_cat<KCAP, kPairStages, 2, true>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
+    return launch_cat<KCAP, STAGES, 1, false>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
+}
+
 }  // namespace ofx
 
 using namespace ofx;
@@ -1208,7 +1655,7 @@ int ofx_gallery_pack(const float* gallery, int64_t n_rows, int32_t dim, void* pa
     const PackedGallery L = gallery_layout(n_rows, dim);
     uint8_t* base = static_cast<uint8_t*>(packed);
     OFX_CUDA(cudaMemsetAsync(base + L.stats, 0, 256, static_cast<cudaStream_t>(stream)));
-    gallery_pack_kernel<<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
+    gallery_pack_kernel<false><<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, static_cast<cudaStream_t>(stream)>>>(
         gallery, n_rows, dim, reinterpret_cast<__nv_bfloat16*>(base), reinterpret_cast<float*>(base + L.rows_bytes),
         reinterpret_cast<unsigned int*>(base + L.stats));
     OFX_LAUNCH_CHECK();
@@ -1359,9 +1806,9 @@ int ofx_topk_search(const void* packed, const float* gallery_f32, int64_t n_rows
     const size_t smem = static_cast<size_t>(n_pad + kMergeSmall) * 8;
     static DeviceOnce configured;
     if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(merge_rerank_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (8192 + kMergeSmall) * 8));
+        OFX_CUDA(cudaFuncSetAttribute(merge_rerank_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (8192 + kMergeSmall) * 8));
     }
-    merge_rerank_kernel<<<n_query, kMergeThreads, smem, st>>>(ma);
+    merge_rerank_kernel<false><<<n_query, kMergeThreads, smem, st>>>(ma);
     OFX_LAUNCH_CHECK();
     if (merge_prof) {     // debug only: synchronous dump
         unsigned long long h[8];
@@ -1385,18 +1832,20 @@ size_t ofx_exact_search_workspace_bytes(int64_t n_rows, int32_t n_sel, int32_t k
     return align_up(static_cast<size_t>(exact_chunks(n_rows, k)) * n_sel * k * 16, 256) + 256;
 }
 
-int ofx_exact_search(const float* gallery_f32, int64_t n_rows, int32_t dim, int64_t id_offset,
-                     const float* queries, const int32_t* sel, int32_t n_sel, int32_t k, int32_t metric,
-                     double* out_score, int64_t* out_idx, uint8_t* out_certified, void* workspace,
-                     size_t workspace_bytes, void* stream) {
-    if (k < 1 || k > kMaxK) return fail(OFX_E_SHAPE, "ofx_exact_search: k %d not in [1,%d]", k, kMaxK);
-    if (dim <= 0 || dim % 4 || dim > 4096) return fail(OFX_E_SHAPE, "ofx_exact_search: dim %d (multiple of 4, <= 4096)", dim);
-    if (n_rows < 0 || n_sel < 0) return fail(OFX_E_SHAPE, "ofx_exact_search: n_rows %lld, n_sel %d", (long long)n_rows, n_sel);
-    if (metric != OFX_METRIC_DOT && metric != OFX_METRIC_L2) return fail(OFX_E_ARG, "ofx_exact_search: metric %d", metric);
+// The exhaustive fp64 fallback of both searches.  cat: xc describes the category layout, every selected query
+// scans only its category's segment (one query per CTA row) and ids map through xc.perm.
+static int exact_search(const char* who, bool cat, const ExactCat& xc, const float* gallery_f32, int64_t n_rows,
+                        int32_t dim, int64_t id_offset, const float* queries, const int32_t* sel, int32_t n_sel,
+                        int32_t k, int32_t metric, double* out_score, int64_t* out_idx, uint8_t* out_certified,
+                        void* workspace, size_t workspace_bytes, void* stream) {
+    if (k < 1 || k > kMaxK) return fail(OFX_E_SHAPE, "%s: k %d not in [1,%d]", who, k, kMaxK);
+    if (dim <= 0 || dim % 4 || dim > 4096) return fail(OFX_E_SHAPE, "%s: dim %d (multiple of 4, <= 4096)", who, dim);
+    if (n_rows < 0 || n_sel < 0) return fail(OFX_E_SHAPE, "%s: n_rows %lld, n_sel %d", who, (long long)n_rows, n_sel);
+    if (metric != OFX_METRIC_DOT && metric != OFX_METRIC_L2) return fail(OFX_E_ARG, "%s: metric %d", who, metric);
     if (n_sel == 0) return OFX_OK;
-    if (!queries || !sel || !out_score || !out_idx || (n_rows > 0 && !gallery_f32)) return fail(OFX_E_ARG, "ofx_exact_search: null argument");
+    if (!queries || !sel || !out_score || !out_idx || (n_rows > 0 && !gallery_f32)) return fail(OFX_E_ARG, "%s: null argument", who);
     if (reinterpret_cast<uintptr_t>(gallery_f32) % 16 || reinterpret_cast<uintptr_t>(queries) % 16 || reinterpret_cast<uintptr_t>(workspace) % 256)
-        return fail(OFX_E_ARG, "ofx_exact_search: misaligned pointer");
+        return fail(OFX_E_ARG, "%s: misaligned pointer", who);
     const size_t need = ofx_exact_search_workspace_bytes(n_rows, n_sel, k);
     if (!workspace || workspace_bytes < need) return fail(OFX_E_WORKSPACE, "workspace %zu B < required %zu B", workspace_bytes, need);
     OFX_TRY(require_sm100());
@@ -1409,21 +1858,52 @@ int ofx_exact_search(const float* gallery_f32, int64_t n_rows, int32_t dim, int6
     OFX_CUDA(cudaMemsetAsync(workspace, 0xFF, n_part * 16, st));
     const long long rows_per_chunk = (n_rows + chunks - 1) / chunks;
     const size_t smem = sizeof(float) * kExactQ * dim + static_cast<size_t>(kExactWarps) * kExactQ * k * 16;
+    const int smem_max = static_cast<int>(sizeof(float) * kExactQ * 4096 + kExactWarps * kExactQ * kMaxK * 16);
     static DeviceOnce configured;
-    if (configured.need())
-        OFX_CUDA(cudaFuncSetAttribute(exact_scan_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(sizeof(float) * kExactQ * 4096 + kExactWarps * kExactQ * kMaxK * 16)));
+    if (configured.need()) {
+        OFX_CUDA(cudaFuncSetAttribute(exact_scan_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+        OFX_CUDA(cudaFuncSetAttribute(exact_scan_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_max));
+    }
     if (n_rows > 0) {
-        exact_scan_kernel<<<dim3(chunks, (n_sel + kExactQ - 1) / kExactQ), kExactWarps * 32, smem, st>>>(
-            gallery_f32, n_rows, dim, metric, queries, sel, n_sel, k, rows_per_chunk > 0 ? rows_per_chunk : 1, part_s, part_i);
+        if (cat)
+            exact_scan_kernel<true><<<dim3(n_sel, chunks), kExactWarps * 32, smem, st>>>(
+                gallery_f32, n_rows, dim, metric, queries, sel, n_sel, k, 1, part_s, part_i, xc);
+        else
+            exact_scan_kernel<false><<<dim3(chunks, (n_sel + kExactQ - 1) / kExactQ), kExactWarps * 32, smem, st>>>(
+                gallery_f32, n_rows, dim, metric, queries, sel, n_sel, k, rows_per_chunk > 0 ? rows_per_chunk : 1, part_s, part_i, xc);
         OFX_LAUNCH_CHECK();
     }
     topk_merge_kernel<<<n_sel, 128, static_cast<size_t>(chunks) * k * 16, st>>>(
         part_s, part_i, chunks, n_sel, k, out_score, reinterpret_cast<long long*>(out_idx), sel);
     OFX_LAUNCH_CHECK();
-    add_offset_kernel<<<(n_sel * k + 255) / 256, 256, 0, st>>>(reinterpret_cast<long long*>(out_idx), sel, n_sel, k, id_offset, out_certified);
+    if (cat)
+        add_offset_kernel<true><<<(n_sel * k + 255) / 256, 256, 0, st>>>(reinterpret_cast<long long*>(out_idx), sel, n_sel, k, id_offset, out_certified, xc.perm);
+    else
+        add_offset_kernel<false><<<(n_sel * k + 255) / 256, 256, 0, st>>>(reinterpret_cast<long long*>(out_idx), sel, n_sel, k, id_offset, out_certified, nullptr);
     OFX_LAUNCH_CHECK();
     return OFX_OK;
+}
+
+int ofx_exact_search(const float* gallery_f32, int64_t n_rows, int32_t dim, int64_t id_offset,
+                     const float* queries, const int32_t* sel, int32_t n_sel, int32_t k, int32_t metric,
+                     double* out_score, int64_t* out_idx, uint8_t* out_certified, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+    return exact_search("ofx_exact_search", false, ExactCat{}, gallery_f32, n_rows, dim, id_offset, queries, sel, n_sel,
+                        k, metric, out_score, out_idx, out_certified, workspace, workspace_bytes, stream);
+}
+
+int ofx_category_exact_search(const float* gallery_f32, const int32_t* perm, const int64_t* seg_off,
+                              int32_t n_categories, int64_t n_rows, int32_t dim, int64_t id_offset,
+                              const float* queries, const int32_t* query_category, const int32_t* sel, int32_t n_sel,
+                              int32_t k, int32_t metric, double* out_score, int64_t* out_idx, uint8_t* out_certified,
+                              void* workspace, size_t workspace_bytes, void* stream) {
+    if (n_categories < 1 || n_categories > kMaxCategories)
+        return fail(OFX_E_SHAPE, "ofx_category_exact_search: n_categories %d not in [1,%d]", n_categories, kMaxCategories);
+    if (n_sel > 0 && (!seg_off || !query_category || (n_rows > 0 && !perm)))
+        return fail(OFX_E_ARG, "ofx_category_exact_search: null argument");
+    const ExactCat xc{perm, reinterpret_cast<const long long*>(seg_off), query_category, n_categories};
+    return exact_search("ofx_category_exact_search", true, xc, gallery_f32, n_rows, dim, id_offset, queries, sel, n_sel,
+                        k, metric, out_score, out_idx, out_certified, workspace, workspace_bytes, stream);
 }
 
 int ofx_topk_merge(const double* scores, const int64_t* idx, int32_t n_lists, int32_t n_query, int32_t k,
@@ -1437,6 +1917,136 @@ int ofx_topk_merge(const double* scores, const int64_t* idx, int32_t n_lists, in
     topk_merge_kernel<<<n_query, 128, smem, static_cast<cudaStream_t>(stream)>>>(
         scores, reinterpret_cast<const long long*>(idx), n_lists, n_query, k, out_score,
         reinterpret_cast<long long*>(out_idx));
+    OFX_LAUNCH_CHECK();
+    return OFX_OK;
+}
+
+size_t ofx_category_gallery_packed_bytes(int64_t n_rows, int32_t dim, int32_t n_categories) {
+    if (n_rows < 0 || dim <= 0 || n_categories < 1 || n_categories > kMaxCategories) return 0;
+    return cat_gallery_layout(n_rows, dim, n_categories).total;
+}
+
+int ofx_category_gallery_pack(const float* gallery, const int32_t* categories, int64_t n_rows, int32_t dim,
+                              int32_t n_categories, void* packed, int32_t* perm, int64_t* seg_off,
+                              float* cat_max_half_sqnorm, void* stream) {
+    if (n_rows < 0 || n_rows >= (1ll << 31) - 256)
+        return fail(OFX_E_SHAPE, "ofx_category_gallery_pack: n_rows %lld", (long long)n_rows);
+    if (dim <= 0 || dim % 128) return fail(OFX_E_SHAPE, "ofx_category_gallery_pack: dim %d must be a multiple of 128", dim);
+    if (n_categories < 1 || n_categories > kMaxCategories)
+        return fail(OFX_E_SHAPE, "ofx_category_gallery_pack: n_categories %d not in [1,%d]", n_categories, kMaxCategories);
+    if (!packed || !seg_off || !cat_max_half_sqnorm || (n_rows > 0 && (!gallery || !categories || !perm)))
+        return fail(OFX_E_ARG, "ofx_category_gallery_pack: null argument");
+    if (reinterpret_cast<uintptr_t>(gallery) % 16 || reinterpret_cast<uintptr_t>(packed) % 256)
+        return fail(OFX_E_ARG, "ofx_category_gallery_pack: misaligned pointer (gallery 16 B, packed 256 B)");
+    OFX_TRY(require_sm100());
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const CatGalleryLayout L = cat_gallery_layout(n_rows, dim, n_categories);
+    uint8_t* base = static_cast<uint8_t*>(packed);
+    int* cnt = reinterpret_cast<int*>(base + L.cnt);
+    OFX_CUDA(cudaMemsetAsync(base + L.cnt, 0, L.total - L.cnt, st));
+    OFX_CUDA(cudaMemsetAsync(cat_max_half_sqnorm, 0, static_cast<size_t>(n_categories) * 4, st));
+    if (n_rows > 0) {
+        cat_count_kernel<<<static_cast<unsigned>((n_rows + 255) / 256), 256, 0, st>>>(categories, n_rows, n_categories, cnt);
+        OFX_LAUNCH_CHECK();
+    }
+    cat_scan_kernel<<<1, 1024, 0, st>>>(cnt, n_categories + 1, reinterpret_cast<long long*>(seg_off));
+    OFX_LAUNCH_CHECK();
+    if (n_rows == 0) return OFX_OK;
+    cat_sort_kernel<<<static_cast<unsigned>((n_rows + kSortChunk - 1) / kSortChunk), 512, 0, st>>>(
+        categories, n_rows, n_categories, reinterpret_cast<const long long*>(seg_off), reinterpret_cast<int*>(base + L.cursor),
+        reinterpret_cast<int*>(base + L.chain), perm);
+    OFX_LAUNCH_CHECK();
+    gallery_pack_kernel<true><<<static_cast<unsigned>((n_rows + 7) / 8), 256, 0, st>>>(
+        gallery, n_rows, dim, reinterpret_cast<__nv_bfloat16*>(base), nullptr,
+        reinterpret_cast<unsigned int*>(cat_max_half_sqnorm), perm, categories, n_categories);
+    OFX_LAUNCH_CHECK();
+    return OFX_OK;
+}
+
+size_t ofx_category_search_workspace_bytes(int32_t dim, int32_t n_categories, int32_t n_query, int32_t k) {
+    if (dim <= 0 || n_query < 0 || k < 1 || k > kMaxK || n_categories < 1 || n_categories > kMaxCategories) return 0;
+    const CatWs W = cat_ws(dim, n_categories, n_query, k);
+    return W.q_rows >= (1ll << 31) ? 0 : W.total;
+}
+
+int ofx_category_search(const void* packed, const int32_t* perm, const int64_t* seg_off, const float* cat_max_half_sqnorm,
+                        int32_t n_categories, const float* gallery_f32, int64_t n_rows, int32_t dim, int64_t id_offset,
+                        const float* queries, const int32_t* query_category, int32_t n_query, int32_t k, int32_t metric,
+                        double* out_score, int64_t* out_idx, uint8_t* out_certified, void* workspace,
+                        size_t workspace_bytes, void* stream) {
+    if (k < 1 || k > kMaxK) return fail(OFX_E_SHAPE, "ofx_category_search: k %d not in [1,%d]", k, kMaxK);
+    if (dim <= 0 || dim % 128) return fail(OFX_E_SHAPE, "ofx_category_search: dim %d must be a multiple of 128", dim);
+    if (n_rows < 0 || n_rows >= (1ll << 31) - 256) return fail(OFX_E_SHAPE, "ofx_category_search: n_rows %lld", (long long)n_rows);
+    if (n_query < 0) return fail(OFX_E_SHAPE, "ofx_category_search: n_query %d", n_query);
+    if (n_categories < 1 || n_categories > kMaxCategories)
+        return fail(OFX_E_SHAPE, "ofx_category_search: n_categories %d not in [1,%d]", n_categories, kMaxCategories);
+    if (metric != OFX_METRIC_DOT && metric != OFX_METRIC_L2) return fail(OFX_E_ARG, "ofx_category_search: metric %d", metric);
+    if (n_query == 0) return OFX_OK;
+    if (!queries || !query_category || !out_score || !out_idx || !seg_off || !cat_max_half_sqnorm ||
+        (n_rows > 0 && (!packed || !perm)))
+        return fail(OFX_E_ARG, "ofx_category_search: null argument");
+    if (reinterpret_cast<uintptr_t>(queries) % 16 || reinterpret_cast<uintptr_t>(packed) % 256 ||
+        reinterpret_cast<uintptr_t>(workspace) % 256 || reinterpret_cast<uintptr_t>(gallery_f32) % 16)
+        return fail(OFX_E_ARG, "ofx_category_search: misaligned pointer");
+    OFX_TRY(require_sm100());
+    const CatWs W = cat_ws(dim, n_categories, n_query, k);
+    if (W.q_rows >= (1ll << 31)) return fail(OFX_E_SHAPE, "ofx_category_search: n_query %d too large", n_query);
+    if (!workspace || workspace_bytes < W.total)
+        return fail(OFX_E_WORKSPACE, "workspace %zu B < required %zu B", workspace_bytes, W.total);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    __nv_bfloat16* q_bf16 = reinterpret_cast<__nv_bfloat16*>(ws + W.q_bf16);
+    uint32_t* thr = reinterpret_cast<uint32_t*>(ws + W.thr);
+    int* cand_n = reinterpret_cast<int*>(ws + W.cand_n);
+    float* cand_s = reinterpret_cast<float*>(ws + W.cand_s);
+    int* cand_i = reinterpret_cast<int*>(ws + W.cand_i);
+    int* qcnt = reinterpret_cast<int*>(ws + W.qcnt);
+    int* cat_g0 = reinterpret_cast<int*>(ws + W.cat_g0);
+    int* qpos = reinterpret_cast<int*>(ws + W.qpos);
+    int4* units = reinterpret_cast<int4*>(ws + W.units);
+    int* grp = reinterpret_cast<int*>(ws + W.grp);
+    int* n_units = reinterpret_cast<int*>(ws + W.n_units);
+    const long long* seg = reinterpret_cast<const long long*>(seg_off);
+
+    OFX_CUDA(cudaMemsetAsync(qcnt, 0, static_cast<size_t>(n_categories) * 8, st));
+    OFX_CUDA(cudaMemsetAsync(thr, 0, static_cast<size_t>(W.q_rows) * 4, st));
+    cat_query_count_kernel<<<(n_query + 255) / 256, 256, 0, st>>>(query_category, n_query, n_categories, qcnt);
+    OFX_LAUNCH_CHECK();
+    cat_plan_kernel<<<1, 1024, 0, st>>>(seg, n_categories, qcnt, W.cl, W.n_cta, cat_g0, units, grp, n_units);
+    OFX_LAUNCH_CHECK();
+    cat_query_pack_kernel<<<(n_query + 7) / 8, 256, 0, st>>>(queries, query_category, n_query, dim, n_categories,
+        metric == OFX_METRIC_L2 ? 1.f : 0.f, cat_g0, W.cl, qcnt + n_categories, qpos, q_bf16);
+    OFX_LAUNCH_CHECK();
+    if (n_rows > 0) {
+        const SchedCat::Params sp{units, n_units, W.cl};
+        const int grid = W.n_cta * W.cl;
+        if (W.kcap == 32) {
+            EpiTopK<32, SchedCat>::Params ep{n_rows, n_query, thr, cand_s, cand_i, cand_n, nullptr, nullptr, nullptr, k};
+            OFX_TRY((launch_cat_cl<32, 4, 6>(W.cl, q_bf16, W.q_rows, packed, n_rows, sp, grid, ep, dim, st)));
+        } else if (W.kcap == 64) {
+            EpiTopK<64, SchedCat>::Params ep{n_rows, n_query, thr, cand_s, cand_i, cand_n, nullptr, nullptr, nullptr, k};
+            OFX_TRY((launch_cat_cl<64, 3, 5>(W.cl, q_bf16, W.q_rows, packed, n_rows, sp, grid, ep, dim, st)));
+        } else {
+            EpiTopK<128, SchedCat>::Params ep{n_rows, n_query, thr, cand_s, cand_i, cand_n, nullptr, nullptr, nullptr, k};
+            OFX_TRY((launch_cat_cl<128, 2, 3>(W.cl, q_bf16, W.q_rows, packed, n_rows, sp, grid, ep, dim, st)));
+        }
+    }
+    MergeArgs ma{};
+    ma.cand_s = cand_s; ma.cand_i = cand_i; ma.cand_n = cand_n;
+    ma.kcap = W.kcap; ma.cl = W.cl;
+    int n_pad = 2;
+    while (n_pad < kMaxCatRanges * W.kcap) n_pad <<= 1;
+    ma.n_pad = n_pad;
+    ma.queries = queries; ma.gallery_f32 = gallery_f32; ma.dim = dim; ma.metric = metric; ma.k = k;
+    ma.id_offset = id_offset; ma.out_score = out_score; ma.out_idx = reinterpret_cast<long long*>(out_idx);
+    ma.thr_enc = n_rows > 0 ? thr : nullptr;
+    ma.max_half_sqnorm = cat_max_half_sqnorm;
+    ma.certified = out_certified;
+    ma.qpos = qpos; ma.grp = grp; ma.perm = perm; ma.q_cat = query_category;
+    static DeviceOnce configured;
+    if (configured.need())
+        OFX_CUDA(cudaFuncSetAttribute(merge_rerank_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (8192 + kMergeSmall) * 8));
+    merge_rerank_kernel<true><<<n_query, kMergeThreads, static_cast<size_t>(n_pad + kMergeSmall) * 8, st>>>(ma);
     OFX_LAUNCH_CHECK();
     return OFX_OK;
 }

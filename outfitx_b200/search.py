@@ -32,40 +32,107 @@ def shard_rows(n_rows: int, rank: int, world: int) -> Tuple[int, int]:
 
 class Gallery:
     """A gallery shard resident in HBM: bf16 rows + 0.5|g|^2 for the tensor-core pass and
-    (optionally) the fp32 rows for the exact fp64 re-rank."""
+    (optionally) the fp32 rows for the exact fp64 re-rank.
+
+    A categorised gallery (``build(..., categories=...)``) is searched per category: its packed rows are
+    sorted stably by category, ``perm`` maps a packed row to the shard row, ``seg_off`` (n_categories + 1)
+    delimits each category's packed rows and ``cat_max`` holds each category's max 0.5|g|^2 (the
+    certificate's bound).  ``rows_f32`` stays in the caller's row order."""
 
     def __init__(self, packed: torch.Tensor, n_rows: int, dim: int, id_offset: int,
-                 rows_f32: Optional[torch.Tensor]):
+                 rows_f32: Optional[torch.Tensor], n_categories: Optional[int] = None,
+                 perm: Optional[torch.Tensor] = None, seg_off: Optional[torch.Tensor] = None,
+                 cat_max: Optional[torch.Tensor] = None):
         self.packed, self.n_rows, self.dim = packed, n_rows, dim
         self.id_offset, self.rows_f32 = id_offset, rows_f32
+        self.n_categories, self.perm, self.seg_off, self.cat_max = n_categories, perm, seg_off, cat_max
 
     @property
     def device(self):
         return self.packed.device
 
     @classmethod
-    def build(cls, embeddings: torch.Tensor, id_offset: int = 0, keep_fp32: bool = True) -> "Gallery":
-        """embeddings: (n_rows, dim) fp32 CUDA tensor holding THIS rank's rows."""
+    def build(cls, embeddings: torch.Tensor, id_offset: int = 0, keep_fp32: bool = True,
+              categories: Optional[torch.Tensor] = None, n_categories: Optional[int] = None) -> "Gallery":
+        """embeddings: (n_rows, dim) fp32 CUDA tensor holding THIS rank's rows.
+        categories: optional (n_rows,) integer CUDA tensor of category ids in [0, n_categories); the gallery is
+        then searched per category (``local_search(..., query_category=...)``).  n_categories defaults to
+        max id + 1; give it explicitly when shards of one catalogue are built separately, so that every shard
+        accepts the same query categories.  Checking the ids costs one small device->host sync."""
         if not embeddings.is_cuda:
             raise RuntimeError("gallery embeddings must be a CUDA tensor: outfitx_b200 has no CPU path")
         g = embeddings.detach().to(torch.float32).contiguous()
         n, dim = g.shape
         L = _lib.lib()
+        stream = torch.cuda.current_stream(g.device).cuda_stream
+        if categories is not None:
+            cat, n_cat = _gallery_categories(categories, n, g.device, n_categories)
+            nbytes = L.ofx_category_gallery_packed_bytes(n, dim, n_cat)
+            packed = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=g.device)
+            perm = torch.empty(n, dtype=torch.int32, device=g.device)
+            seg_off = torch.empty(n_cat + 1, dtype=torch.int64, device=g.device)
+            cat_max = torch.empty(n_cat, dtype=torch.float32, device=g.device)
+            with torch.cuda.device(g.device):
+                _lib.check(L.ofx_category_gallery_pack(g.data_ptr(), cat.data_ptr(), n, dim, n_cat, packed.data_ptr(),
+                                                       perm.data_ptr(), seg_off.data_ptr(), cat_max.data_ptr(), stream))
+                if not keep_fp32:
+                    torch.cuda.current_stream(g.device).synchronize()
+            return cls(packed, n, dim, id_offset, g if keep_fp32 else None, n_cat, perm, seg_off, cat_max)
+        if n_categories is not None:
+            raise ValueError("n_categories is given without categories")
         nbytes = L.ofx_gallery_packed_bytes(n, dim)
         packed = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=g.device)
         with torch.cuda.device(g.device):
-            _lib.check(L.ofx_gallery_pack(g.data_ptr(), n, dim, packed.data_ptr(),
-                                          torch.cuda.current_stream(g.device).cuda_stream))
+            _lib.check(L.ofx_gallery_pack(g.data_ptr(), n, dim, packed.data_ptr(), stream))
             if not keep_fp32:
                 torch.cuda.current_stream(g.device).synchronize()
         return cls(packed, n, dim, id_offset, g if keep_fp32 else None)
 
     @classmethod
-    def build_sharded(cls, embeddings: torch.Tensor, rank: int, world: int, keep_fp32: bool = True):
+    def build_sharded(cls, embeddings: torch.Tensor, rank: int, world: int, keep_fp32: bool = True,
+                      categories: Optional[torch.Tensor] = None, n_categories: Optional[int] = None):
         """Takes the FULL gallery (n, dim) and keeps rank's slice -- for tests / small galleries;
         large galleries should be generated or loaded shard by shard and passed to build()."""
         lo, hi = shard_rows(embeddings.shape[0], rank, world)
-        return cls.build(embeddings[lo:hi], id_offset=lo, keep_fp32=keep_fp32)
+        if categories is None:
+            return cls.build(embeddings[lo:hi], id_offset=lo, keep_fp32=keep_fp32, n_categories=n_categories)
+        if n_categories is None and categories.numel():
+            n_categories = int(categories.max()) + 1          # of the whole catalogue, the same on every rank
+        return cls.build(embeddings[lo:hi], id_offset=lo, keep_fp32=keep_fp32, categories=categories[lo:hi],
+                         n_categories=n_categories)
+
+
+MAX_CATEGORIES = 65536
+
+
+def _check_ids(ids: torch.Tensor, n: int, dev, what: str) -> None:
+    if not isinstance(ids, torch.Tensor) or not ids.is_cuda or ids.device != torch.device(dev):
+        raise ValueError(f"{what} must be a CUDA tensor on {dev}")
+    if ids.shape != (n,):
+        raise ValueError(f"{what} must have shape ({n},), got {tuple(ids.shape)}")
+    if ids.dtype.is_floating_point or ids.dtype.is_complex or ids.dtype == torch.bool:
+        raise ValueError(f"{what} must be an integer tensor, got {ids.dtype}")
+
+
+def _gallery_categories(categories, n: int, dev, n_categories: Optional[int]):
+    _check_ids(categories, n, dev, "categories")
+    if n_categories is None:
+        n_categories = int(categories.max()) + 1 if n else 1
+    if not 1 <= n_categories <= MAX_CATEGORIES:
+        raise ValueError(f"n_categories must be in [1, {MAX_CATEGORIES}], got {n_categories}")
+    if n and (int(categories.min()) < 0 or int(categories.max()) >= n_categories):
+        raise ValueError(f"categories holds an id outside [0, {n_categories})")
+    return categories.to(torch.int32).contiguous(), n_categories
+
+
+def _query_categories(query_category, nq: int, dev, n_categories: int) -> torch.Tensor:
+    _check_ids(query_category, nq, dev, "query_category")
+    # the range check reads two numbers back; inside CUDA-graph capture it is skipped (the kernels answer an
+    # out-of-range category with padding and never read outside the gallery)
+    if nq and not torch.cuda.is_current_stream_capturing():
+        if int(query_category.min()) < 0 or int(query_category.max()) >= n_categories:
+            raise ValueError(f"query_category holds an id outside [0, {n_categories})")
+    return query_category.to(torch.int32).contiguous()
 
 
 class _Workspace:
@@ -91,7 +158,7 @@ class SearchStats:
 
 @torch.no_grad()
 def local_search(queries: torch.Tensor, gallery: Gallery, k: int = 10, metric: str = "l2",
-                 exact: bool = True, return_certified: bool = False):
+                 exact: bool = True, return_certified: bool = False, query_category: Optional[torch.Tensor] = None):
     """Top-k of every query over one shard -> (idx (nq,k) int64 GLOBAL ids, score (nq,k) fp64).
 
     exact=True re-scores the tensor-core pass's candidates in fp64 from the fp32 rows and PROVES, per query,
@@ -100,7 +167,10 @@ def local_search(queries: torch.Tensor, gallery: Gallery, k: int = 10, metric: s
     re-searched exhaustively in fp64 (``ofx_exact_search``), so the indices ARE those of an fp64 exhaustive
     search.  Reading the certificate flags costs one small device->host sync per call.
     exact=False returns the bf16-pass ranking (no certificate, no sync).
-    return_certified=True appends the (nq,) bool tensor "proved by the bound alone"."""
+    return_certified=True appends the (nq,) bool tensor "proved by the bound alone".
+    query_category: (nq,) integer CUDA tensor, required for (and only for) a gallery built with categories:
+    query q is ranked against the shard's rows of category query_category[q] only
+    (``ofx_category_search``); -1 / -inf pad a list past the category's rows here."""
     if metric not in _METRIC:
         raise ValueError(f"metric must be 'dot' or 'l2', got {metric!r}")
     if not 1 <= k <= MAX_K:
@@ -112,7 +182,12 @@ def local_search(queries: torch.Tensor, gallery: Gallery, k: int = 10, metric: s
         raise ValueError(f"queries must be (nq, {gallery.dim})")
     if exact and gallery.rows_f32 is None:
         raise ValueError("exact search needs Gallery.build(..., keep_fp32=True)")
+    if gallery.n_categories is not None and query_category is None:
+        raise ValueError("a gallery built with categories is searched with query_category")
+    if gallery.n_categories is None and query_category is not None:
+        raise ValueError("query_category needs a gallery built with categories")
     nq, dev = q.shape[0], q.device
+    qc = _query_categories(query_category, nq, dev, gallery.n_categories) if query_category is not None else None
     L = _lib.lib()
     score = torch.empty(nq, k, dtype=torch.float64, device=dev)
     idx = torch.empty(nq, k, dtype=torch.int64, device=dev)
@@ -120,14 +195,24 @@ def local_search(queries: torch.Tensor, gallery: Gallery, k: int = 10, metric: s
     if nq == 0:
         return (idx, score, proved) if return_certified else (idx, score)
     cert = torch.zeros(nq, dtype=torch.uint8, device=dev) if exact else None
-    nbytes = L.ofx_search_workspace_bytes(gallery.n_rows, gallery.dim, nq, k)
-    ws = _workspace(nbytes, dev)
+    g32 = gallery.rows_f32.data_ptr() if exact else None
     with torch.cuda.device(dev):
         st = torch.cuda.current_stream(dev).cuda_stream
-        _lib.check(L.ofx_topk_search(
-            gallery.packed.data_ptr(), gallery.rows_f32.data_ptr() if exact else None,
-            gallery.n_rows, gallery.dim, gallery.id_offset, q.data_ptr(), nq, k, _METRIC[metric],
-            score.data_ptr(), idx.data_ptr(), cert.data_ptr() if exact else None, ws.data_ptr(), ws.numel(), st))
+        if qc is None:
+            nbytes = L.ofx_search_workspace_bytes(gallery.n_rows, gallery.dim, nq, k)
+            ws = _workspace(nbytes, dev)
+            _lib.check(L.ofx_topk_search(
+                gallery.packed.data_ptr(), g32, gallery.n_rows, gallery.dim, gallery.id_offset, q.data_ptr(), nq, k,
+                _METRIC[metric], score.data_ptr(), idx.data_ptr(), cert.data_ptr() if exact else None, ws.data_ptr(),
+                ws.numel(), st))
+        else:
+            nbytes = L.ofx_category_search_workspace_bytes(gallery.dim, gallery.n_categories, nq, k)
+            ws = _workspace(nbytes, dev)
+            _lib.check(L.ofx_category_search(
+                gallery.packed.data_ptr(), gallery.perm.data_ptr(), gallery.seg_off.data_ptr(),
+                gallery.cat_max.data_ptr(), gallery.n_categories, g32, gallery.n_rows, gallery.dim, gallery.id_offset,
+                q.data_ptr(), qc.data_ptr(), nq, k, _METRIC[metric], score.data_ptr(), idx.data_ptr(),
+                cert.data_ptr() if exact else None, ws.data_ptr(), ws.numel(), st))
         if exact:
             proved = cert.bool()
             sel = torch.nonzero(~proved).flatten().to(torch.int32)       # the one host sync of an exact search
@@ -136,10 +221,17 @@ def local_search(queries: torch.Tensor, gallery: Gallery, k: int = 10, metric: s
             if sel.numel():
                 nb = L.ofx_exact_search_workspace_bytes(gallery.n_rows, sel.numel(), k)
                 ws2 = torch.empty(max(nb, 256), dtype=torch.uint8, device=dev)
-                _lib.check(L.ofx_exact_search(
-                    gallery.rows_f32.data_ptr(), gallery.n_rows, gallery.dim, gallery.id_offset, q.data_ptr(),
-                    sel.data_ptr(), sel.numel(), k, _METRIC[metric], score.data_ptr(), idx.data_ptr(), None,
-                    ws2.data_ptr(), ws2.numel(), st))
+                if qc is None:
+                    _lib.check(L.ofx_exact_search(
+                        gallery.rows_f32.data_ptr(), gallery.n_rows, gallery.dim, gallery.id_offset, q.data_ptr(),
+                        sel.data_ptr(), sel.numel(), k, _METRIC[metric], score.data_ptr(), idx.data_ptr(), None,
+                        ws2.data_ptr(), ws2.numel(), st))
+                else:
+                    _lib.check(L.ofx_category_exact_search(
+                        gallery.rows_f32.data_ptr(), gallery.perm.data_ptr(), gallery.seg_off.data_ptr(),
+                        gallery.n_categories, gallery.n_rows, gallery.dim, gallery.id_offset, q.data_ptr(),
+                        qc.data_ptr(), sel.data_ptr(), sel.numel(), k, _METRIC[metric], score.data_ptr(),
+                        idx.data_ptr(), None, ws2.data_ptr(), ws2.numel(), st))
     return (idx, score, proved) if return_certified else (idx, score)
 
 
@@ -169,9 +261,12 @@ class ShardedSearch:
     def __init__(self, group=None, local=local_search, merge=merge_lists):
         self.group, self._local, self._merge = group, local, merge
 
-    def search(self, queries, gallery, k: int = 10, metric: str = "l2", exact: bool = True):
+    def search(self, queries, gallery, k: int = 10, metric: str = "l2", exact: bool = True, query_category=None):
         import torch.distributed as dist
-        idx, score = self._local(queries, gallery, k, metric, exact)
+        if query_category is None:
+            idx, score = self._local(queries, gallery, k, metric, exact)
+        else:
+            idx, score = self._local(queries, gallery, k, metric, exact, query_category=query_category)
         world = dist.get_world_size(self.group) if dist.is_initialized() else 1
         if world == 1:
             return idx, score
@@ -186,13 +281,15 @@ class ShardedSearch:
 
 
 def cir_search(queries, gallery: Gallery, k: int = 10, metric: str = "l2", exact: bool = True,
-               group=None):
+               group=None, query_category=None):
     """Top-k gallery items per query.  With an initialised process group the gallery is taken to
-    be sharded across its ranks (each rank passes its own shard and the same queries)."""
+    be sharded across its ranks (each rank passes its own shard and the same queries).  With a
+    categorised gallery, query_category (nq,) picks the category each query is ranked in -- the
+    reference's per-category retrieval (complementary_item_retrieval_trainer.py:192-249)."""
     import torch.distributed as dist
     if dist.is_available() and dist.is_initialized() and dist.get_world_size(group) > 1:
-        return ShardedSearch(group).search(queries, gallery, k, metric, exact)
-    return local_search(queries, gallery, k, metric, exact)
+        return ShardedSearch(group).search(queries, gallery, k, metric, exact, query_category=query_category)
+    return local_search(queries, gallery, k, metric, exact, query_category=query_category)
 
 
 # ---------------------------------------------------------------------------------------------
