@@ -47,7 +47,7 @@ enum {
 /* arithmetic of the hot GEMMs */
 enum {
     OFX_PREC_BF16 = 0, /* bf16 operands on tcgen05 tensor cores, fp32 accumulate (TMEM)   */
-    OFX_PREC_FP32 = 1  /* fp32 CUDA-core path: the <=1e-3-relative parity mode             */
+    OFX_PREC_FP32 = 1  /* fp32 (split-bf16 tensor-core GEMMs): the <=1e-3-relative parity mode */
 };
 
 enum { OFX_TASK_CP = 0, OFX_TASK_CIR = 1 }; /* FITB uses the CIR task (outfit_x.py:86-87) */
@@ -297,8 +297,8 @@ OFX_API int ofx_ffn_block_bf16(float* x, int32_t rows, int32_t d_model, int32_t 
 /* Same block, and in the same kernel h_next (rows, d_model) bf16 <- LayerNorm(x_new; next_ln_w,
  * next_ln_b): norm1 of the FOLLOWING encoder layer (transformer.py:944-947), computed by otherwise idle
  * warps from the rows the block has just written, so the inter-layer LayerNorm kernel disappears.
- * workspace (256-byte aligned, ofx_ffn_block_workspace_bytes): the ring through which the cooperating CTA
- * pairs exchange bf16 hidden chunks, plus their counters; contents are scratch. */
+ * workspace: at least ofx_ffn_block_workspace_bytes bytes, required by both entries (a smaller one fails with
+ * OFX_E_WORKSPACE); the kernel keeps nothing in it. */
 OFX_API int ofx_ffn_block_ln_bf16(float* x, int32_t rows, int32_t d_model, int32_t d_ffn_padded,
                           const float* ln_w, const float* ln_b, const void* w1, const float* b1,
                           const void* w2, const float* b2, void* h_next, const float* next_ln_w,

@@ -21,7 +21,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 OBJ = os.path.join(HERE, "build")
 LIB = os.path.join(HERE, "libofx.so")
-SOURCES = ["common.cu", "gemm.cu", "encoder_ops.cu", "encoder.cu", "search.cu", "ffn_block.cu", "ffn_block2.cu", "pool_search.cu", "losses.cu"]
+SOURCES = ["common.cu", "gemm.cu", "encoder_ops.cu", "encoder.cu", "search.cu", "ffn_block.cu", "pool_search.cu", "losses.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

@@ -1,7 +1,6 @@
 #include "common.h"
 
 #include <stdarg.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include <atomic>
@@ -51,18 +50,6 @@ int sm_count() {
     if (cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || n <= 0) n = 148;
     __atomic_store_n(&g_sm_count[dev], n, __ATOMIC_RELAXED);
     return n;
-}
-
-int cluster_size() {
-    static int cl = 0;
-    if (cl == 0) {
-        cl = 2;
-        if (const char* e = getenv("OFX_CLUSTER")) {
-            const int v = atoi(e);
-            if (v == 1 || v == 2) cl = v;
-        }
-    }
-    return cl;
 }
 
 typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,

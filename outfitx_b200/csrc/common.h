@@ -69,10 +69,6 @@ int make_tmap_bf16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t c
 int make_tmap_f32(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t ld,
                   uint32_t box_rows);
 
-// CTAs per MMA group in the tcgen05 GEMM / search kernels: 2 = CTA pairs (cta_group::2, default),
-// 1 = independent CTAs (OFX_CLUSTER=1, for A/B timing)
-int cluster_size();
-
 static inline size_t align_up(size_t x, size_t a) { return (x + a - 1) / a * a; }
 
 }  // namespace ofx

@@ -3,7 +3,6 @@
 // Mirrors OutfitX._cp_forward / _cir_forward (/root/reference/src/models/outfit_x.py:120-172)
 // with the exact simplifications of SURVEY.md App. A.4: padded tokens dropped, last layer
 // evaluated for the prefix-token query row only.
-#include <stdlib.h>
 
 #include "encoder_ops.h"
 #include "gemm.h"
@@ -136,7 +135,7 @@ static WsLayout make_ws(const ofx_shape* s, int batch) {
     W.q0 = take(static_cast<size_t>(batch) * dm * esz);
     W.a0 = take(static_cast<size_t>(batch) * dm * esz);
     W.u0 = take(static_cast<size_t>(batch) * fp * (s->precision == OFX_PREC_FP32 ? 6 : esz));
-    // the fused FFN block's exchange ring + counters (bf16 path, d_model 512)
+    // the fused FFN block's workspace (bf16 path, d_model 512; the kernel itself uses none of it)
     W.ffn_bytes = (s->precision == OFX_PREC_BF16 && ffn_block_supported(s->d_model, static_cast<int>(fp))) ? ffn_block_workspace_bytes() : 0;
     W.ffn = take(W.ffn_bytes);
     // fp32 precision: bf16 hi / lo pieces of the current GEMM's activation operand (3 x K bf16 per token row)
@@ -144,40 +143,6 @@ static WsLayout make_ws(const ofx_shape* s, int batch) {
     W.total = o;
     return W;
 }
-
-// OFX_FUSED_FFN=0 falls back to LN + two separate GEMMs (for A/B timing; same results within bf16 noise)
-static bool fused_ffn_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char* e = getenv("OFX_FUSED_FFN");
-        on = (e && e[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-
-// OFX_FFN_LN=0: separate LayerNorm-1 kernel between layers instead of the FFN block emitting it (A/B timing)
-static bool ffn_emits_ln() {
-    static int on = -1;
-    if (on < 0) {
-        const char* e = getenv("OFX_FFN_LN");
-        on = (e && e[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-
-// OFX_FP32_TC=0: the fp32 mode's linear layers on the CUDA cores (gemm_f32) instead of the split-bf16 tensor-core form
-static bool fp32_tc_enabled() {
-    static int on = -1;
-    if (on < 0) {
-        const char* e = getenv("OFX_FP32_TC");
-        on = (e && e[0] == '0') ? 0 : 1;
-    }
-    return on == 1;
-}
-
-template <class T> static int gemm(const GemmArgs& g, cudaStream_t st);
-template <> int gemm<float>(const GemmArgs& g, cudaStream_t st) { return gemm_f32(g, st); }
-template <> int gemm<__nv_bfloat16>(const GemmArgs& g, cudaStream_t st) { return gemm_bf16(g, st); }
 
 template <class T>
 static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_args* a, uint8_t* ws,
@@ -199,38 +164,35 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
     // linear layer: bf16 mode -> tcgen05 GEMM on the bf16 operands; fp32 mode -> the activation operand is cut into
     // bf16 hi / lo pieces and multiplied with the pre-split weights on the same tensor-core pipeline (gemm.h)
     uint8_t* split_a = ws + W.split;
-    const bool tc32 = sizeof(T) == 4 && L.s_qkv && fp32_tc_enabled();
+    constexpr bool f32 = sizeof(T) == 4;
     // a_pre: the activation operand already lies somewhere as pieces (layernorm_split3 / a piece-output GEMM wrote it);
     // piece_out: write the result as the pieces of the NEXT GEMM's operand instead of fp32
     auto mm = [&](const GemmArgs& g, const uint8_t* w_split, const void* a_pre = nullptr, void* piece_out = nullptr) -> int {
         if constexpr (sizeof(T) == 4) {
-            if (tc32) {
-                if (!a_pre) {
-                    OFX_TRY(split_bf16x3(static_cast<const float*>(g.a), g.lda, g.m, g.m_dev, g.k, split_a, kSplitA, st));
-                    a_pre = split_a;
-                }
-                GemmArgs t = g;
-                t.a = a_pre; t.lda = 3LL * g.k; t.w = w_split; t.ldw = 3LL * g.k; t.out_f32 = 1;
-                if (piece_out) { t.out = piece_out; t.ldo = 3LL * g.n; t.out_f32 = 2; }
-                return gemm_f32_split(t, st);
+            if (!a_pre) {
+                OFX_TRY(split_bf16x3(static_cast<const float*>(g.a), g.lda, g.m, g.m_dev, g.k, split_a, kSplitA, st));
+                a_pre = split_a;
             }
+            GemmArgs t = g;
+            t.a = a_pre; t.lda = 3LL * g.k; t.w = w_split; t.ldw = 3LL * g.k; t.out_f32 = 1;
+            if (piece_out) { t.out = piece_out; t.ldo = 3LL * g.n; t.out_f32 = 2; }
+            return gemm_f32_split(t, st);
+        } else {
+            (void)w_split; (void)a_pre; (void)piece_out;
+            return gemm_bf16(g, st);
         }
-        (void)w_split; (void)a_pre; (void)piece_out;
-        return gemm<T>(g, st);
     };
-    // LayerNorm in front of a linear layer: h = LN(x); in the fp32 tensor-core mode the pieces of the GEMM operand are
+    // LayerNorm in front of a linear layer: h = LN(x); in fp32 mode the pieces of the GEMM operand are
     // written straight into split_a instead (*pre = where they are)
     auto ln_mm = [&](int rows, const int* rows_dev, const float* w, const float* b, const void** pre) -> int {
         *pre = nullptr;
         if constexpr (sizeof(T) == 4) {
-            if (tc32) {
-                *pre = split_a;
-                return layernorm_split3(x, rows, rows_dev, dm, w, b, split_a, st);
-            }
+            *pre = split_a;
+            return layernorm_split3(x, rows, rows_dev, dm, w, b, split_a, st);
         }
         return layernorm<T>(x, rows, rows_dev, dm, w, b, h, st);
     };
-    const bool fused_ffn = sizeof(T) == 2 && ffn_block_supported(dm, fp) && fused_ffn_enabled();
+    const bool fused_ffn = sizeof(T) == 2 && ffn_block_supported(dm, fp);
 
     OFX_TRY(scan_valid(a->mask, B, s->max_items, off, n_tok, st));
     AssembleArgs as{};
@@ -251,7 +213,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
         const bool last = l == L.nl - 1;
         // with the fused FFN block the previous layer has already emitted h = norm1_l(x)
         const void* pre1 = nullptr;      // pieces of norm1's output, when the LayerNorm wrote them itself
-        if (l > 0 && !(fused_ffn && ffn_emits_ln()))
+        if (l > 0 && !fused_ffn)
             OFX_TRY(ln_mm(W.t_max, n_tok, lf(l, L.ln1w), lf(l, L.ln1b), &pre1));
         AttnArgs at{};
         at.batch = B; at.n_head = s->n_head; at.off = off; at.max_s = s->max_items + 1;
@@ -269,16 +231,16 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
             if (fused_ffn) {
                 FfnBlockArgs fa{x, W.t_max, n_tok, dm, fp, lf(l, L.ln2w), lf(l, L.ln2b), lw(l, L.w_1),
                                 lf(l, L.b_1), lw(l, L.w_2), lf(l, L.b_2)};
-                if (ffn_emits_ln()) { fa.h_next = h; fa.lnn_w = lf(l + 1, L.ln1w); fa.lnn_b = lf(l + 1, L.ln1b); }
+                fa.h_next = h; fa.lnn_w = lf(l + 1, L.ln1w); fa.lnn_b = lf(l + 1, L.ln1b);
                 fa.workspace = ws + W.ffn; fa.workspace_bytes = W.ffn_bytes;
                 OFX_TRY(ffn_block_bf16(fa, st));
             } else {
                 const void* pre2 = nullptr;
                 OFX_TRY(ln_mm(W.t_max, n_tok, lf(l, L.ln2w), lf(l, L.ln2b), &pre2));
                 GemmArgs g1{h, dm, lw(l, L.w_1), dm, W.t_max, n_tok, fp, dm, lf(l, L.b_1), 1, nullptr, 0, big, fp, 0};
-                OFX_TRY(mm(g1, lw(l, L.s_1), pre2, tc32 ? big : nullptr));          // fp32 tc: hidden as pieces
+                OFX_TRY(mm(g1, lw(l, L.s_1), pre2, f32 ? big : nullptr));          // fp32: hidden as pieces
                 GemmArgs g2{big, fp, lw(l, L.w_2), fp, W.t_max, n_tok, dm, fp, lf(l, L.b_2), 0, x, dm, x, dm, 1};
-                OFX_TRY(mm(g2, lw(l, L.s_2), tc32 ? big : nullptr));
+                OFX_TRY(mm(g2, lw(l, L.s_2), f32 ? big : nullptr));
             }
         } else {
             // last layer: K,V for every token, everything else for the prefix row only
@@ -288,7 +250,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
             OFX_TRY(mm(gkv, lw(l, L.s_qkv) + static_cast<size_t>(dm) * 3 * dm * 2, pre1));     // rows dm.. of the split W_qkv
             GemmArgs gq{h, dm, w_in, dm, B, nullptr, dm, dm, lf(l, L.b_qkv), 0, nullptr, 0, q0, dm, 0};
             // without pre1 (single-layer model) the K/V GEMM above has just split all of h into split_a: rows [0, B) of it
-            OFX_TRY(mm(gq, lw(l, L.s_qkv), tc32 ? static_cast<const void*>(split_a) : nullptr));
+            OFX_TRY(mm(gq, lw(l, L.s_qkv), f32 ? static_cast<const void*>(split_a) : nullptr));
             at.row0_only = 1;
             at.q = q0; at.ldq = dm; at.k = big; at.v = big + dm; at.ldk = at.ldv = 2 * dm;
             at.out = a0; at.ldo = dm;
@@ -304,9 +266,9 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
                 const void* pre2 = nullptr;
                 OFX_TRY(ln_mm(B, nullptr, lf(l, L.ln2w), lf(l, L.ln2b), &pre2));
                 GemmArgs g1{h, dm, lw(l, L.w_1), dm, B, nullptr, fp, dm, lf(l, L.b_1), 1, nullptr, 0, u0, fp, 0};
-                OFX_TRY(mm(g1, lw(l, L.s_1), pre2, tc32 ? u0 : nullptr));
+                OFX_TRY(mm(g1, lw(l, L.s_1), pre2, f32 ? u0 : nullptr));
                 GemmArgs g2{u0, fp, lw(l, L.w_2), fp, B, nullptr, dm, fp, lf(l, L.b_2), 0, x, dm, x, dm, 1};
-                OFX_TRY(mm(g2, lw(l, L.s_2), tc32 ? u0 : nullptr));
+                OFX_TRY(mm(g2, lw(l, L.s_2), f32 ? u0 : nullptr));
             }
         }
     }

@@ -11,8 +11,6 @@
 // encoding, so valid items may come from any slot.
 #include "encoder_ops.h"
 
-#include <stdlib.h>
-
 namespace ofx {
 
 template <class T> __device__ __forceinline__ float to_f(T v);
@@ -767,38 +765,23 @@ attention_mma_kernel(const AttnArgs a) {
     extern __shared__ __align__(16) uint8_t attn_sm[];
     const int b = blockIdx.x;
     const int n_items = a.off[b + 1] - a.off[b];
-    if (n_items < 8 && a.small_ok) attention_mma_body<HD, false, NSPLIT, true>(a, attn_sm);   // S = 1 + n <= 8
+    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, true>(a, attn_sm);   // S = 1 + n <= 8
     else if (n_items < 16) attention_mma_body<HD, false, NSPLIT>(a, attn_sm);         // S <= 16
     else attention_mma_body<HD, true, NSPLIT>(a, attn_sm);
 }
 
-template <int HD, int NSPLIT>
-static int launch_attention_mma_split(const AttnArgs& a, cudaStream_t stream) {
-    constexpr int smem = (3 * kAttnMaxS + 1) * (16 * HD / NSPLIT + 8) * 2;
-    static DeviceOnce configured;
-    if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, NSPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-    }
-    static int small_ok = -1;    // OFX_ATTN_SMALL=0: no S <= 8 specialisation (A/B timing)
-    if (small_ok < 0) { const char* e = getenv("OFX_ATTN_SMALL"); small_ok = (e && e[0] == '0') ? 0 : 1; }
-    AttnArgs b = a;
-    b.small_ok = small_ok;
-    attention_mma_kernel<HD, NSPLIT><<<dim3(a.batch, NSPLIT), 128, smem, stream>>>(b);
-    OFX_LAUNCH_CHECK();
-    return OFX_OK;
-}
-
+// the 16 heads of an outfit split over two CTAs
 template <int HD>
 static int launch_attention_mma(const AttnArgs& a, cudaStream_t stream) {
-    static int split = -1;   // OFX_ATTN_SPLIT = 1 | 2 | 4 (A/B timing); default 2
-    if (split < 0) {
-        const char* e = getenv("OFX_ATTN_SPLIT");
-        split = e ? atoi(e) : 2;
-        if (split != 1 && split != 2 && split != 4) split = 2;
+    constexpr int kSplit = 2;
+    constexpr int smem = (3 * kAttnMaxS + 1) * (16 * HD / kSplit + 8) * 2;
+    static DeviceOnce configured;
+    if (configured.need()) {
+        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, kSplit>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     }
-    if (split == 4) return launch_attention_mma_split<HD, 4>(a, stream);
-    if (split == 2) return launch_attention_mma_split<HD, 2>(a, stream);
-    return launch_attention_mma_split<HD, 1>(a, stream);
+    attention_mma_kernel<HD, kSplit><<<dim3(a.batch, kSplit), 128, smem, stream>>>(a);
+    OFX_LAUNCH_CHECK();
+    return OFX_OK;
 }
 
 template <class T>
@@ -806,9 +789,7 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     if (a.batch <= 0) return OFX_OK;
     if (a.n_head != 16) return fail(OFX_E_SHAPE, "attention: n_head %d != 16", a.n_head);
     if constexpr (sizeof(T) == 2) {
-        static int legacy = -1;   // OFX_ATTN_LEGACY=1: the CUDA-core kernel (A/B timing)
-        if (legacy < 0) { const char* e = getenv("OFX_ATTN_LEGACY"); legacy = (e && e[0] == '1') ? 1 : 0; }
-        if (!legacy && (a.ldq % 8 == 0) && (a.ldk % 8 == 0) && (a.ldv % 8 == 0) && (a.ldo % 8 == 0)) {
+        if ((a.ldq % 8 == 0) && (a.ldk % 8 == 0) && (a.ldv % 8 == 0) && (a.ldo % 8 == 0)) {
             switch (head_dim) {
                 case 32: return launch_attention_mma<32>(a, stream);
                 case 64: return launch_attention_mma<64>(a, stream);

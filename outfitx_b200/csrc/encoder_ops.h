@@ -32,7 +32,6 @@ struct AttnArgs {
     const void* k; long long ldk;
     const void* v; long long ldv;
     void* out; long long ldo;
-    int small_ok = 1;      // allow the S <= 8 body of the tensor-core attention kernel
 };
 
 // fused LN2 -> linear1 -> mish -> linear2 -> +residual on the fp32 residual stream (ffn_block.cu)
@@ -50,18 +49,12 @@ struct FfnBlockArgs {
     void* h_next = nullptr;        // optional (rows, dm) bf16: LayerNorm (lnn_w, lnn_b) of the updated x,
     const float* lnn_w = nullptr;  // i.e. norm1 of the next layer, emitted by the same kernel
     const float* lnn_b = nullptr;
-    void* workspace = nullptr;     // ffn_block_workspace_bytes(): hidden-chunk exchange ring + counters (v2 kernel)
+    void* workspace = nullptr;     // at least ffn_block_workspace_bytes() (unused by the kernel)
     size_t workspace_bytes = 0;
 };
-// v2 (ffn_block2.cu): four SMs per 256 rows, hidden chunks through TMEM / L2; v1 (ffn_block.cu): the round-1 kernel,
-// kept for A/B timing (OFX_FFN_V1=1) -- same arithmetic, same rounding points.
 bool ffn_block_supported(int dm, int fp);
 size_t ffn_block_workspace_bytes();
 int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream);
-bool ffn_block2_supported(int dm, int fp);
-size_t ffn_block2_workspace_bytes(int sm);
-int ffn_block2_bf16(const FfnBlockArgs& a, cudaStream_t stream);
-int ffn_block1_bf16(const FfnBlockArgs& a, cudaStream_t stream);
 
 int scan_valid(const uint8_t* mask, int batch, int max_items, int* off, int* n_tok, cudaStream_t stream);
 int fuse_rows(const float* img, const float* txt, long long rows, int dpm, int mode, int normalize,

@@ -616,32 +616,13 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
 
 bool ffn_block_supported(int dm, int fp) { return dm == ffnb::DM && fp > 0 && fp % ffnb::CH == 0; }
 
-// Which kernel: v2 (ffn_block2.cu) when OFX_FFN_V2=1, else the round-1 kernel below.  Same arithmetic and rounding
-// points.  v2 is EXPERIMENTAL: its MMA schedule needs half the shared-memory traffic per row, but as measured at the
-// end of round 2 it is slower (400 vs 345 us plain, 82 158 rows) and its LayerNorm-emitting form showed an intermittent
-// cross-cluster stall under back-to-back launches that was not root-caused -- see DESIGN.md section 4.
-static bool use_v1() {
-    static int v1 = -1;
-    if (v1 < 0) {
-        const char* e = getenv("OFX_FFN_V2");
-        const char* f = getenv("OFX_FFN_V1");
-        v1 = (e && e[0] == '1' && !(f && f[0] == '1')) ? 0 : 1;
-    }
-    return v1 == 1;
-}
-// v1 needs no scratch; v2 needs its exchange ring, counters and the staged LayerNorm rows (~115 MB on 148 SMs)
-size_t ffn_block_workspace_bytes() { return use_v1() ? 256 : ffn_block2_workspace_bytes(sm_count()); }
+// The kernel needs no scratch; the workspace the C ABI asks for (ofx_ffn_block_workspace_bytes) is a fixed 256 B.
+size_t ffn_block_workspace_bytes() { return 256; }
 
 int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream) {
-    // one contract for both kernels: the caller always provides ffn_block_workspace_bytes() of scratch
+    using namespace ffnb;
     if (a.rows > 0 && ffn_block_supported(a.dm, a.fp) && (!a.workspace || a.workspace_bytes < ffn_block_workspace_bytes()))
         return fail(OFX_E_WORKSPACE, "ffn_block workspace %zu B < required %zu B", a.workspace_bytes, ffn_block_workspace_bytes());
-    if (!use_v1() && ffn_block2_supported(a.dm, a.fp)) return ffn_block2_bf16(a, stream);
-    return ffn_block1_bf16(a, stream);
-}
-
-int ffn_block1_bf16(const FfnBlockArgs& a, cudaStream_t stream) {
-    using namespace ffnb;
     if (a.rows <= 0) return OFX_OK;
     if (a.dm != DM || a.fp <= 0 || a.fp % CH != 0)
         return fail(OFX_E_SHAPE, "ffn_block: needs d_model 512 and padded d_ffn %% 256 == 0 (got %d, %d)", a.dm, a.fp);

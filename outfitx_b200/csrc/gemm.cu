@@ -1,6 +1,6 @@
 // Linear layers of the outfit encoder: C = A . W^T (+bias) (+mish) (+fp32 residual).
 //   bf16 mode: tcgen05 / TMEM / TMA pipeline (tc_pipeline.cuh) with the fused epilogue below
-//   fp32 mode: CUDA-core tiled GEMM (the <=1e-3-relative parity mode)
+//   fp32 mode: the same pipeline on split-bf16 operands (gemm_f32_split, gemm.h)
 // Replaces the cuBLAS calls behind torch.nn.functional.linear in the reference's
 // nn.TransformerEncoderLayer (in_proj, out_proj, linear1+mish, linear2; SURVEY.md 2.1).
 #include "gemm.h"
@@ -21,12 +21,6 @@ __device__ __forceinline__ float mish_fast(float x) {
     const float n = fmaf(w, w, w + w);
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(n + 2.f));
     return x * n * r;
-}
-__device__ __forceinline__ float mish_precise(float x) {
-    float w = expf(fminf(x, 20.f));
-    float n = w * (w + 2.f);
-    float y = x * (n / (n + 2.f));
-    return x > 20.f ? x : y;
 }
 
 // -------------------------------------------------------------------------------------
@@ -365,9 +359,9 @@ static int launch_tc(const GemmArgs& g, cudaStream_t stream) {
     constexpr bool kBigEpi = Epi::kSmemBytes > 40 * 1024;   // the residual epilogue keeps 64 KB of staging tiles
     constexpr int kStages = BN >= 256 ? (CL == 2 ? (kBigEpi ? 5 : 6) : (kBigEpi ? 3 : 4))
                                       : (CL == 2 ? (kBigEpi ? 6 : 7) : (kBigEpi ? 4 : 5));
-    constexpr bool kPair = CL == 2;    // the linear layers run as CTA pairs (QKV: 116 -> 102 us at 82k tokens)
-    auto kern = tc_kernel<BN, kStages, CL, SchedGemm, Epi, kPair>;
-    constexpr int smem = tc_smem_bytes<BN, kStages, Epi, kPair>();
+    // CL = 2: the linear layers run as CTA pairs (QKV: 116 -> 102 us at 82k tokens)
+    auto kern = tc_kernel<BN, kStages, CL, SchedGemm, Epi>;
+    constexpr int smem = tc_smem_bytes<BN, kStages, Epi, CL>();
     static DeviceOnce configured;  // per instantiation
     if (configured.need()) {
         OFX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -419,8 +413,7 @@ static int launch_tc(const GemmArgs& g, cudaStream_t stream) {
 template <int BN>
 static int launch_tc_cl(const GemmArgs& g, cudaStream_t stream) {
     const long long m_tiles = (g.m + kBM - 1) / kBM;
-    int cl = cluster_size();
-    if (m_tiles < 2) cl = 1;  // a single M tile: nothing to pair
+    const int cl = m_tiles < 2 ? 1 : 2;  // CTA pairs; a single M tile: nothing to pair
     // bf16 output without residual (QKV, linear1): TMA-store epilogue; otherwise the fp32 / residual one
     const bool bf16_store = !g.out_f32 && !g.residual;
     if (bf16_store) {
@@ -428,10 +421,8 @@ static int launch_tc_cl(const GemmArgs& g, cudaStream_t stream) {
         return launch_tc<BN, 1, EpiStoreBf16<BN>>(g, stream);
     }
     // in-place fp32 residual update (out-proj, linear2): TMA load / add / TMA store epilogue
-    static int legacy = -1;   // OFX_EPI_LEGACY=1: the smem-staged coalesced-store epilogue (A/B timing)
-    if (legacy < 0) { const char* e = getenv("OFX_EPI_LEGACY"); legacy = (e && e[0] == '1') ? 1 : 0; }
     const bool inplace = g.out_f32 && g.residual == g.out && g.ldr == g.ldo && !g.act_mish && g.ldo % 4 == 0;
-    if (inplace && !legacy) {
+    if (inplace) {
         if (cl == 2) return launch_tc<BN, 2, EpiResidualTma<BN>>(g, stream);
         return launch_tc<BN, 1, EpiResidualTma<BN>>(g, stream);
     }
@@ -500,72 +491,6 @@ int gemm_f32_split(const GemmArgs& g, cudaStream_t stream) {
     GemmArgs t = g;
     t.k = 3 * g.k;
     return gemm_bf16(t, stream);
-}
-
-// -------------------------------------------------------------------------------------
-// fp32 CUDA-core path: 64x64 tile, 16-deep K slices, 4x4 outputs per thread
-// -------------------------------------------------------------------------------------
-constexpr int kFT = 64, kFK = 16;
-
-__global__ void __launch_bounds__(256)
-gemm_f32_kernel(const float* __restrict__ a, long long lda, const float* __restrict__ w,
-                long long ldw, int m, const int* __restrict__ m_dev, int n, int k,
-                const float* __restrict__ bias, int act_mish, const float* residual,
-                long long ldr, float* out, long long ldo) {
-    const int m_actual = m_dev ? min(*m_dev, m) : m;
-    const int m0 = blockIdx.y * kFT, n0 = blockIdx.x * kFT;
-    if (m0 >= m_actual) return;
-    __shared__ float sa[kFK][kFT + 4];
-    __shared__ float sw[kFK][kFT + 4];
-    const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
-    const int lr = threadIdx.x >> 2, lc = (threadIdx.x & 3) * 4;  // 64 rows x 4 float4 per slice
-    float acc[4][4] = {};
-    for (int k0 = 0; k0 < k; k0 += kFK) {
-        float4 va = make_float4(0, 0, 0, 0), vw = make_float4(0, 0, 0, 0);
-        if (m0 + lr < m_actual) va = *reinterpret_cast<const float4*>(a + (m0 + lr) * lda + k0 + lc);
-        if (n0 + lr < n) vw = *reinterpret_cast<const float4*>(w + (n0 + lr) * ldw + k0 + lc);
-        __syncthreads();
-        sa[lc][lr] = va.x; sa[lc + 1][lr] = va.y; sa[lc + 2][lr] = va.z; sa[lc + 3][lr] = va.w;
-        sw[lc][lr] = vw.x; sw[lc + 1][lr] = vw.y; sw[lc + 2][lr] = vw.z; sw[lc + 3][lr] = vw.w;
-        __syncthreads();
-#pragma unroll
-        for (int kk = 0; kk < kFK; ++kk) {
-            float ra[4], rw[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) { ra[i] = sa[kk][ty * 4 + i]; rw[i] = sw[kk][tx * 4 + i]; }
-#pragma unroll
-            for (int i = 0; i < 4; ++i)
-#pragma unroll
-                for (int j = 0; j < 4; ++j) acc[i][j] = fmaf(ra[i], rw[j], acc[i][j]);
-        }
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const int row = m0 + ty * 4 + i;
-        if (row >= m_actual) continue;
-#pragma unroll
-        for (int j = 0; j < 4; ++j) {
-            const int col = n0 + tx * 4 + j;
-            if (col >= n) continue;
-            float v = acc[i][j];
-            if (bias) v += bias[col];
-            if (act_mish) v = mish_precise(v);
-            if (residual) v += residual[row * ldr + col];
-            out[row * ldo + col] = v;
-        }
-    }
-}
-
-int gemm_f32(const GemmArgs& g, cudaStream_t stream) {
-    if (g.m <= 0) return OFX_OK;
-    if (g.k % kFK != 0 || (g.lda % 4) || (g.ldw % 4))
-        return fail(OFX_E_SHAPE, "gemm_f32: need K %% 16 == 0 and 16-byte aligned rows");
-    dim3 grid((g.n + kFT - 1) / kFT, (g.m + kFT - 1) / kFT);
-    gemm_f32_kernel<<<grid, 256, 0, stream>>>(
-        static_cast<const float*>(g.a), g.lda, static_cast<const float*>(g.w), g.ldw, g.m, g.m_dev,
-        g.n, g.k, g.bias, g.act_mish, g.residual, g.ldr, static_cast<float*>(g.out), g.ldo);
-    OFX_LAUNCH_CHECK();
-    return OFX_OK;
 }
 
 }  // namespace ofx

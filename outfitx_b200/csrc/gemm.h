@@ -22,7 +22,6 @@ struct GemmArgs {
 };
 
 int gemm_bf16(const GemmArgs& g, cudaStream_t stream);
-int gemm_f32(const GemmArgs& g, cudaStream_t stream);
 
 // fp32 operands on the tensor cores: every fp32 value v is carried as two bf16 pieces hi = bf16(v), lo = bf16(v - hi)
 // (16 mantissa bits), laid out along K as three blocks so that an ordinary bf16 GEMM with K' = 3K evaluates

@@ -103,17 +103,6 @@ __device__ __forceinline__ void tma_prefetch_l2_2d(const void* tmap, int32_t c_i
                  "r"(c_inner), "r"(c_outer)
                  : "memory");
 }
-// Multicast variant: the box lands at the same shared-memory offset in every CTA of `mask`, and
-// complete_tx is signalled on the mbarrier at the same offset in each of them.
-__device__ __forceinline__ void tma_load_2d_mc(void* smem_dst, const void* tmap, uint64_t* bar,
-                                               int32_t c_inner, int32_t c_outer, uint16_t mask) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-        " [%0], [%1, {%3, %4}], [%2], %5;"
-        ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(tmap)), "r"(smem_u32(bar)),
-        "r"(c_inner), "r"(c_outer), "h"(mask)
-        : "memory");
-}
 // Same encodings CUTLASS uses for TMA::CacheHintSm90
 constexpr uint64_t kEvictFirst = 0x12F0000000000000ull;
 constexpr uint64_t kEvictLast = 0x14F0000000000000ull;
@@ -199,13 +188,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::
                      "r"(smem_u32(bar))
                  : "memory");
-}
-// as umma_commit, but the arrive lands on the barrier at this offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-    asm volatile(
-        "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;" ::
-            "r"(smem_u32(bar)), "h"(mask)
-        : "memory");
 }
 __device__ __forceinline__ uint32_t cluster_ctarank() {
     uint32_t r;

@@ -54,27 +54,25 @@ __device__ __forceinline__ float next_up(float x) {
 // ---------------------------------------------------------------------------------------
 struct SchedSearch {
     struct Params {
-        int n_qgroups, n_tiles, seg_tiles, n_units, sub_tiles, cl;
-        int pf_dist;   // > 0: in-order sweep, query group 0 of every segment prefetches the tile pf_dist ahead into L2
+        int n_qgroups, n_tiles, seg_tiles, n_units, cl;
         int* progress; // [n_units] tile index each unit's producer has reached (-1 not started, huge = done), or null
-        int window;    // a unit may run at most `window` tiles ahead of the slowest co-scheduled unit of its segment
-        int check;     // pacing check every `check` tiles (power of two)
-        int lead;      // bit 0: the first unit of a round also prefetches (its segment's group 0 ran a round earlier);
-                       // bit 1: the last pf_dist tiles of a unit prefetch the head of the segment its CTA leads next
     };
     static constexpr bool kPrefetch = true;
     static constexpr bool kThrottle = true;
+    static constexpr int kPfDist = 8;   // query group 0 of every segment prefetches the tile kPfDist ahead into L2
+    static constexpr int kWindow = 8;   // a unit may run at most kWindow tiles ahead of the slowest co-scheduled unit of its segment
+    static constexpr int kCheck = 8;    // pacing check every kCheck tiles (power of two)
     // Pacing (producer thread only).  The query groups that sweep the same gallery segment share its tiles
     // through L2: whoever touches a tile first pulls it from HBM, the others hit.  Nothing keeps them together,
     // though, and measured at 10 M rows the main sweep read 316 GB from HBM for a 21.8 GB gallery (L2 hit rate
     // 72 %): the units drift further apart than L2 holds.  Every unit publishes the tile it has reached; every
-    // `check`-th tile a unit waits until it is at most `window` tiles ahead of the slowest unit that was launched in
+    // kCheck-th tile a unit waits until it is at most kWindow tiles ahead of the slowest unit that was launched in
     // the same round of the same segment.  The slowest unit never waits, so this cannot deadlock.
     __device__ void throttle() {
         if (!p.progress) return;
         volatile int* pr = p.progress;
         if (rank == 0) pr[unit] = last ? 0x3fffffff : it;
-        if ((it & (p.check - 1)) != 0 || it == 0 || last) return;
+        if ((it & (kCheck - 1)) != 0 || it == 0 || last) return;
         const int seg = unit / p.n_qgroups, round = unit / step;
         const int base = seg * p.n_qgroups;
         // bounded: pacing is an optimisation, never a correctness condition -- after ~20 ms of waiting the unit
@@ -110,7 +108,7 @@ struct SchedSearch {
                     if (x >= 0 && x < mn) mn = x;
                 }
             }
-            if (it - mn <= p.window) break;
+            if (it - mn <= kWindow) break;
             __nanosleep(200);
         }
     }
@@ -131,11 +129,13 @@ struct SchedSearch {
         pf_n0 = -1;
         first = last = false;
     }
-    // A unit's segment is swept as consecutive L2-sized sub-blocks of p.sub_tiles tiles.  Inside a
-    // sub-block every query block starts at a different tile and wraps around, so the CTAs that
-    // share the sub-block are spread over it instead of all missing on the same lines at once
-    // (L2 merges only a few concurrent misses per line); whoever touches a tile first pulls it
-    // from HBM, everyone else hits it in L2 whatever their relative pace.
+    // Every query group walks the segment in the same order; group 0 runs the L2 prefetch kPfDist
+    // tiles ahead, so that the other groups (and group 0 itself) hit L2 and each gallery tile
+    // crosses HBM once per segment sweep (33 GB instead of 43 GB of DRAM reads at 2 M rows against
+    // a sweep that starts every query block at a different tile, +1.5 % throughput).
+    // Prefetch leaders besides group 0 (DESIGN.md 4.2): the first unit of a round (its segment's
+    // group 0 ran a round earlier), and, in the last kPfDist tiles of a unit, the CTA that leads
+    // a segment in the next round pulls in that segment's first tiles.
     __device__ bool next() {
         if (it + 1 < seg_len) {
             ++it;
@@ -152,31 +152,17 @@ struct SchedSearch {
             first = true;
         }
         last = it + 1 == seg_len;
-        if (p.pf_dist > 0) {
-            // every query group walks the segment in the same order; group 0 runs the L2 prefetch
-            // pf_dist tiles ahead, so that the other groups (and group 0 itself) hit L2 and each
-            // gallery tile crosses HBM once per segment sweep
-            n0 = (seg_lo + it) * kSearchBN;
-            const bool lead = qg == 0 || ((p.lead & 1) && unit % step == 0);
-            pf_n0 = (lead && it + p.pf_dist < seg_len) ? (seg_lo + it + p.pf_dist) * kSearchBN : -1;
-            if ((p.lead & 2) && it + p.pf_dist >= seg_len && unit + step < p.n_units) {
-                // nothing left to pull ahead in this segment: warm the first tiles of the segment this CTA
-                // leads in the next round, so that round does not start on pf_dist cold tiles
-                const int nu = unit + step, nseg = nu / p.n_qgroups;
-                const int j = it + p.pf_dist - seg_len;
-                if ((nu - nseg * p.n_qgroups == 0 || nu % step == 0) && nseg * p.seg_tiles + j < p.n_tiles)
-                    pf_n0 = (nseg * p.seg_tiles + j) * kSearchBN;
-            }
-            return true;
+        n0 = (seg_lo + it) * kSearchBN;
+        const bool lead = qg == 0 || unit % step == 0;
+        pf_n0 = (lead && it + kPfDist < seg_len) ? (seg_lo + it + kPfDist) * kSearchBN : -1;
+        if (it + kPfDist >= seg_len && unit + step < p.n_units) {
+            // nothing left to pull ahead in this segment: warm the first tiles of the segment this CTA
+            // leads in the next round, so that round does not start on kPfDist cold tiles
+            const int nu = unit + step, nseg = nu / p.n_qgroups;
+            const int j = it + kPfDist - seg_len;
+            if ((nu - nseg * p.n_qgroups == 0 || nu % step == 0) && nseg * p.seg_tiles + j < p.n_tiles)
+                pf_n0 = (nseg * p.seg_tiles + j) * kSearchBN;
         }
-        const int sub = it / p.sub_tiles;
-        const int sub_lo = sub * p.sub_tiles;
-        const int sub_len = min(p.sub_tiles, seg_len - sub_lo);
-        const int j = it - sub_lo;
-        const int rot = (qg * 5) % sub_len;
-        int t = j + rot;
-        if (t >= sub_len) t -= sub_len;
-        n0 = (seg_lo + sub_lo + t) * kSearchBN;
         return true;
     }
     // query rows >= m_end and gallery rows >= n_end are not part of the unit (EpiTopK)
@@ -239,15 +225,14 @@ struct SchedCat {
 };
 
 struct SearchPlan {
-    int n_qblocks, n_qgroups, cl, n_tiles, n_seg, seg_tiles, n_units, grid, sub_tiles;
+    int n_qblocks, n_qgroups, cl, n_tiles, n_seg, seg_tiles, n_units, grid;
 };
 
 // Pick the segment count that minimises (rounds of units per CTA) x (tiles per unit).
 static SearchPlan make_plan(long long n_rows, int n_query, int n_sm) {
     SearchPlan pl{};
     pl.n_qblocks = (n_query + kBM - 1) / kBM;
-    pl.cl = cluster_size();
-    if (pl.n_qblocks < 2) pl.cl = 1;
+    pl.cl = pl.n_qblocks < 2 ? 1 : 2;   // CTA pairs; a single query block: nothing to pair
     pl.n_qgroups = (pl.n_qblocks + pl.cl - 1) / pl.cl;
     const int n_cta = n_sm / pl.cl;  // clusters that fit
     pl.n_tiles = static_cast<int>((n_rows + kSearchBN - 1) / kSearchBN);
@@ -266,11 +251,6 @@ static SearchPlan make_plan(long long n_rows, int n_query, int n_sm) {
     if (pl.n_tiles == 0) { pl.n_seg = 0; pl.seg_tiles = 1; }
     pl.n_units = pl.n_qgroups * pl.n_seg;
     pl.grid = (pl.n_units < n_cta ? pl.n_units : n_cta) * pl.cl;
-    // sub-blocks: keep (segments in flight) x (sub-block bytes) around 48 MB of the 126 MB L2
-    const int lanes = pl.n_qblocks > 0 ? (pl.grid + pl.n_qblocks - 1) / pl.n_qblocks : 1;  // segments in flight
-    int sub = 96 / (lanes > 0 ? lanes : 1);  // tiles of 256 rows x 1024 x bf16 = 512 KB
-    if (const char* e = getenv("OFX_SEARCH_SUB_TILES")) sub = atoi(e);
-    pl.sub_tiles = sub < 4 ? 4 : (sub > 64 ? 64 : sub);
     return pl;
 }
 
@@ -1457,7 +1437,7 @@ static SearchWs search_ws(long long n_rows, int dim, int n_query, int k) {
     return w;
 }
 
-template <class Epi, int STAGES, int CL, bool PAIR = false>
+template <class Epi, int STAGES, int CL>
 static int launch_search(const void* q_bf16, int n_query, const void* gallery, long long n_rows,
                          const SearchPlan& pl, const typename Epi::Params& ep, int dim,
                          cudaStream_t stream) {
@@ -1465,26 +1445,15 @@ static int launch_search(const void* q_bf16, int n_query, const void* gallery, l
     const int kdim = dim + kAugCols;   // contraction length including the bias k-block
     OFX_TRY(make_tmap_bf16(&tm_q, q_bf16, static_cast<uint64_t>(n_query), kdim, kdim, kBM));
     OFX_TRY(make_tmap_bf16(&tm_g, gallery, static_cast<uint64_t>(n_rows), kdim, kdim, kSearchBN / CL));
-    auto kern = tc_kernel<kSearchBN, STAGES, CL, SchedSearch, Epi, PAIR>;   // CL = 2: multicast cluster or CTA pair
-    constexpr int smem = tc_smem_bytes<kSearchBN, STAGES, Epi, PAIR>();
+    auto kern = tc_kernel<kSearchBN, STAGES, CL, SchedSearch, Epi>;   // CL = 2: CTA pair
+    constexpr int smem = tc_smem_bytes<kSearchBN, STAGES, Epi, CL>();
     static_assert(smem <= 232448, "search kernel shared memory");
     static DeviceOnce configured;
     if (configured.need()) {
         OFX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     }
-    static int pf_dist = -1;
-    // default: in-order sweep with group 0 prefetching 8 tiles ahead (33 GB instead of 43 GB of DRAM reads at
-    // 2 M rows, +1.5 % throughput); OFX_SEARCH_PREFETCH=0 selects the rotated sub-block sweep
-    if (pf_dist < 0) { const char* e = getenv("OFX_SEARCH_PREFETCH"); pf_dist = e ? atoi(e) : 8; }
-    static int window = -1;     // OFX_SEARCH_WINDOW: pacing window in tiles (0 = off)
-    if (window < 0) { const char* e = getenv("OFX_SEARCH_WINDOW"); window = e ? atoi(e) : 8; }
-    int* progress = (window > 0 && pf_dist > 0) ? ep.progress : nullptr;
-    if (progress) OFX_CUDA(cudaMemsetAsync(progress, 0xFF, static_cast<size_t>(pl.n_units) * 4, stream));
-    static int check = -1;      // OFX_SEARCH_CHECK: tiles between pacing checks (power of two)
-    if (check < 0) { const char* e = getenv("OFX_SEARCH_CHECK"); check = e ? atoi(e) : 8; if (check < 1 || (check & (check - 1))) check = 8; }
-    static int lead = -1;       // OFX_SEARCH_LEAD: prefetch-leader policy bits (SchedSearch::Params::lead)
-    if (lead < 0) { const char* e = getenv("OFX_SEARCH_LEAD"); lead = e ? atoi(e) : 3; }
-    SchedSearch::Params sp{pl.n_qgroups, pl.n_tiles, pl.seg_tiles, pl.n_units, pl.sub_tiles, CL, pf_dist, progress, window, check, lead};
+    if (ep.progress) OFX_CUDA(cudaMemsetAsync(ep.progress, 0xFF, static_cast<size_t>(pl.n_units) * 4, stream));
+    SchedSearch::Params sp{pl.n_qgroups, pl.n_tiles, pl.seg_tiles, pl.n_units, CL, ep.progress};
     cudaLaunchConfig_t cfg{};
     cfg.gridDim = dim3(pl.grid);
     cfg.blockDim = dim3(tc_threads<Epi>());
@@ -1516,8 +1485,8 @@ static int launch_search(const void* q_bf16, int n_query, const void* gallery, l
         long long h[8 * 256];
         OFX_CUDA(cudaStreamSynchronize(stream));
         OFX_CUDA(cudaMemcpy(h, prof_dev, sizeof(h), cudaMemcpyDeviceToHost));
-        fprintf(stderr, "search prof nq=%d rows=%lld grid=%d cl=%d seg_tiles=%d sub=%d: cta0 mma total %lld wait_full %lld wait_tmem_empty %lld | epi total %lld wait_tmem_full %lld ; cta100 mma %lld %lld %lld | epi %lld %lld\n",
-                n_query, n_rows, pl.grid, CL, pl.seg_tiles, pl.sub_tiles, h[0], h[1], h[2], h[4], h[5], h[800], h[801], h[802], h[804], h[805]);
+        fprintf(stderr, "search prof nq=%d rows=%lld grid=%d cl=%d seg_tiles=%d: cta0 mma total %lld wait_full %lld wait_tmem_empty %lld | epi total %lld wait_tmem_full %lld ; cta100 mma %lld %lld %lld | epi %lld %lld\n",
+                n_query, n_rows, pl.grid, CL, pl.seg_tiles, h[0], h[1], h[2], h[4], h[5], h[800], h[801], h[802], h[804], h[805]);
         // per-unit timeline of CTA 0's first epilogue warp: wall cycles, of which inside Epi::tile (busy includes the
         // wait share measured separately = waiting for the accumulator)
         for (int u = 0; u < h[1199] && u < 40; ++u)
@@ -1531,13 +1500,10 @@ static int launch_search_cl(const void* q_bf16, int n_query, const void* gallery
                             const SearchPlan& pl, const typename Epi::Params& ep, int dim,
                             cudaStream_t stream) {
     // CTA pairs (cta_group::2, M = 256: each CTA parks only half of the gallery tile, 32 KB stages, 6-deep ring)
-    // are the default since the pacing window removed the HBM traffic: 133.4 vs 137.6 ms at 10 M rows, 20.4 vs
-    // 21.1 ms at 1.25 M.  (Before it the multicast cluster was ahead, 1004 vs 940 TFLOP/s.)  OFX_SEARCH_PAIR=0
-    // selects the multicast cluster.  What is left is L2 -> SM throughput: 1.39 TB per sweep = ~11 TB/s.
-    static int pair = -1;
-    if (pair < 0) { const char* e = getenv("OFX_SEARCH_PAIR"); pair = (e && e[0] == '0') ? 0 : 1; }
-    if (pl.cl == 2 && pair) return launch_search<Epi, kPairStages, 2, true>(q_bf16, n_query, gallery, n_rows, pl, ep, dim, stream);
-    if (pl.cl == 2) return launch_search<Epi, STAGES, 2>(q_bf16, n_query, gallery, n_rows, pl, ep, dim, stream);
+    // beat a multicast cluster (both CTAs park the whole tile) once the pacing window removed the HBM traffic:
+    // 133.4 vs 137.6 ms at 10 M rows, 20.4 vs 21.1 ms at 1.25 M.  (Before it the multicast cluster was ahead,
+    // 1004 vs 940 TFLOP/s.)  What is left is L2 -> SM throughput: 1.39 TB per sweep = ~11 TB/s.
+    if (pl.cl == 2) return launch_search<Epi, kPairStages, 2>(q_bf16, n_query, gallery, n_rows, pl, ep, dim, stream);
     return launch_search<Epi, STAGES, 1>(q_bf16, n_query, gallery, n_rows, pl, ep, dim, stream);
 }
 
@@ -1569,7 +1535,7 @@ struct CatWs {
 static CatWs cat_ws(int dim, int n_cat, int n_query, int k) {
     CatWs w{};
     w.kcap = kcap_for(k);
-    w.cl = cluster_size();
+    w.cl = 2;   // CTA pairs
     w.n_cta = sm_count() / w.cl;
     const long long groups = (n_query + kBM - 1) / kBM + (n_query < n_cat ? n_query : n_cat);
     w.q_rows = groups * w.cl * kBM;
@@ -1592,9 +1558,9 @@ static CatWs cat_ws(int dim, int n_cat, int n_query, int k) {
     return w;
 }
 
-// pass 1 of the category search: the same tcgen05 kernel as the flat search on the category schedule (CTA pairs,
-// or single CTAs with OFX_CLUSTER=1); CTAs past the last unit leave at once
-template <int KCAP, int STAGES, int CL, bool PAIR>
+// pass 1 of the category search: the same tcgen05 kernel as the flat search on the category schedule (CTA pairs);
+// CTAs past the last unit leave at once
+template <int KCAP, int STAGES, int CL>
 static int launch_cat(const void* q_bf16, long long q_rows, const void* gallery, long long n_rows,
                       const SchedCat::Params& sp, int grid, const typename EpiTopK<KCAP, SchedCat>::Params& ep, int dim,
                       cudaStream_t stream) {
@@ -1603,8 +1569,8 @@ static int launch_cat(const void* q_bf16, long long q_rows, const void* gallery,
     const int kdim = dim + kAugCols;
     OFX_TRY(make_tmap_bf16(&tm_q, q_bf16, static_cast<uint64_t>(q_rows), kdim, kdim, kBM));
     OFX_TRY(make_tmap_bf16(&tm_g, gallery, static_cast<uint64_t>(n_rows), kdim, kdim, kSearchBN / CL));
-    auto kern = tc_kernel<kSearchBN, STAGES, CL, SchedCat, Epi, PAIR>;
-    constexpr int smem = tc_smem_bytes<kSearchBN, STAGES, Epi, PAIR>();
+    auto kern = tc_kernel<kSearchBN, STAGES, CL, SchedCat, Epi>;
+    constexpr int smem = tc_smem_bytes<kSearchBN, STAGES, Epi, CL>();
     static_assert(smem <= 232448, "search kernel shared memory");
     static DeviceOnce configured;
     if (configured.need()) OFX_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -1629,8 +1595,8 @@ template <int KCAP, int STAGES, int kPairStages>
 static int launch_cat_cl(int cl, const void* q_bf16, long long q_rows, const void* gallery, long long n_rows,
                          const SchedCat::Params& sp, int grid, const typename EpiTopK<KCAP, SchedCat>::Params& ep,
                          int dim, cudaStream_t stream) {
-    if (cl == 2) return launch_cat<KCAP, kPairStages, 2, true>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
-    return launch_cat<KCAP, STAGES, 1, false>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
+    if (cl == 2) return launch_cat<KCAP, kPairStages, 2>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
+    return launch_cat<KCAP, STAGES, 1>(q_bf16, q_rows, gallery, n_rows, sp, grid, ep, dim, stream);
 }
 
 }  // namespace ofx
@@ -1706,67 +1672,43 @@ int ofx_topk_search(const void* packed, const float* gallery_f32, int64_t n_rows
         OFX_CUDA(cudaMemsetAsync(thr, 0, static_cast<size_t>(W.plan.n_qgroups) * W.plan.cl * 128 * 4, st));
         // Threshold seeding (EpiBlockMax): the kcap-th largest of 2 kcap block maxima over the first rows is a
         // valid lower bound of every query's final kcap-th best, so the main sweep starts near the 0.5 %
-        // quantile instead of cold and most of the divergent list insertions never happen.  OFX_WARM_ROWS sets
-        // the rows swept (multiple of 256, default 64 blocks x 128 = 8192; 0 = off); OFX_WARM_LEGACY=1 runs the
-        // previous warm-up (the real top-k epilogue over 4096 rows, 1.15 ms) for A/B timing.
-        static long long kWarmRows = -1;
-        static int warm_legacy = -1;
-        if (kWarmRows < 0) {
-            const char* e = getenv("OFX_WARM_ROWS");
-            const char* l = getenv("OFX_WARM_LEGACY");
-            warm_legacy = (l && l[0] == '1') ? 1 : 0;
-            kWarmRows = e ? atoll(e) : (warm_legacy ? 4096 : 8192);
-            if (kWarmRows % 256) kWarmRows = warm_legacy ? 4096 : 8192;
-        }
-        const long long warm_rows = kWarmRows * (W.kcap / 32);    // 2 kcap blocks of 128 rows by default
-        static int use_hist = -1;       // OFX_SEARCH_HIST=0: no counting bound (A/B timing)
-        if (use_hist < 0) { const char* e = getenv("OFX_SEARCH_HIST"); use_hist = (e && e[0] == '0') ? 0 : 1; }
+        // quantile instead of cold and most of the divergent list insertions never happen.  A sample segment is
+        // 2 kcap blocks of 128 rows; shards of fewer than 16 such segments are not seeded.
+        const long long warm_rows = 8192LL * (W.kcap / 32);
         float* bm = reinterpret_cast<float*>(ws + W.bm);
         float4* hq = nullptr;
         uint32_t* hist = nullptr;
-        if (kWarmRows > 0 && n_rows >= 16 * warm_rows) {
-            if (warm_legacy) {
-                SearchPlan wp = make_plan(kWarmRows, n_query, sm_count());
-                if (W.kcap == 32 && wp.cl == W.plan.cl && wp.n_units <= W.plan.n_units) {
-                    EpiTopK<32>::Params ep{kWarmRows, n_query, thr, cand_s, cand_i, cand_n, prog, nullptr, nullptr, k};
-                    OFX_TRY((launch_search_cl<EpiTopK<32>, 4, 6>(q_bf16, n_query, pk, kWarmRows, wp, ep, dim, st)));
-                }
-            } else if (warm_rows / 128 >= W.kcap) {
-                // same query blocks / cluster shape; one sample segment of warm_rows rows per idle CTA pair of a
-                // query group (all units run in one wave), at most kSeedSegments and 1/16 of the shard
-                SearchPlan wp = W.plan;
-                const int n_cl = sm_count() / wp.cl;
-                int n_seg = n_cl / (wp.n_qgroups > 0 ? wp.n_qgroups : 1);
-                n_seg = n_seg < 1 ? 1 : (n_seg > kSeedSegments ? kSeedSegments : n_seg);
-                while (n_seg > 1 && n_rows < 16 * warm_rows * n_seg) --n_seg;
-                static int seed_seg = -1;       // OFX_SEED_SEGMENTS: cap (A/B timing)
-                if (seed_seg < 0) { const char* e = getenv("OFX_SEED_SEGMENTS"); seed_seg = e ? atoi(e) : kSeedSegments; }
-                if (seed_seg >= 1 && n_seg > seed_seg) n_seg = seed_seg;
-                const long long sample_rows = warm_rows * n_seg;
-                wp.seg_tiles = static_cast<int>(warm_rows / kSearchBN);
-                wp.n_seg = n_seg;
-                wp.n_tiles = wp.seg_tiles * n_seg;
-                wp.n_units = wp.n_qgroups * n_seg;
-                wp.grid = (wp.n_units < n_cl ? wp.n_units : n_cl) * wp.cl;
-                const int nb_seg = static_cast<int>(warm_rows / 128), nb_total = nb_seg * n_seg;
-                if (W.kcap == 32) {
-                    EpiBlockMax<64>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
-                    OFX_TRY((launch_search_cl<EpiBlockMax<64>, 4, 6>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
-                } else if (W.kcap == 64) {
-                    EpiBlockMax<128>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
-                    OFX_TRY((launch_search_cl<EpiBlockMax<128>, 3, 5>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
-                } else {
-                    EpiBlockMax<256>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
-                    OFX_TRY((launch_search_cl<EpiBlockMax<256>, 2, 3>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
-                }
-                if (use_hist) {       // every query gets a seeded bound and a sample maximum: the counting bound can run
-                    hq = reinterpret_cast<float4*>(ws + W.hq);
-                    hist = reinterpret_cast<uint32_t*>(ws + W.hist);
-                }
-                seed_finish_kernel<<<(n_query + 7) / 8, 256, 0, st>>>(queries, n_query, dim, metric, bm, nb_total, W.kcap, thr,
-                    reinterpret_cast<const float*>(pk + L.stats), hq, hist);
-                OFX_LAUNCH_CHECK();
+        if (n_rows >= 16 * warm_rows) {
+            // same query blocks / cluster shape; one sample segment of warm_rows rows per idle CTA pair of a
+            // query group (all units run in one wave), at most kSeedSegments and 1/16 of the shard
+            SearchPlan wp = W.plan;
+            const int n_cl = sm_count() / wp.cl;
+            int n_seg = n_cl / (wp.n_qgroups > 0 ? wp.n_qgroups : 1);
+            n_seg = n_seg < 1 ? 1 : (n_seg > kSeedSegments ? kSeedSegments : n_seg);
+            while (n_seg > 1 && n_rows < 16 * warm_rows * n_seg) --n_seg;
+            const long long sample_rows = warm_rows * n_seg;
+            wp.seg_tiles = static_cast<int>(warm_rows / kSearchBN);
+            wp.n_seg = n_seg;
+            wp.n_tiles = wp.seg_tiles * n_seg;
+            wp.n_units = wp.n_qgroups * n_seg;
+            wp.grid = (wp.n_units < n_cl ? wp.n_units : n_cl) * wp.cl;
+            const int nb_seg = static_cast<int>(warm_rows / 128), nb_total = nb_seg * n_seg;
+            if (W.kcap == 32) {
+                EpiBlockMax<64>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
+                OFX_TRY((launch_search_cl<EpiBlockMax<64>, 4, 6>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
+            } else if (W.kcap == 64) {
+                EpiBlockMax<128>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
+                OFX_TRY((launch_search_cl<EpiBlockMax<128>, 3, 5>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
+            } else {
+                EpiBlockMax<256>::Params ep{sample_rows, n_query, prog, bm, nb_seg, nb_total};
+                OFX_TRY((launch_search_cl<EpiBlockMax<256>, 2, 3>(q_bf16, n_query, pk, sample_rows, wp, ep, dim, st)));
             }
+            // every query gets a seeded bound and a sample maximum: the counting bound can run
+            hq = reinterpret_cast<float4*>(ws + W.hq);
+            hist = reinterpret_cast<uint32_t*>(ws + W.hist);
+            seed_finish_kernel<<<(n_query + 7) / 8, 256, 0, st>>>(queries, n_query, dim, metric, bm, nb_total, W.kcap, thr,
+                reinterpret_cast<const float*>(pk + L.stats), hq, hist);
+            OFX_LAUNCH_CHECK();
         }
         if (W.kcap == 32) {
             EpiTopK<32>::Params ep{n_rows, n_query, thr, cand_s, cand_i, cand_n, prog, hist, hq, k};

@@ -13,17 +13,16 @@
 // Three barrier rings: smem full/empty (TMA <-> MMA), TMEM full/empty (MMA <-> epilogue).
 // The tile sequence comes from a Sched object that all roles evaluate identically.
 //
-// CL == 2, PAIR = false: a multicast cluster -- two CTAs with different A tiles and the SAME B tile;
-// each fetches half of the B rows and TMA-multicasts them into both, every CTA issues its own
-// M = 128 MMAs.  (Was best for the search kernel while it was HBM / power bound: 1004 vs 940 TFLOP/s at
-// 10 M rows; with the pacing window of SchedSearch the pair mode below is 3 % ahead and is its default.)
-// CL == 2, PAIR = true: a CTA PAIR (cluster of 2, tcgen05 cta_group::2).  The two CTAs own consecutive M
+// CL == 1: a single CTA issues its own M = 128 MMAs on a whole B tile.
+// CL == 2: a CTA PAIR (cluster of 2, tcgen05 cta_group::2).  The two CTAs own consecutive M
 // tiles (256 rows together) and the same B tile (n0); the even CTA issues M = 256 MMAs, each CTA
 // supplies its own 128 rows of A and HALF of the B tile from its own shared memory and receives
 // its 128 accumulator rows in its own TMEM.  Against two independent CTAs (or a multicast
 // cluster, which still parks the whole B tile in both CTAs) this cuts the shared-memory traffic
 // per SM from 192 B/clk (96 operand reads + 96 TMA fills at full tensor rate, above the 128 B/clk
-// the SM can move) to 128 B/clk, and the stage footprint from 48 KB to 32 KB (6 stages).
+// the SM can move) to 128 B/clk, and the stage footprint from 48 KB to 32 KB (6 stages).  (A
+// multicast cluster was ahead for the search kernel while it was HBM / power bound, 1004 vs 940
+// TFLOP/s at 10 M rows; with the pacing window of SchedSearch the pair is 3 % ahead.)
 // The Sched must give both CTAs of a pair the same tile count and n0.
 #pragma once
 #include <cuda.h>
@@ -37,10 +36,10 @@ constexpr int kBK = 64;        // bf16 elements per smem row = 128 B = one swizz
 constexpr int kUmmaK = 16;     // K per tcgen05.mma for 16-bit inputs
 constexpr int kEpiWarp0 = 4;   // first epilogue warp (warp % 4 selects the TMEM lane quarter)
 
-template <int BN, int STAGES, bool PAIR = false>
+template <int BN, int STAGES, int CL = 1>
 struct TcCfg {
     static constexpr int kABytes = kBM * kBK * 2;
-    static constexpr int kBBytes = (PAIR ? BN / 2 : BN) * kBK * 2;   // pair: each CTA holds half of the B tile
+    static constexpr int kBBytes = BN / CL * kBK * 2;   // pair: each CTA holds half of the B tile
     static constexpr int kStageBytes = kABytes + kBBytes;
     static constexpr int kStages = STAGES;
     static constexpr int kTmemCols = 2 * BN;  // power of two for BN in {64,128,256}
@@ -48,9 +47,9 @@ struct TcCfg {
     static constexpr int kBarBytes = 1024;  // barriers + tmem slot; keeps the epilogue smem 1024-byte aligned (TMA swizzle)
 };
 
-template <int BN, int STAGES, class Epi, bool PAIR = false>
+template <int BN, int STAGES, class Epi, int CL = 1>
 constexpr int tc_smem_bytes() {
-    return 1024 /*alignment slack*/ + TcCfg<BN, STAGES, PAIR>::kRingBytes + TcCfg<BN, STAGES, PAIR>::kBarBytes +
+    return 1024 /*alignment slack*/ + TcCfg<BN, STAGES, CL>::kRingBytes + TcCfg<BN, STAGES, CL>::kBarBytes +
            Epi::kSmemBytes;
 }
 
@@ -78,17 +77,14 @@ constexpr int tc_threads() { return 128 + 32 * Epi::kWarps; }
 // {total, wait smem-full, wait tmem-empty} and of epilogue warp 0 {total, wait tmem-full}.
 __device__ long long* g_tc_prof = nullptr;
 
-template <int BN, int STAGES, int CL, class Sched, class Epi, bool PAIR = false>
+template <int BN, int STAGES, int CL, class Sched, class Epi>
 __global__ void __launch_bounds__(128 + 32 * Epi::kWarps, 1)
 tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b,
           const typename Sched::Params sp, const __grid_constant__ typename Epi::Params ep,
           const int num_k_blocks) {
-    static_assert(CL == 1 || CL == 2, "CL = 1 (single CTA) or 2 (multicast cluster or CTA pair)");
-    static_assert(!PAIR || CL == 2, "a pair is a cluster of 2");
-    using Cfg = TcCfg<BN, STAGES, PAIR>;
-    constexpr bool kPair = PAIR;
-    constexpr bool kMcast = CL == 2 && !PAIR;   // B tile multicast into both CTAs, independent MMAs
-    constexpr uint16_t kAllCtas = static_cast<uint16_t>((1u << CL) - 1u);
+    static_assert(CL == 1 || CL == 2, "CL = 1 (single CTA) or 2 (CTA pair)");
+    using Cfg = TcCfg<BN, STAGES, CL>;
+    constexpr bool kPair = CL == 2;
     extern __shared__ uint8_t smem_raw[];
     // SWIZZLE_128B tiles need 1024-byte aligned bases
     uint8_t* smem = reinterpret_cast<uint8_t*>(
@@ -115,7 +111,7 @@ tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
     if (warp == 1 && lane == 0) {
         for (int i = 0; i < Cfg::kStages; ++i) {
             mbar_init(&full[i], 1);     // pair: the leader's collects the bytes of both CTAs
-            mbar_init(&empty[i], kMcast ? CL : 1);   // multicast: every CTA's MMAs must retire before a refill
+            mbar_init(&empty[i], 1);
         }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&tmem_full[i], 1);
@@ -151,12 +147,7 @@ tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
                     if constexpr (!kPair) {
                         mbar_arrive_expect_tx(&full[stage], Cfg::kStageBytes);
                         tma_load_2d(s_a + stage * Cfg::kABytes, &tm_a, &full[stage], kb * kBK, sched.m0);
-                        if constexpr (!kMcast) {
-                            tma_load_2d(s_b + stage * Cfg::kBBytes, &tm_b, &full[stage], kb * kBK, sched.n0);
-                        } else {   // this CTA's half of the B rows lands in BOTH CTAs (and signals both barriers)
-                            tma_load_2d_mc(s_b + stage * Cfg::kBBytes + crank * (kBRowsPerCta * kBK * 2), &tm_b,
-                                           &full[stage], kb * kBK, sched.n0 + crank * kBRowsPerCta, kAllCtas);
-                        }
+                        tma_load_2d(s_b + stage * Cfg::kBBytes, &tm_b, &full[stage], kb * kBK, sched.n0);
                     } else {
                         // both CTAs' bytes are accounted on the leader's barrier
                         if (crank == 0) mbar_arrive_expect_tx(&full[stage], 2 * Cfg::kStageBytes);
@@ -209,7 +200,6 @@ tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
                         }
                         // frees the smem slot (in both CTAs of a pair) when the MMAs retire
                         if constexpr (kPair) umma_commit_pair(&empty[stage], 0b11);
-                        else if constexpr (kMcast) umma_commit_mc(&empty[stage], kAllCtas);
                         else umma_commit(&empty[stage]);
                     }
                     __syncwarp();

@@ -1,5 +1,5 @@
 """GPU: the fused feed-forward block (ofx_ffn_block_bf16: LayerNorm -> linear1 -> mish -> linear2
--> +residual in one tcgen05 cta_group::2 kernel; OFX_FFN_V1=1 runs the round-1 kernel through the same tests) against a torch fp32 evaluation of the same
+-> +residual in one tcgen05 cta_group::2 kernel) against a torch fp32 evaluation of the same
 arithmetic (torch TransformerEncoderLayer._ff_block as the reference configures it,
 /root/reference/src/models/outfit_x.py:32-45), with the operands rounded to bf16 where the
 kernel rounds them (LN output, weights, hidden activation)."""

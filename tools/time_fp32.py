@@ -1,5 +1,5 @@
-"""CP pass in precision="fp32": linear layers on the tensor cores (bf16 hi / lo split, default) against the CUDA-core
-GEMM (OFX_FP32_TC=0).  Usage: [OFX_FP32_TC=0] python tools/time_fp32.py [batch]"""
+"""CP pass in precision="fp32": linear layers on the tensor cores (bf16 hi / lo split).
+Usage: python tools/time_fp32.py [batch]"""
 import os, sys, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench
