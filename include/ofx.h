@@ -47,7 +47,13 @@ enum {
 /* arithmetic of the hot GEMMs */
 enum {
     OFX_PREC_BF16 = 0, /* bf16 operands on tcgen05 tensor cores, fp32 accumulate (TMEM)   */
-    OFX_PREC_FP32 = 1  /* fp32 (split-bf16 tensor-core GEMMs): the <=1e-3-relative parity mode */
+    OFX_PREC_FP32 = 1, /* fp32 (split-bf16 tensor-core GEMMs): the <=1e-3-relative parity mode */
+    OFX_PREC_FP16 = 2  /* fp16 operands, fp32 accumulate: the arithmetic of the reference's
+                        * evaluation under torch.autocast(float16).  The residual stream,
+                        * LayerNorm / softmax statistics and the heads stay fp32 as in bf16 mode;
+                        * an operand outside the fp16 range (|v| > 65504) overflows to inf, as it
+                        * does under autocast -- nothing is clamped.  Packed weights and workspace
+                        * have the bf16 sizes. */
 };
 
 enum { OFX_TASK_CP = 0, OFX_TASK_CIR = 1 }; /* FITB uses the CIR task (outfit_x.py:86-87) */
@@ -270,6 +276,12 @@ OFX_API int ofx_cp_metrics(const float* logits, const float* labels, int64_t n, 
 OFX_API int ofx_gemm_bf16(const void* a, int64_t lda, const void* w, int64_t ldw, int32_t m, int32_t n,
                   int32_t k, const float* bias, int32_t act_mish, const float* residual,
                   int64_t ldr, void* out, int64_t ldo, int32_t out_f32, void* stream);
+/* The same with fp16 A and W (the linear layers of precision OFX_PREC_FP16).  out_f32 = 0 writes fp16 and takes no
+ * residual (OFX_E_ARG); out_f32 = 1 writes fp32 with or without the fp32 residual.  Results outside the fp16 range
+ * overflow to inf, as under the reference's autocast; nothing is clamped. */
+OFX_API int ofx_gemm_f16(const void* a, int64_t lda, const void* w, int64_t ldw, int32_t m, int32_t n,
+                 int32_t k, const float* bias, int32_t act_mish, const float* residual,
+                 int64_t ldr, void* out, int64_t ldo, int32_t out_f32, void* stream);
 
 /* ---- the fp32 mode's linear layer (the nn.Linear / F.linear calls inside the nn.TransformerEncoderLayer stack of
  * src/models/outfit_x.py:32-45 and the CIR head :62-66 when the model runs without autocast) on the tensor cores:
@@ -303,6 +315,15 @@ OFX_API int ofx_ffn_block_ln_bf16(float* x, int32_t rows, int32_t d_model, int32
                           const float* ln_w, const float* ln_b, const void* w1, const float* b1,
                           const void* w2, const float* b2, void* h_next, const float* next_ln_w,
                           const float* next_ln_b, void* workspace, size_t workspace_bytes, void* stream);
+
+/* The fp16 form of both (precision OFX_PREC_FP16): w1 / w2 fp16, LayerNorm output, hidden activation and h_next
+ * rounded to fp16, fp32 accumulation and residual stream.  h_next (rows, d_model) fp16 may be NULL: the plain block
+ * (next_ln_w / next_ln_b are then ignored).  Same shapes and workspace rule as ofx_ffn_block_bf16.  Values outside
+ * the fp16 range overflow to inf, as under the reference's autocast; nothing is clamped. */
+OFX_API int ofx_ffn_block_f16(float* x, int32_t rows, int32_t d_model, int32_t d_ffn_padded,
+                      const float* ln_w, const float* ln_b, const void* w1, const float* b1,
+                      const void* w2, const float* b2, void* h_next, const float* next_ln_w,
+                      const float* next_ln_b, void* workspace, size_t workspace_bytes, void* stream);
 
 #ifdef __cplusplus
 }

@@ -14,7 +14,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("OFX_LIB_PATH") or os.path.join(HERE, "libofx.so")
 
 OFX_OK = 0
-PREC_BF16, PREC_FP32 = 0, 1
+PREC_BF16, PREC_FP32, PREC_FP16 = 0, 1, 2
 TASK_CP, TASK_CIR = 0, 1
 FUSE_CONCAT, FUSE_MEAN = 0, 1
 METRIC_DOT, METRIC_L2 = 0, 1
@@ -104,6 +104,12 @@ _SIGNATURES = {
     "ofx_gemm_bf16": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
                                 C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64,
                                 C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "ofx_gemm_f16": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
+                               C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64,
+                               C.c_void_p, C.c_int64, C.c_int32, C.c_void_p]),
+    "ofx_ffn_block_f16": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "ofx_gemm_f32_tc_workspace_bytes": (C.c_size_t, [C.c_int32, C.c_int32, C.c_int32]),
     "ofx_gemm_f32_tc": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
                                   C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64,

@@ -3,6 +3,7 @@
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -62,6 +63,8 @@ struct DeviceOnce {
 
 // 2-D bf16 tensor map: `rows` x `cols` elements, row pitch `ld` elements, box = box_rows x 64
 // elements (128 B) with the 128-byte swizzle the UMMA descriptors expect; OOB reads give zeros.
+// TMA moves the 2-byte elements without interpreting them (OOB_FILL_NONE writes zero bits), so the
+// same map carries fp16 rows.
 int make_tmap_bf16(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t ld,
                    uint32_t box_rows);
 

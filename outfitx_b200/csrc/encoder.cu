@@ -1,5 +1,5 @@
 // Encoder forward of the outfit-scoring path behind the C ABI:
-//   ofx_pack_weights / ofx_encoder_forward / ofx_fuse / ofx_gemm_bf16.
+//   ofx_pack_weights / ofx_encoder_forward / ofx_fuse / ofx_gemm_bf16 / ofx_gemm_f16.
 // Mirrors OutfitX._cp_forward / _cir_forward (/root/reference/src/models/outfit_x.py:120-172)
 // with the exact simplifications of SURVEY.md App. A.4: padded tokens dropped, last layer
 // evaluated for the prefix-token query row only.
@@ -30,15 +30,15 @@ static int check_shape(const ofx_shape* s) {
     if (s->d_ffn < 1 || s->d_ffn > 16384) return fail(OFX_E_SHAPE, "d_ffn %d", s->d_ffn);
     if (s->d_embed < 128 || s->d_embed % 128) return fail(OFX_E_SHAPE, "d_embed %d must be a multiple of 128", s->d_embed);
     if (s->max_items < 1 || s->max_items > 16) return fail(OFX_E_SHAPE, "max_items %d not in [1,16]", s->max_items);
-    if (s->precision != OFX_PREC_BF16 && s->precision != OFX_PREC_FP32)
-        return fail(OFX_E_ARG, "precision %d", s->precision);
+    if (s->precision != OFX_PREC_BF16 && s->precision != OFX_PREC_FP32 && s->precision != OFX_PREC_FP16)
+        return fail(OFX_E_ARG, "precision %d not in {0 (bf16), 1 (fp32), 2 (fp16)}", s->precision);
     return OFX_OK;
 }
 
 static WLayout make_layout(const ofx_shape* s) {
     WLayout L{};
     L.dm = s->d_model; L.de = s->d_embed; L.f = s->d_ffn; L.fp = round_up(s->d_ffn, 128); L.nl = s->n_layers;
-    L.esz = s->precision == OFX_PREC_BF16 ? 2 : 4;
+    L.esz = s->precision == OFX_PREC_FP32 ? 4 : 2;     // bf16 and fp16: 2-byte matrices
     size_t o = 0;
     auto take = [&](size_t bytes) { size_t at = o; o = align_up(o + bytes, 256); return at; };
     const size_t dm = L.dm, fp = L.fp;
@@ -117,7 +117,7 @@ struct WsLayout {
 };
 static WsLayout make_ws(const ofx_shape* s, int batch) {
     WsLayout W{};
-    const size_t esz = s->precision == OFX_PREC_BF16 ? 2 : 4;
+    const size_t esz = s->precision == OFX_PREC_FP32 ? 4 : 2;
     const size_t dm = s->d_model, fp = round_up(s->d_ffn, 128);
     W.t_max = batch * (s->max_items + 1);
     W.big_ld = static_cast<int>(3 * dm > fp ? 3 * dm : fp);
@@ -135,13 +135,23 @@ static WsLayout make_ws(const ofx_shape* s, int batch) {
     W.q0 = take(static_cast<size_t>(batch) * dm * esz);
     W.a0 = take(static_cast<size_t>(batch) * dm * esz);
     W.u0 = take(static_cast<size_t>(batch) * fp * (s->precision == OFX_PREC_FP32 ? 6 : esz));
-    // the fused FFN block's workspace (bf16 path, d_model 512; the kernel itself uses none of it)
-    W.ffn_bytes = (s->precision == OFX_PREC_BF16 && ffn_block_supported(s->d_model, static_cast<int>(fp))) ? ffn_block_workspace_bytes() : 0;
+    // the fused FFN block's workspace (bf16 / fp16 path, d_model 512; the kernel itself uses none of it)
+    W.ffn_bytes = (s->precision != OFX_PREC_FP32 && ffn_block_supported(s->d_model, static_cast<int>(fp))) ? ffn_block_workspace_bytes() : 0;
     W.ffn = take(W.ffn_bytes);
     // fp32 precision: bf16 hi / lo pieces of the current GEMM's activation operand (3 x K bf16 per token row)
     W.split = take(s->precision == OFX_PREC_FP32 ? t * 3 * (dm > fp ? dm : fp) * 2 : 0);
     W.total = o;
     return W;
+}
+
+// the 16-bit building blocks for operand type T (__nv_bfloat16 or __half)
+template <class T>
+static int gemm_16(const GemmArgs& g, cudaStream_t st) {
+    return std::is_same<T, __half>::value ? gemm_f16(g, st) : gemm_bf16(g, st);
+}
+template <class T>
+static int ffn_block_16(const FfnBlockArgs& a, cudaStream_t st) {
+    return std::is_same<T, __half>::value ? ffn_block_f16(a, st) : ffn_block_bf16(a, st);
 }
 
 template <class T>
@@ -161,7 +171,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
     T* u0 = reinterpret_cast<T*>(ws + W.u0);
     auto lw = [&](int l, size_t o) { return wts + L.layer_bytes * l + o; };
     auto lf = [&](int l, size_t o) { return reinterpret_cast<const float*>(lw(l, o)); };
-    // linear layer: bf16 mode -> tcgen05 GEMM on the bf16 operands; fp32 mode -> the activation operand is cut into
+    // linear layer: bf16 / fp16 mode -> tcgen05 GEMM on the 16-bit operands; fp32 mode -> the activation operand is cut into
     // bf16 hi / lo pieces and multiplied with the pre-split weights on the same tensor-core pipeline (gemm.h)
     uint8_t* split_a = ws + W.split;
     constexpr bool f32 = sizeof(T) == 4;
@@ -179,7 +189,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
             return gemm_f32_split(t, st);
         } else {
             (void)w_split; (void)a_pre; (void)piece_out;
-            return gemm_bf16(g, st);
+            return gemm_16<T>(g, st);
         }
     };
     // LayerNorm in front of a linear layer: h = LN(x); in fp32 mode the pieces of the GEMM operand are
@@ -233,7 +243,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
                                 lf(l, L.b_1), lw(l, L.w_2), lf(l, L.b_2)};
                 fa.h_next = h; fa.lnn_w = lf(l + 1, L.ln1w); fa.lnn_b = lf(l + 1, L.ln1b);
                 fa.workspace = ws + W.ffn; fa.workspace_bytes = W.ffn_bytes;
-                OFX_TRY(ffn_block_bf16(fa, st));
+                OFX_TRY(ffn_block_16<T>(fa, st));
             } else {
                 const void* pre2 = nullptr;
                 OFX_TRY(ln_mm(W.t_max, n_tok, lf(l, L.ln2w), lf(l, L.ln2b), &pre2));
@@ -261,7 +271,7 @@ static int forward(const ofx_shape* s, const uint8_t* wts, const ofx_forward_arg
                 FfnBlockArgs fa{x, B, nullptr, dm, fp, lf(l, L.ln2w), lf(l, L.ln2b), lw(l, L.w_1),
                                 lf(l, L.b_1), lw(l, L.w_2), lf(l, L.b_2)};
                 fa.workspace = ws + W.ffn; fa.workspace_bytes = W.ffn_bytes;
-                OFX_TRY(ffn_block_bf16(fa, st));
+                OFX_TRY(ffn_block_16<T>(fa, st));
             } else {
                 const void* pre2 = nullptr;
                 OFX_TRY(ln_mm(B, nullptr, lf(l, L.ln2w), lf(l, L.ln2b), &pre2));
@@ -306,6 +316,8 @@ int ofx_pack_weights(const ofx_shape* shape, const float* const* params, void* p
     OFX_CUDA(cudaMemsetAsync(packed, 0, L.total, st));
     if (shape->precision == OFX_PREC_BF16)
         return pack_all<__nv_bfloat16>(L, params, static_cast<uint8_t*>(packed), st);
+    if (shape->precision == OFX_PREC_FP16)
+        return pack_all<__half>(L, params, static_cast<uint8_t*>(packed), st);
     return pack_all<float>(L, params, static_cast<uint8_t*>(packed), st);
 }
 
@@ -348,6 +360,9 @@ int ofx_encoder_forward(const ofx_shape* shape, const void* packed_weights, cons
     if (shape->precision == OFX_PREC_BF16)
         return forward<__nv_bfloat16>(shape, static_cast<const uint8_t*>(packed_weights), a,
                                       static_cast<uint8_t*>(workspace), st);
+    if (shape->precision == OFX_PREC_FP16)
+        return forward<__half>(shape, static_cast<const uint8_t*>(packed_weights), a,
+                               static_cast<uint8_t*>(workspace), st);
     return forward<float>(shape, static_cast<const uint8_t*>(packed_weights), a,
                           static_cast<uint8_t*>(workspace), st);
 }
@@ -369,6 +384,15 @@ int ofx_gemm_bf16(const void* a, int64_t lda, const void* w, int64_t ldw, int32_
     OFX_TRY(require_sm100());
     GemmArgs g{a, lda, w, ldw, m, nullptr, n, k, bias, act_mish, residual, ldr, out, ldo, out_f32};
     return gemm_bf16(g, static_cast<cudaStream_t>(stream));
+}
+
+int ofx_gemm_f16(const void* a, int64_t lda, const void* w, int64_t ldw, int32_t m, int32_t n, int32_t k,
+                 const float* bias, int32_t act_mish, const float* residual, int64_t ldr, void* out,
+                 int64_t ldo, int32_t out_f32, void* stream) {
+    if (!a || !w || !out) return fail(OFX_E_ARG, "ofx_gemm_f16: null operand");
+    OFX_TRY(require_sm100());
+    GemmArgs g{a, lda, w, ldw, m, nullptr, n, k, bias, act_mish, residual, ldr, out, ldo, out_f32};
+    return gemm_f16(g, static_cast<cudaStream_t>(stream));
 }
 
 size_t ofx_gemm_f32_tc_workspace_bytes(int32_t m, int32_t n, int32_t k) {
@@ -427,5 +451,22 @@ int ofx_ffn_block_ln_bf16(float* x, int32_t rows, int32_t d_model, int32_t d_ffn
     fa.h_next = h_next; fa.lnn_w = next_ln_w; fa.lnn_b = next_ln_b;
     fa.workspace = workspace; fa.workspace_bytes = workspace_bytes;
     return ffn_block_bf16(fa, static_cast<cudaStream_t>(stream));
+}
+
+int ofx_ffn_block_f16(float* x, int32_t rows, int32_t d_model, int32_t d_ffn_padded, const float* ln_w,
+                      const float* ln_b, const void* w1, const float* b1, const void* w2, const float* b2,
+                      void* h_next, const float* next_ln_w, const float* next_ln_b, void* workspace,
+                      size_t workspace_bytes, void* stream) {
+    if (!x || !ln_w || !ln_b || !w1 || !b1 || !w2 || !b2 || (h_next && (!next_ln_w || !next_ln_b)))
+        return fail(OFX_E_ARG, "ofx_ffn_block_f16: null argument");
+    if (rows < 0) return fail(OFX_E_SHAPE, "ofx_ffn_block_f16: rows %d", rows);
+    if (!ffn_block_supported(d_model, d_ffn_padded))
+        return fail(OFX_E_SHAPE, "ofx_ffn_block_f16: needs d_model 512 and d_ffn_padded %% 256 == 0");
+    if (reinterpret_cast<uintptr_t>(h_next) % 16) return fail(OFX_E_ARG, "ofx_ffn_block_f16: misaligned h_next");
+    OFX_TRY(require_sm100());
+    FfnBlockArgs fa{x, rows, nullptr, d_model, d_ffn_padded, ln_w, ln_b, w1, b1, w2, b2};
+    fa.h_next = h_next; fa.lnn_w = next_ln_w; fa.lnn_b = next_ln_b;
+    fa.workspace = workspace; fa.workspace_bytes = workspace_bytes;
+    return ffn_block_f16(fa, static_cast<cudaStream_t>(stream));
 }
 }

@@ -10,17 +10,20 @@
 // the heads, so the result is unchanged (SURVEY.md App. A.4); the model has no positional
 // encoding, so valid items may come from any slot.
 #include "encoder_ops.h"
+#include "ptx.cuh"
 
 namespace ofx {
 
 template <class T> __device__ __forceinline__ float to_f(T v);
 template <> __device__ __forceinline__ float to_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ float to_f<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <> __device__ __forceinline__ float to_f<__half>(__half v) { return __half2float(v); }
 template <class T> __device__ __forceinline__ T from_f(float v);
 template <> __device__ __forceinline__ float from_f<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 from_f<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half from_f<__half>(float v) { return __float2half_rn(v); }
 
-// 8 consecutive elements (16-byte aligned for bf16, 32-byte for fp32) <-> fp32 registers
+// 8 consecutive elements (16-byte aligned for bf16 / fp16, 32-byte for fp32) <-> fp32 registers
 __device__ __forceinline__ void load8(const float* p, float (&v)[8]) {
     float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + 4);
     v[0] = a.x; v[1] = a.y; v[2] = a.z; v[3] = a.w; v[4] = b.x; v[5] = b.y; v[6] = b.z; v[7] = b.w;
@@ -31,6 +34,12 @@ __device__ __forceinline__ void load8(const __nv_bfloat16* p, float (&v)[8]) {
 #pragma unroll
     for (int i = 0; i < 4; ++i) { float2 f = __bfloat1622float2(h[i]); v[2 * i] = f.x; v[2 * i + 1] = f.y; }
 }
+__device__ __forceinline__ void load8(const __half* p, float (&v)[8]) {
+    uint4 u = *reinterpret_cast<const uint4*>(p);
+    const __half2* h = reinterpret_cast<const __half2*>(&u);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { float2 f = __half22float2(h[i]); v[2 * i] = f.x; v[2 * i + 1] = f.y; }
+}
 __device__ __forceinline__ void store8(float* p, const float (&v)[8]) {
     *reinterpret_cast<float4*>(p) = make_float4(v[0], v[1], v[2], v[3]);
     *reinterpret_cast<float4*>(p + 4) = make_float4(v[4], v[5], v[6], v[7]);
@@ -40,6 +49,13 @@ __device__ __forceinline__ void store8(__nv_bfloat16* p, const float (&v)[8]) {
     __nv_bfloat162* h = reinterpret_cast<__nv_bfloat162*>(&u);
 #pragma unroll
     for (int i = 0; i < 4; ++i) h[i] = __floats2bfloat162_rn(v[2 * i], v[2 * i + 1]);
+    *reinterpret_cast<uint4*>(p) = u;
+}
+__device__ __forceinline__ void store8(__half* p, const float (&v)[8]) {
+    uint4 u;
+    __half2* h = reinterpret_cast<__half2*>(&u);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) h[i] = __floats2half2_rn(v[2 * i], v[2 * i + 1]);
     *reinterpret_cast<uint4*>(p) = u;
 }
 
@@ -203,11 +219,7 @@ __device__ __forceinline__ void ln_store(const float4 (&v)[DM / 128], const floa
         if constexpr (sizeof(T) == 4) {
             *reinterpret_cast<float4*>(out + e) = make_float4(y0, y1, y2, y3);
         } else {
-            __nv_bfloat162 p0 = __floats2bfloat162_rn(y0, y1), p1 = __floats2bfloat162_rn(y2, y3);
-            uint2 u;
-            u.x = *reinterpret_cast<uint32_t*>(&p0);
-            u.y = *reinterpret_cast<uint32_t*>(&p1);
-            *reinterpret_cast<uint2*>(out + e) = u;
+            *reinterpret_cast<uint2*>(out + e) = make_uint2(pack2_16<T>(y0, y1), pack2_16<T>(y2, y3));
         }
     }
 }
@@ -282,6 +294,7 @@ int assemble(const AssembleArgs& a, int dm, float* x, T* h, cudaStream_t stream)
 }
 template int assemble<float>(const AssembleArgs&, int, float*, float*, cudaStream_t);
 template int assemble<__nv_bfloat16>(const AssembleArgs&, int, float*, __nv_bfloat16*, cudaStream_t);
+template int assemble<__half>(const AssembleArgs&, int, float*, __half*, cudaStream_t);
 
 int scan_valid(const uint8_t* mask, int batch, int max_items, int* off, int* n_tok, cudaStream_t stream) {
     scan_valid_kernel<<<1, 1024, 0, stream>>>(mask, batch, max_items, off, n_tok);
@@ -383,6 +396,7 @@ int layernorm_split3(const float* x, int rows, const int* rows_dev, int dm, cons
 
 template int layernorm<float>(const float*, int, const int*, int, const float*, const float*, float*, cudaStream_t);
 template int layernorm<__nv_bfloat16>(const float*, int, const int*, int, const float*, const float*, __nv_bfloat16*, cudaStream_t);
+template int layernorm<__half>(const float*, int, const int*, int, const float*, const float*, __half*, cudaStream_t);
 
 // ------------------------------------------------------------------ cast rows fp32 -> T
 template <class T>
@@ -401,6 +415,7 @@ int cast_rows(const float* in, long long n, T* out, cudaStream_t stream) {
 }
 template int cast_rows<float>(const float*, long long, float*, cudaStream_t);
 template int cast_rows<__nv_bfloat16>(const float*, long long, __nv_bfloat16*, cudaStream_t);
+template int cast_rows<__half>(const float*, long long, __half*, cudaStream_t);
 
 // ------------------------------------------------------------------ attention
 // Four consecutive lanes serve one (token row, head): lane `sub` owns dims {32p + 8 sub .. +8}
@@ -514,11 +529,11 @@ attention_kernel(AttnArgs a) {
     }
 }
 
-// ------------------------------------------------------------------ attention, bf16 path
+// ------------------------------------------------------------------ attention, bf16 / fp16 path
 // One CTA (4 warps) per outfit.  The outfit's q / K / V rows (S <= 17 tokens x d_model) are
 // gathered into shared memory once with 16-byte cp.async (row stride d_model + 8 elements, so
 // the ldmatrix row addresses of a fragment fall into distinct banks); every warp then serves 4
-// of the 16 heads with warp-level tensor-core MMAs (mma.sync m16n8k16, bf16 in / fp32 out):
+// of the 16 heads with warp-level tensor-core MMAs (mma.sync m16n8k16, bf16 or fp16 in / fp32 out):
 // scores = q.K^T over 16-key tiles, masked warp-shuffle softmax in registers, out = P.V with V
 // read through ldmatrix.trans.  The S x S problem is far below a tcgen05 tile (SURVEY.md H1);
 // what matters is that each q / K / V element is read from global memory exactly once and that
@@ -533,21 +548,25 @@ __device__ __forceinline__ void ldsm_x4_trans(uint32_t (&r)[4], uint32_t addr) {
     asm volatile("ldmatrix.sync.aligned.m8n8.x4.trans.shared.b16 {%0, %1, %2, %3}, [%4];"
                  : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
 }
-__device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
-    asm volatile(
-        "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
-        "{%0, %1, %2, %3};"
-        : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-        : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+template <class T>
+__device__ __forceinline__ void mma_16816(float (&d)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
+    if constexpr (std::is_same<T, __half>::value)
+        asm volatile(
+            "mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
+            "{%0, %1, %2, %3};"
+            : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+            : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
+    else
+        asm volatile(
+            "mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, "
+            "{%0, %1, %2, %3};"
+            : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
+            : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 __device__ __forceinline__ float ex2_fast(float x) {
     float y;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x));
     return y;
-}
-__device__ __forceinline__ uint32_t pack2_bf16(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&v);
 }
 
 constexpr int kAttnMaxS = 17;
@@ -562,7 +581,8 @@ constexpr int kAttnMaxS = 17;
 // overlap inside a CTA), so residency is what hides the gather.
 // SMALL: S <= 8 tokens (40 % of the outfits at n ~ U{2..16}): only query rows 0..7 (h = 0) and the first
 // 8-key n-tile exist, so the second score MMA, half of the softmax and half of the output stores are skipped.
-template <int HD, bool BIG, int NSPLIT, bool SMALL = false>
+// T: the 16-bit type of q / K / V, P and the output (__nv_bfloat16 or __half)
+template <int HD, bool BIG, int NSPLIT, class T, bool SMALL = false>
 __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* sm) {
     static_assert(!(BIG && SMALL), "one or the other");
     constexpr int MT = BIG ? 2 : 1, KT = BIG ? 2 : 1;
@@ -583,13 +603,13 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
     const int S = min(1 + (a.off[b + 1] - a.off[b]), kAttnMaxS);
     const int n_q = a.row0_only ? 1 : S;
     const int gcol = NSPLIT > 1 ? static_cast<int>(blockIdx.y) * DM : 0;     // first global column of this CTA
-    const __nv_bfloat16* gq = static_cast<const __nv_bfloat16*>(a.q) + gcol;
-    const __nv_bfloat16* gk = static_cast<const __nv_bfloat16*>(a.k) + gcol;
-    const __nv_bfloat16* gv = static_cast<const __nv_bfloat16*>(a.v) + gcol;
+    const T* gq = static_cast<const T*>(a.q) + gcol;
+    const T* gk = static_cast<const T*>(a.k) + gcol;
+    const T* gv = static_cast<const T*>(a.v) + gcol;
 
     for (int i = tid; i < STRIDE / 16; i += 128) reinterpret_cast<uint4*>(s_z)[i] = make_uint4(0, 0, 0, 0);
     // gather: 16-byte cp.async chunks, (row, chunk) advanced incrementally (no per-chunk division)
-    auto load_rows = [&](const __nv_bfloat16* g, long long ld, uint8_t* dst, int n_rows) {
+    auto load_rows = [&](const T* g, long long ld, uint8_t* dst, int n_rows) {
         int j = tid / CPR, cc = tid - j * CPR;
         while (j < n_rows) {
             const long long row = j == 0 ? b : base + j - 1;
@@ -654,8 +674,8 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
 #pragma unroll
                     for (int mt = 0; mt < MT; ++mt) {
                         if (mt < n_mt) {
-                            mma_bf16_16816(sc[mt][2 * kt], qa[mt], kb[0], kb[1]);
-                            if constexpr (!SMALL) mma_bf16_16816(sc[mt][2 * kt + 1], qa[mt], kb[2], kb[3]);
+                            mma_16816<T>(sc[mt][2 * kt], qa[mt], kb[0], kb[1]);
+                            if constexpr (!SMALL) mma_16816<T>(sc[mt][2 * kt + 1], qa[mt], kb[2], kb[3]);
                         }
                     }
                 }
@@ -695,13 +715,13 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
                 }
 #pragma unroll
                 for (int kt = 0; kt < KT; ++kt) {
-                    pa[mt][kt][0] = pack2_bf16(sc[mt][2 * kt][0], sc[mt][2 * kt][1]);
+                    pa[mt][kt][0] = pack2_16<T>(sc[mt][2 * kt][0], sc[mt][2 * kt][1]);
                     if constexpr (SMALL) {     // rows 8..15 and keys 8..15 do not exist
                         pa[mt][kt][1] = pa[mt][kt][2] = pa[mt][kt][3] = 0u;
                     } else {
-                        pa[mt][kt][1] = pack2_bf16(sc[mt][2 * kt][2], sc[mt][2 * kt][3]);
-                        pa[mt][kt][2] = pack2_bf16(sc[mt][2 * kt + 1][0], sc[mt][2 * kt + 1][1]);
-                        pa[mt][kt][3] = pack2_bf16(sc[mt][2 * kt + 1][2], sc[mt][2 * kt + 1][3]);
+                        pa[mt][kt][1] = pack2_16<T>(sc[mt][2 * kt][2], sc[mt][2 * kt][3]);
+                        pa[mt][kt][2] = pack2_16<T>(sc[mt][2 * kt + 1][0], sc[mt][2 * kt + 1][1]);
+                        pa[mt][kt][3] = pack2_16<T>(sc[mt][2 * kt + 1][2], sc[mt][2 * kt + 1][3]);
                     }
                 }
             }
@@ -725,8 +745,8 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
 #pragma unroll
                     for (int mt = 0; mt < MT; ++mt) {
                         if (mt < n_mt) {
-                            mma_bf16_16816(o[mt][0], pa[mt][kt], vb[0], vb[1]);
-                            mma_bf16_16816(o[mt][1], pa[mt][kt], vb[2], vb[3]);
+                            mma_16816<T>(o[mt][0], pa[mt][kt], vb[0], vb[1]);
+                            mma_16816<T>(o[mt][1], pa[mt][kt], vb[2], vb[3]);
                         }
                     }
                 }
@@ -743,7 +763,7 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
 #pragma unroll
                             for (int x = 0; x < 2; ++x)
                                 *reinterpret_cast<uint32_t*>(s_q + r * STRIDE + (col0 + dp * 16 + x * 8 + 2 * t4) * 2) =
-                                    pack2_bf16(o[mt][x][2 * h] * inv[mt][h], o[mt][x][2 * h + 1] * inv[mt][h]);
+                                    pack2_16<T>(o[mt][x][2 * h] * inv[mt][h], o[mt][x][2 * h + 1] * inv[mt][h]);
                         }
                     }
                 }
@@ -751,7 +771,7 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
         }
     }
     __syncthreads();
-    __nv_bfloat16* go = static_cast<__nv_bfloat16*>(a.out) + gcol;
+    T* go = static_cast<T*>(a.out) + gcol;
     for (int c = tid; c < n_q * CPR; c += 128) {
         const int r = c / CPR, cc = c - r * CPR;
         const long long row = r == 0 ? b : base + r - 1;
@@ -759,27 +779,27 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
     }
 }
 
-template <int HD, int NSPLIT>
+template <int HD, int NSPLIT, class T>
 __global__ void __launch_bounds__(128)
 attention_mma_kernel(const AttnArgs a) {
     extern __shared__ __align__(16) uint8_t attn_sm[];
     const int b = blockIdx.x;
     const int n_items = a.off[b + 1] - a.off[b];
-    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, true>(a, attn_sm);   // S = 1 + n <= 8
-    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT>(a, attn_sm);         // S <= 16
-    else attention_mma_body<HD, true, NSPLIT>(a, attn_sm);
+    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm);   // S = 1 + n <= 8
+    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm);         // S <= 16
+    else attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm);
 }
 
 // the 16 heads of an outfit split over two CTAs
-template <int HD>
+template <int HD, class T>
 static int launch_attention_mma(const AttnArgs& a, cudaStream_t stream) {
     constexpr int kSplit = 2;
     constexpr int smem = (3 * kAttnMaxS + 1) * (16 * HD / kSplit + 8) * 2;
     static DeviceOnce configured;
     if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, kSplit>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, kSplit, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     }
-    attention_mma_kernel<HD, kSplit><<<dim3(a.batch, kSplit), 128, smem, stream>>>(a);
+    attention_mma_kernel<HD, kSplit, T><<<dim3(a.batch, kSplit), 128, smem, stream>>>(a);
     OFX_LAUNCH_CHECK();
     return OFX_OK;
 }
@@ -791,9 +811,9 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     if constexpr (sizeof(T) == 2) {
         if ((a.ldq % 8 == 0) && (a.ldk % 8 == 0) && (a.ldv % 8 == 0) && (a.ldo % 8 == 0)) {
             switch (head_dim) {
-                case 32: return launch_attention_mma<32>(a, stream);
-                case 64: return launch_attention_mma<64>(a, stream);
-                case 96: return launch_attention_mma<96>(a, stream);
+                case 32: return launch_attention_mma<32, T>(a, stream);
+                case 64: return launch_attention_mma<64, T>(a, stream);
+                case 96: return launch_attention_mma<96, T>(a, stream);
                 default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
             }
         }
@@ -811,6 +831,7 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
 }
 template int attention<float>(const AttnArgs&, int, cudaStream_t);
 template int attention<__nv_bfloat16>(const AttnArgs&, int, cudaStream_t);
+template int attention<__half>(const AttnArgs&, int, cudaStream_t);
 
 // ------------------------------------------------------------------ CP head: warp per outfit
 __global__ void __launch_bounds__(256)
@@ -900,5 +921,6 @@ int pack_matrix(const float* src, int rows, int cols, T* dst, int prow, int pcol
 }
 template int pack_matrix<float>(const float*, int, int, float*, int, int, cudaStream_t);
 template int pack_matrix<__nv_bfloat16>(const float*, int, int, __nv_bfloat16*, int, int, cudaStream_t);
+template int pack_matrix<__half>(const float*, int, int, __half*, int, int, cudaStream_t);
 
 }  // namespace ofx

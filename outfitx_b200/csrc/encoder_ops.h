@@ -42,11 +42,11 @@ struct FfnBlockArgs {
     int dm, fp;            // d_model, padded d_ffn
     const float* ln_w;     // norm2
     const float* ln_b;
-    const void* w1;        // (fp, dm) bf16
+    const void* w1;        // (fp, dm) bf16 / fp16 (ffn_block_bf16 / ffn_block_f16)
     const float* b1;       // (fp)
-    const void* w2;        // (dm, fp) bf16
+    const void* w2;        // (dm, fp), the same type
     const float* b2;       // (dm)
-    void* h_next = nullptr;        // optional (rows, dm) bf16: LayerNorm (lnn_w, lnn_b) of the updated x,
+    void* h_next = nullptr;        // optional (rows, dm), the same type: LayerNorm (lnn_w, lnn_b) of the updated x,
     const float* lnn_w = nullptr;  // i.e. norm1 of the next layer, emitted by the same kernel
     const float* lnn_b = nullptr;
     void* workspace = nullptr;     // at least ffn_block_workspace_bytes() (unused by the kernel)
@@ -55,6 +55,7 @@ struct FfnBlockArgs {
 bool ffn_block_supported(int dm, int fp);
 size_t ffn_block_workspace_bytes();
 int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream);
+int ffn_block_f16(const FfnBlockArgs& a, cudaStream_t stream);
 
 int scan_valid(const uint8_t* mask, int batch, int max_items, int* off, int* n_tok, cudaStream_t stream);
 int fuse_rows(const float* img, const float* txt, long long rows, int dpm, int mode, int normalize,

@@ -6,7 +6,7 @@
 // torch/nn/modules/transformer.py:950,980-982) as the reference builds it at
 // /root/reference/src/models/outfit_x.py:32-45 (activation = F.mish, d_ffn 2024 zero-padded to 2048).
 // The 2048-wide hidden activation never leaves the SM: it goes TMEM -> registers (bias + mish)
-// -> shared memory (bf16, UMMA operand layout) -> second GEMM.  HBM traffic per token is one
+// -> shared memory (bf16 or fp16, the operand type; UMMA operand layout) -> second GEMM.  HBM traffic per token is one
 // fp32 row in and one out (4 KB) instead of the 16 KB of LN + two separate GEMMs.
 //
 // Work decomposition: a CTA PAIR (cluster of 2, tcgen05 cta_group::2) owns 128 consecutive
@@ -74,7 +74,7 @@ struct Params {
     const float* b1;        // (n_chunks * 256) fp32, zero beyond d_ffn
     const float* b2;        // (512)
     int n_chunks;           // padded d_ffn / 256
-    __nv_bfloat16* h_next;  // optional (rows, 512) bf16: LayerNorm 1 of the NEXT layer applied to the new x
+    void* h_next;           // optional (rows, 512) 16-bit (the operand type): LayerNorm 1 of the NEXT layer applied to the new x
     const float* lnn_w;     // its affine terms
     const float* lnn_b;
     int debug;              // OFX_FFN_DEBUG bit mask, timing experiments only (results are WRONG with 1 / 256 / 512):
@@ -92,17 +92,14 @@ __device__ __forceinline__ float mish_fast(float x) {
     return x * n * r;
 }
 
-__device__ __forceinline__ uint32_t pack_bf16(float a, float b) {
-    __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-    return *reinterpret_cast<uint32_t*>(&v);
-}
-
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
     return v;
 }
 
+// T: the 16-bit operand type (__nv_bfloat16 or __half) of H, U, the weights and h_next
+template <class T>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NTHREADS, 1)
 ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constant__ CUtensorMap tm_w2,
                  const Params p) {
@@ -208,7 +205,7 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
         // stage, and the mbarrier poll for the NEXT stage is issued before this stage's MMAs so
         // that its ~100-cycle latency overlaps them.
         if (rank == 0) {
-            constexpr uint32_t idesc = umma_idesc_bf16(128, 256);
+            constexpr uint32_t idesc = umma_idesc_16<T>(128, 256);
             constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO, version, SW128
             const uint32_t h_lo = ((smem_u32(s_h) & 0x3FFFF) >> 4) | (1u << 16);
             const uint32_t u_lo = ((smem_u32(s_u) & 0x3FFFF) >> 4) | (1u << 16);
@@ -374,8 +371,8 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
                         float v2 = __uint_as_float(raw[8 * j + 4 * h + 2]) + bb.z;
                         float v3 = __uint_as_float(raw[8 * j + 4 * h + 3]) + bb.w;
                         if (!(p.debug & 1)) { v0 = mish_fast(v0); v1 = mish_fast(v1); v2 = mish_fast(v2); v3 = mish_fast(v3); }
-                        w[2 * h] = pack_bf16(v0, v1);
-                        w[2 * h + 1] = pack_bf16(v2, v3);
+                        w[2 * h] = pack2_16<T>(v0, v1);
+                        w[2 * h + 1] = pack2_16<T>(v2, v3);
                     }
                     *reinterpret_cast<uint4*>(dst + (((s * 4 + j) ^ sw) << 4)) = make_uint4(w[0], w[1], w[2], w[3]);
                 }
@@ -486,9 +483,9 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
 #undef EPROF_END
     } else if (warp >= LN_WARP0) {
         // ------------------------------------------------------------ LayerNorm warps
-        // (1) prologue: LN2 of this tile's x rows -> H (bf16, swizzled K-major operand layout);
+        // (1) prologue: LN2 of this tile's x rows -> H (16-bit, swizzled K-major operand layout);
         // (2) in the idle time that follows, LN1 of the NEXT layer on the PREVIOUS tile's freshly
-        //     written x rows -> h_next (bf16, row-major), re-read from L2: the separate LayerNorm
+        //     written x rows -> h_next (16-bit, row-major), re-read from L2: the separate LayerNorm
         //     kernel between two layers (one more read of x from HBM) disappears.
         const int lw = warp - LN_WARP0;
         const uint32_t hfull = mapa_shared(smem_u32(h_full), 0);
@@ -547,8 +544,8 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
                 norm4(v, gam, bet, [&](int u, int i, float y0, float y1, float y2, float y3) {
                     const long long row = row0 + rb + u;
                     if (row < n_rows)
-                        *reinterpret_cast<uint2*>(p.h_next + row * DM + i * 128 + lane * 4) =
-                            make_uint2(pack_bf16(y0, y1), pack_bf16(y2, y3));
+                        *reinterpret_cast<uint2*>(static_cast<T*>(p.h_next) + row * DM + i * 128 + lane * 4) =
+                            make_uint2(pack2_16<T>(y0, y1), pack2_16<T>(y2, y3));
                 });
             }
         };
@@ -592,7 +589,7 @@ ffn_block_kernel(const __grid_constant__ CUtensorMap tm_w1, const __grid_constan
                     const int c16 = (lane & 15) >> 1;
                     uint8_t* dst = s_h + kb * KBLK_BYTES + (r >> 3) * 1024 + (r & 7) * 128 +
                                    ((c16 ^ (r & 7)) << 4) + (lane & 1) * 8;
-                    *reinterpret_cast<uint2*>(dst) = make_uint2(pack_bf16(y0, y1), pack_bf16(y2, y3));
+                    *reinterpret_cast<uint2*>(dst) = make_uint2(pack2_16<T>(y0, y1), pack2_16<T>(y2, y3));
                 });
             }
             fence_proxy_async();
@@ -619,7 +616,8 @@ bool ffn_block_supported(int dm, int fp) { return dm == ffnb::DM && fp > 0 && fp
 // The kernel needs no scratch; the workspace the C ABI asks for (ofx_ffn_block_workspace_bytes) is a fixed 256 B.
 size_t ffn_block_workspace_bytes() { return 256; }
 
-int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream) {
+template <class T>
+static int ffn_block(const FfnBlockArgs& a, cudaStream_t stream) {
     using namespace ffnb;
     if (a.rows > 0 && ffn_block_supported(a.dm, a.fp) && (!a.workspace || a.workspace_bytes < ffn_block_workspace_bytes()))
         return fail(OFX_E_WORKSPACE, "ffn_block workspace %zu B < required %zu B", a.workspace_bytes, ffn_block_workspace_bytes());
@@ -635,25 +633,25 @@ int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream) {
 #else
     constexpr int debug = 0;
 #endif
+    // the 2-byte tensor map moves fp16 weights unchanged (common.h)
     OFX_TRY(make_tmap_bf16(&tm_w1, a.w1, static_cast<uint64_t>(a.fp), DM, DM, 128));
     OFX_TRY(make_tmap_bf16(&tm_w2, a.w2, DM, static_cast<uint64_t>(a.fp), a.fp, 128));
     static DeviceOnce configured;
     if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(ffn_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
+        OFX_CUDA(cudaFuncSetAttribute(ffn_block_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     }
     const int n_tiles = (a.rows + TILE - 1) / TILE;
     const int max_pairs = sm_count() / 2;
     const int pairs = n_tiles < max_pairs ? n_tiles : max_pairs;
     if (a.h_next && (!a.lnn_w || !a.lnn_b)) return fail(OFX_E_ARG, "ffn_block: h_next needs the next layer's LayerNorm terms");
-    Params p{a.x, a.rows, a.rows_dev, a.ln_w, a.ln_b, a.b1, a.b2, a.fp / CH,
-             static_cast<__nv_bfloat16*>(a.h_next), a.lnn_w, a.lnn_b, debug, nullptr};
+    Params p{a.x, a.rows, a.rows_dev, a.ln_w, a.ln_b, a.b1, a.b2, a.fp / CH, a.h_next, a.lnn_w, a.lnn_b, debug, nullptr};
     static long long* prof_dev = nullptr;
     if (debug & 8) {
         if (!prof_dev) OFX_CUDA(cudaMalloc(&prof_dev, 8 * 16 * 128));
         OFX_CUDA(cudaMemsetAsync(prof_dev, 0, 8 * 16 * 128, stream));
         p.prof = prof_dev;
     }
-    ffn_block_kernel<<<pairs * 2, NTHREADS, SMEM_BYTES, stream>>>(tm_w1, tm_w2, p);
+    ffn_block_kernel<T><<<pairs * 2, NTHREADS, SMEM_BYTES, stream>>>(tm_w1, tm_w2, p);
     OFX_LAUNCH_CHECK();
     if (debug & 8) {   // debug only: synchronous dump of the MMA warp's wait-cycle counters
         static int dumps = 0;
@@ -669,5 +667,8 @@ int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream) {
     }
     return OFX_OK;
 }
+
+int ffn_block_bf16(const FfnBlockArgs& a, cudaStream_t stream) { return ffn_block<__nv_bfloat16>(a, stream); }
+int ffn_block_f16(const FfnBlockArgs& a, cudaStream_t stream) { return ffn_block<__half>(a, stream); }
 
 }  // namespace ofx

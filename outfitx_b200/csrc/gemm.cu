@@ -1,5 +1,5 @@
 // Linear layers of the outfit encoder: C = A . W^T (+bias) (+mish) (+fp32 residual).
-//   bf16 mode: tcgen05 / TMEM / TMA pipeline (tc_pipeline.cuh) with the fused epilogue below
+//   bf16 / fp16 mode: tcgen05 / TMEM / TMA pipeline (tc_pipeline.cuh) with the fused epilogue below
 //   fp32 mode: the same pipeline on split-bf16 operands (gemm_f32_split, gemm.h)
 // Replaces the cuBLAS calls behind torch.nn.functional.linear in the reference's
 // nn.TransformerEncoderLayer (in_proj, out_proj, linear1+mish, linear2; SURVEY.md 2.1).
@@ -175,20 +175,23 @@ struct EpiLinear {
     }
 };
 
-// Epilogue of the bf16-output linear layers (QKV projection, linear1 + mish): TMEM -> registers
-// (bias, mish, bf16 pack) -> a per-warp 32-row x 128-byte staging tile in the 128B-swizzle layout
+// Epilogue of the 16-bit-output linear layers (QKV projection, linear1 + mish): TMEM -> registers
+// (bias, mish, bf16 / fp16 pack: T is also the operand type) -> a per-warp 32-row x 128-byte staging
+// tile in the 128B-swizzle layout
 // -> ONE TMA store per 64 output columns.  No per-thread global addressing and no transposing
 // read-back: ~2 instructions per output element instead of ~11, and a code footprint that fits
 // the instruction cache (the unrolled version stalled on instruction fetch).  Rows beyond the
 // tensor map's row count are clipped by the TMA unit; rows between the device-side row count
 // and the host bound land in caller scratch that nobody reads.
-template <int BN>
-struct EpiStoreBf16 {
-    struct alignas(64) Params {
-        CUtensorMap tm_c;      // (M, N) bf16 output, box = 64 columns x 32 rows, 128B swizzle
-        const float* bias;
-        int act_mish;
-    };
+struct alignas(64) EpiStoreParams {
+    CUtensorMap tm_c;      // (M, N) 16-bit output, box = 64 columns x 32 rows, 128B swizzle
+    const float* bias;
+    int act_mish;
+};
+template <int BN, class T>
+struct EpiStore16 {
+    using Operand = T;
+    using Params = EpiStoreParams;
     static constexpr int kWarps = 8;
     static constexpr int kSmemBytes = kWarps * 32 * 128;
     __device__ void begin(const Params&, const SchedGemm&, int, int, uint8_t*) {}
@@ -228,11 +231,8 @@ struct EpiStoreBf16 {
 #pragma unroll
                     for (int e = 0; e < 8; ++e) v[e] = mish_fast(v[e]);
                 }
-                uint4 u;
-                __nv_bfloat162 t0 = __floats2bfloat162_rn(v[0], v[1]), t1 = __floats2bfloat162_rn(v[2], v[3]);
-                __nv_bfloat162 t2 = __floats2bfloat162_rn(v[4], v[5]), t3 = __floats2bfloat162_rn(v[6], v[7]);
-                u.x = *reinterpret_cast<uint32_t*>(&t0); u.y = *reinterpret_cast<uint32_t*>(&t1);
-                u.z = *reinterpret_cast<uint32_t*>(&t2); u.w = *reinterpret_cast<uint32_t*>(&t3);
+                const uint4 u = make_uint4(pack2_16<T>(v[0], v[1]), pack2_16<T>(v[2], v[3]),
+                                           pack2_16<T>(v[4], v[5]), pack2_16<T>(v[6], v[7]));
                 *reinterpret_cast<uint4*>(my_row + ((j ^ sw) << 4)) = u;
             }
             fence_proxy_async();       // staging writes -> visible to the TMA unit
@@ -327,13 +327,21 @@ struct EpiResidualTma {
     }
 };
 
+// fp16 operands under an epilogue that only sees the fp32 accumulator and writes fp32
+template <class Epi>
+struct F16Operands : Epi {
+    using Operand = __half;
+};
+template <class T, class Epi>
+using WithOperands = std::conditional_t<std::is_same<T, __half>::value, F16Operands<Epi>, Epi>;
+
 template <int BN>
 static int make_epi_params(const GemmArgs& g, typename EpiLinear<BN>::Params* ep) {
     *ep = typename EpiLinear<BN>::Params{g.bias, g.residual, g.ldr, g.out, g.ldo, g.act_mish, g.out_f32};
     return OFX_OK;
 }
 template <int BN>
-static int make_epi_params(const GemmArgs& g, typename EpiStoreBf16<BN>::Params* ep) {
+static int make_epi_params(const GemmArgs& g, EpiStoreParams* ep) {
     OFX_TRY(make_tmap_bf16(&ep->tm_c, g.out, static_cast<uint64_t>(g.m), g.n, g.ldo, 32));
     ep->bias = g.bias;
     ep->act_mish = g.act_mish;
@@ -410,41 +418,51 @@ static int launch_tc(const GemmArgs& g, cudaStream_t stream) {
     return OFX_OK;
 }
 
-template <int BN>
+// T: the operand type, __nv_bfloat16 or __half (the caller has rejected 16-bit output with a residual for __half)
+template <int BN, class T>
 static int launch_tc_cl(const GemmArgs& g, cudaStream_t stream) {
     const long long m_tiles = (g.m + kBM - 1) / kBM;
     const int cl = m_tiles < 2 ? 1 : 2;  // CTA pairs; a single M tile: nothing to pair
-    // bf16 output without residual (QKV, linear1): TMA-store epilogue; otherwise the fp32 / residual one
-    const bool bf16_store = !g.out_f32 && !g.residual;
-    if (bf16_store) {
-        if (cl == 2) return launch_tc<BN, 2, EpiStoreBf16<BN>>(g, stream);
-        return launch_tc<BN, 1, EpiStoreBf16<BN>>(g, stream);
+    // 16-bit output without residual (QKV, linear1): TMA-store epilogue; otherwise the fp32 / residual one
+    const bool store16 = !g.out_f32 && !g.residual;
+    if (store16) {
+        if (cl == 2) return launch_tc<BN, 2, EpiStore16<BN, T>>(g, stream);
+        return launch_tc<BN, 1, EpiStore16<BN, T>>(g, stream);
     }
     // in-place fp32 residual update (out-proj, linear2): TMA load / add / TMA store epilogue
     const bool inplace = g.out_f32 && g.residual == g.out && g.ldr == g.ldo && !g.act_mish && g.ldo % 4 == 0;
     if (inplace) {
-        if (cl == 2) return launch_tc<BN, 2, EpiResidualTma<BN>>(g, stream);
-        return launch_tc<BN, 1, EpiResidualTma<BN>>(g, stream);
+        if (cl == 2) return launch_tc<BN, 2, WithOperands<T, EpiResidualTma<BN>>>(g, stream);
+        return launch_tc<BN, 1, WithOperands<T, EpiResidualTma<BN>>>(g, stream);
     }
-    if (cl == 2) return launch_tc<BN, 2, EpiLinear<BN>>(g, stream);
-    return launch_tc<BN, 1, EpiLinear<BN>>(g, stream);
+    if (cl == 2) return launch_tc<BN, 2, WithOperands<T, EpiLinear<BN>>>(g, stream);
+    return launch_tc<BN, 1, WithOperands<T, EpiLinear<BN>>>(g, stream);
 }
 
-int gemm_bf16(const GemmArgs& g, cudaStream_t stream) {
+template <class T>
+static int gemm_16(const GemmArgs& g, cudaStream_t stream) {
+    constexpr bool f16 = std::is_same<T, __half>::value;
+    const char* name = f16 ? "gemm_f16" : "gemm_bf16";
     if (g.m <= 0) return OFX_OK;
     if (g.n % 128 != 0 || g.k % kBK != 0 || g.n <= 0 || g.k <= 0)
-        return fail(OFX_E_SHAPE, "gemm_bf16: need N %% 128 == 0 and K %% 64 == 0 (N=%d K=%d)", g.n, g.k);
+        return fail(OFX_E_SHAPE, "%s: need N %% 128 == 0 and K %% 64 == 0 (N=%d K=%d)", name, g.n, g.k);
     if ((reinterpret_cast<uintptr_t>(g.a) | reinterpret_cast<uintptr_t>(g.w) |
          reinterpret_cast<uintptr_t>(g.out)) & 15)
-        return fail(OFX_E_ARG, "gemm_bf16: operands must be 16-byte aligned");
+        return fail(OFX_E_ARG, "%s: operands must be 16-byte aligned", name);
     if ((g.lda % 8) || (g.ldw % 8) || (g.ldo % 8) || (g.residual && (g.ldr % 4)))
-        return fail(OFX_E_ARG, "gemm_bf16: pitches must keep rows 16-byte aligned");
+        return fail(OFX_E_ARG, "%s: pitches must keep rows 16-byte aligned", name);
+    // the fp16 forms of the epilogues: fp16 output (TMA store, no residual) and fp32 output
+    if (f16 && (g.out_f32 == 2 || (!g.out_f32 && g.residual)))
+        return fail(OFX_E_ARG, "gemm_f16: a residual needs fp32 output (out_f32 = 1)");
     // BN = 256 halves the A re-reads; use 128 when 256 does not divide N or the grid would
     // leave most SMs idle.
     const long long tiles256 = static_cast<long long>((g.m + kBM - 1) / kBM) * (g.n / 256);
-    if (g.n % 256 == 0 && tiles256 >= sm_count()) return launch_tc_cl<256>(g, stream);
-    return launch_tc_cl<128>(g, stream);
+    if (g.n % 256 == 0 && tiles256 >= sm_count()) return launch_tc_cl<256, T>(g, stream);
+    return launch_tc_cl<128, T>(g, stream);
 }
+
+int gemm_bf16(const GemmArgs& g, cudaStream_t stream) { return gemm_16<__nv_bfloat16>(g, stream); }
+int gemm_f16(const GemmArgs& g, cudaStream_t stream) { return gemm_16<__half>(g, stream); }
 
 // -------------------------------------------------------------------------------------
 // fp32 operands as bf16 hi / lo pieces (gemm.h): one thread per 4 consecutive K elements

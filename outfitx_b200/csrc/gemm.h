@@ -5,7 +5,7 @@ namespace ofx {
 
 // C[m,n] = A[m,k] . W[n,k]^T  (+bias[n]) (mish) (+residual[m,n] fp32)
 struct GemmArgs {
-    const void* a;         // bf16 (tc) or fp32 (simt), row pitch lda elements
+    const void* a;         // bf16 or fp16, row pitch lda elements
     long long lda;
     const void* w;         // same element type as a, row pitch ldw
     long long ldw;
@@ -16,12 +16,14 @@ struct GemmArgs {
     int act_mish;
     const float* residual; // fp32, may alias out when out_f32
     long long ldr;
-    void* out;             // bf16 or fp32 (tc: out_f32 selects; simt: always fp32)
+    void* out;             // 16-bit (the operand type) or fp32: out_f32 selects
     long long ldo;
     int out_f32;
 };
 
 int gemm_bf16(const GemmArgs& g, cudaStream_t stream);
+// the same with fp16 a / w; a 16-bit output (out_f32 = 0) is fp16 and takes no residual
+int gemm_f16(const GemmArgs& g, cudaStream_t stream);
 
 // fp32 operands on the tensor cores: every fp32 value v is carried as two bf16 pieces hi = bf16(v), lo = bf16(v - hi)
 // (16 mantissa bits), laid out along K as three blocks so that an ordinary bf16 GEMM with K' = 3K evaluates

@@ -3,13 +3,28 @@
 // Nothing here is portable to other architectures on purpose.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
+
+#include <type_traits>
 
 namespace ofx {
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
+}
+
+// two fp32 values -> one 32-bit word of 16-bit operands (round to nearest even), T = __nv_bfloat16 or __half
+template <class T>
+__device__ __forceinline__ uint32_t pack2_16(float a, float b) {
+    if constexpr (std::is_same<T, __half>::value) {
+        __half2 v = __floats2half2_rn(a, b);
+        return *reinterpret_cast<uint32_t*>(&v);
+    } else {
+        __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+        return *reinterpret_cast<uint32_t*>(&v);
+    }
 }
 
 __device__ __forceinline__ bool elect_one() {
@@ -173,7 +188,7 @@ __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols)
                  : "memory");
 }
-// D[tmem] (+)= A[smem] * B[smem]^T, bf16 inputs, fp32 accumulate; issued by ONE thread
+// D[tmem] (+)= A[smem] * B[smem]^T, bf16 or fp16 inputs (idesc), fp32 accumulate; issued by ONE thread
 __device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc,
                                           uint32_t idesc, uint32_t accumulate) {
     asm volatile(
@@ -372,6 +387,15 @@ __device__ __forceinline__ uint64_t umma_desc_k_sw128(uint32_t smem_addr) {
 // a/b_major=K (0) [15],[16], N>>3 [17,23), M>>4 [24,29).
 __host__ __device__ constexpr uint32_t umma_idesc_bf16(uint32_t m, uint32_t n) {
     return (1u << 4) | (1u << 7) | (1u << 10) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// The same for FP16 x FP16 -> FP32: a/b_format = F16 (0)
+__host__ __device__ constexpr uint32_t umma_idesc_f16(uint32_t m, uint32_t n) {
+    return (1u << 4) | ((n >> 3) << 17) | ((m >> 4) << 24);
+}
+// ... chosen by the 16-bit operand type (__nv_bfloat16 or __half)
+template <class T>
+__host__ __device__ constexpr uint32_t umma_idesc_16(uint32_t m, uint32_t n) {
+    return std::is_same<T, __half>::value ? umma_idesc_f16(m, n) : umma_idesc_bf16(m, n);
 }
 
 }  // namespace ofx

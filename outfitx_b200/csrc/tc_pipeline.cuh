@@ -70,8 +70,14 @@ constexpr int tc_smem_bytes() {
 //                        int ewarp /*0..kWarps-1: quarter = ewarp & 3, column group = ewarp >> 2*/,
 //                        int lane, uint8_t* epi_smem);
 //   (an object per epilogue thread: state such as running top-k thresholds lives in it)
+//   using Operand = __half;        optional: fp16 A and B (kind::f16 with F16 inputs); bf16 without it
 template <class Epi>
 constexpr int tc_threads() { return 128 + 32 * Epi::kWarps; }
+
+template <class Epi, class = void>
+struct TcOperand { using type = __nv_bfloat16; };
+template <class Epi>
+struct TcOperand<Epi, std::void_t<typename Epi::Operand>> { using type = typename Epi::Operand; };
 
 // Debug instrumentation (OFX_TC_PROF=1, gemm.cu): per-CTA cycle counters of the MMA warp
 // {total, wait smem-full, wait tmem-empty} and of epilogue warp 0 {total, wait tmem-full}.
@@ -167,7 +173,7 @@ tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUte
         // back to back.  A lane-0-only loop costs ~20 issue slots per MMA in address traffic
         // between the vector and uniform register files.
         if (!kPair || crank == 0) {
-            constexpr uint32_t idesc = umma_idesc_bf16(kPair ? 2 * kBM : kBM, BN);
+            constexpr uint32_t idesc = umma_idesc_16<typename TcOperand<Epi>::type>(kPair ? 2 * kBM : kBM, BN);
             constexpr uint32_t kDescHi = (1024u >> 4) | (1u << 14) | (2u << 29);  // SBO, version, SW128
             const uint32_t a_lo0 = ((smem_u32(s_a) & 0x3FFFF) >> 4) | (1u << 16);
             const uint32_t b_lo0 = ((smem_u32(s_b) & 0x3FFFF) >> 4) | (1u << 16);

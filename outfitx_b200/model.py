@@ -27,7 +27,7 @@ from .configs import OutfitXConfig
 from .datatypes import (OutfitCompatibilityPredictionTask, OutfitComplementaryItemRetrievalTask,
                         OutfitFillInTheBlankTask, OutfitPrecomputeEmbeddingTask)
 
-_PRECISIONS = {"bf16": _lib.PREC_BF16, "fp32": _lib.PREC_FP32}
+_PRECISIONS = {"bf16": _lib.PREC_BF16, "fp32": _lib.PREC_FP32, "fp16": _lib.PREC_FP16}
 _FUSE = {"concat": _lib.FUSE_CONCAT, "mean": _lib.FUSE_MEAN}
 
 
@@ -88,7 +88,7 @@ class OutfitX(nn.Module):
         super().__init__()
         self.cfg = cfg if cfg is not None else OutfitXConfig()
         if precision not in _PRECISIONS:
-            raise ValueError(f"precision must be 'bf16' or 'fp32', got {precision!r}")
+            raise ValueError(f"precision must be 'bf16', 'fp16' or 'fp32', got {precision!r}")
         self.precision = precision
         t = self.cfg.transformer
         if str(getattr(t.activation, "__name__", t.activation)) != "mish":
