@@ -68,7 +68,8 @@ typedef struct ofx_shape {
     int32_t n_head;    /* 16                                                                */
     int32_t n_layers;  /* 6                                                                 */
     int32_t d_ffn;     /* 2024 (zero-padded to a multiple of 64 inside the packed weights)  */
-    int32_t max_items; /* 16 (outfit_x_config.py:13)                                        */
+    int32_t max_items; /* item slots per outfit, 1..64; the reference default is 16         */
+                       /* (max_length, outfit_x_config.py:13)                               */
     int32_t precision; /* OFX_PREC_*                                                        */
 } ofx_shape;
 
@@ -122,19 +123,19 @@ OFX_API int ofx_fuse(const float* img, const float* txt, int64_t rows, int32_t d
  * caller idioms sigmoid (compatibility_prediction_trainer.py:408) and FITB cdist->argmin
  * (fill_in_the_blank_trainer.py:50-53).
  *
- * Inputs: either `emb` (B,16,Dm) fused fp32 embeddings (the reference's outfit_embedding), or
- * raw modalities img/txt (B,16,dpm) fused on the fly (fuse_mode, normalize) with emb == NULL.
- * mask (B,16) bytes, non-zero = padding (outfit_mask, True = pad).  Valid items may sit in
- * any slot; padded slots are never read. */
+ * Inputs: either `emb` (B, max_items, Dm) fused fp32 embeddings (the reference's outfit_embedding),
+ * or raw modalities img/txt (B, max_items, dpm) fused on the fly (fuse_mode, normalize) with
+ * emb == NULL.  mask (B, max_items) bytes, non-zero = padding (outfit_mask, True = pad).  Valid
+ * items may sit in any slot; padded slots are never read. */
 typedef struct ofx_forward_args {
     int32_t task;          /* OFX_TASK_*                                              */
     int32_t batch;         /* B outfits                                               */
-    const float* emb;      /* (B,16,Dm) or NULL                                       */
-    const float* img;      /* (B,16,dpm) or NULL                                      */
-    const float* txt;      /* (B,16,dpm) or NULL                                      */
+    const float* emb;      /* (B, max_items, Dm) or NULL                              */
+    const float* img;      /* (B, max_items, dpm) or NULL                             */
+    const float* txt;      /* (B, max_items, dpm) or NULL                             */
     int32_t fuse_mode;     /* OFX_FUSE_* (used with img/txt)                          */
     int32_t normalize;     /* L2-normalise each modality first (reference: yes)       */
-    const uint8_t* mask;   /* (B,16)                                                  */
+    const uint8_t* mask;   /* (B, max_items)                                          */
     const float* text;     /* CIR: target_item_text_embedding (B, Dm/2)               */
     float* logits;         /* CP out: (B) logits  (== reference (B,1))                */
     float* probs;          /* CP out: (B) sigmoid(logit), may be NULL                 */

@@ -29,7 +29,7 @@ static int check_shape(const ofx_shape* s) {
     if (s->n_layers < 1 || s->n_layers > 64) return fail(OFX_E_SHAPE, "n_layers %d", s->n_layers);
     if (s->d_ffn < 1 || s->d_ffn > 16384) return fail(OFX_E_SHAPE, "d_ffn %d", s->d_ffn);
     if (s->d_embed < 128 || s->d_embed % 128) return fail(OFX_E_SHAPE, "d_embed %d must be a multiple of 128", s->d_embed);
-    if (s->max_items < 1 || s->max_items > 16) return fail(OFX_E_SHAPE, "max_items %d not in [1,16]", s->max_items);
+    if (s->max_items < 1 || s->max_items > 64) return fail(OFX_E_SHAPE, "max_items %d not in [1,64]", s->max_items);
     if (s->precision != OFX_PREC_BF16 && s->precision != OFX_PREC_FP32 && s->precision != OFX_PREC_FP16)
         return fail(OFX_E_ARG, "precision %d not in {0 (bf16), 1 (fp32), 2 (fp16)}", s->precision);
     return OFX_OK;

@@ -1,6 +1,6 @@
 // Non-GEMM pieces of the outfit encoder, fused per row / per outfit:
 //   fuse / assemble (normalise + concat|mean + prefix token + drop padded slots),
-//   LayerNorm, the <=17-token masked attention, CP head (+sigmoid), FITB distances.
+//   LayerNorm, the masked attention over up to 65 tokens, CP head (+sigmoid), FITB distances.
 // Reference arithmetic: SURVEY.md App. A, i.e. torch.nn.TransformerEncoderLayer's pre-LN
 // slow path as driven by /root/reference/src/models/outfit_x.py:120-172.
 //
@@ -417,7 +417,80 @@ template int cast_rows<float>(const float*, long long, float*, cudaStream_t);
 template int cast_rows<__nv_bfloat16>(const float*, long long, __nv_bfloat16*, cudaStream_t);
 template int cast_rows<__half>(const float*, long long, __half*, cudaStream_t);
 
-// ------------------------------------------------------------------ attention
+// ------------------------------------------------------------------ attention, CUDA cores
+// One (token row, head) of an outfit with S > 17 tokens: one pass over groups of 4 keys with a running
+// maximum and sum (online softmax); the output accumulator is rescaled whenever the maximum grows.
+template <int HD, class T>
+__device__ __forceinline__ void attention_row_online(const AttnArgs& a, int b, int base, int S, const T* qp,
+                                                     const T* kp, const T* vp, T* op) {
+    constexpr int NP = HD / 32;
+    float q[NP][8];
+#pragma unroll
+    for (int p = 0; p < NP; ++p) load8(qp + 32 * p, q[p]);
+    const float scale = rsqrtf(static_cast<float>(HD));
+    float mx = -INFINITY, den = 0.f;
+    float o[NP][8];
+#pragma unroll
+    for (int p = 0; p < NP; ++p)
+#pragma unroll
+        for (int e = 0; e < 8; ++e) o[p][e] = 0.f;
+#pragma unroll 1
+    for (int j0 = 0; j0 < S; j0 += 4) {
+        float t[4][NP][8];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const long long r = (j == 0 || j >= S) ? b : base + j - 1;
+#pragma unroll
+            for (int p = 0; p < NP; ++p) load8(kp + r * a.ldk + 32 * p, t[u][p]);
+        }
+        float sc[4];
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            float acc = 0.f;
+#pragma unroll
+            for (int p = 0; p < NP; ++p)
+#pragma unroll
+                for (int e = 0; e < 8; ++e) acc = fmaf(q[p][e], t[u][p][e], acc);
+            acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+            acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+            sc[u] = j0 + u < S ? acc * scale : -INFINITY;
+        }
+        const float m_new = fmaxf(mx, fmaxf(fmaxf(sc[0], sc[1]), fmaxf(sc[2], sc[3])));   // finite: key 0 is valid
+        const float corr = sizeof(T) == 4 ? expf(mx - m_new) : __expf(mx - m_new);      // exp(-inf) = 0 at j0 = 0
+        mx = m_new;
+        den *= corr;
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            sc[u] = sizeof(T) == 4 ? expf(sc[u] - mx) : __expf(sc[u] - mx);
+            den += sc[u];
+        }
+#pragma unroll
+        for (int u = 0; u < 4; ++u) {
+            const int j = j0 + u;
+            const long long r = (j == 0 || j >= S) ? b : base + j - 1;
+#pragma unroll
+            for (int p = 0; p < NP; ++p) load8(vp + r * a.ldv + 32 * p, t[u][p]);
+        }
+#pragma unroll
+        for (int p = 0; p < NP; ++p)
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                float acc = o[p][e] * corr;
+#pragma unroll
+                for (int u = 0; u < 4; ++u) acc = fmaf(sc[u], t[u][p][e], acc);
+                o[p][e] = acc;
+            }
+    }
+    const float inv = 1.f / den;
+#pragma unroll
+    for (int p = 0; p < NP; ++p) {
+#pragma unroll
+        for (int e = 0; e < 8; ++e) o[p][e] *= inv;
+        store8(op + 32 * p, o[p]);
+    }
+}
+
 // Four consecutive lanes serve one (token row, head): lane `sub` owns dims {32p + 8 sub .. +8}
 // of the head for every 32-dim piece p, so each warp-wide 16-byte load covers contiguous 64-byte
 // runs (8 heads x 4 lanes = 512 contiguous bytes of one token row at head_dim 32) -- fully
@@ -426,7 +499,10 @@ template int cast_rows<__half>(const float*, long long, __half*, cudaStream_t);
 // Softmax runs over the outfit's S = 1 + n valid tokens only: the dropped pads are exactly the
 // -inf keys of the reference's float key-padding mask.
 // row0_only: the pruned last layer (queries = the B prefix tokens, from a separate buffer).
-template <int HD, class T>
+// LONG = false: every outfit of the launch has S <= 17 tokens.  LONG = true (max_s > 17): rows of outfits with
+// more tokens take the online softmax of attention_row_online; the others run the same two-pass code as with
+// LONG = false.  All lanes of a row share S, so the branch is warp-uniform.
+template <int HD, class T, bool LONG>
 __global__ void __launch_bounds__(256)
 attention_kernel(AttnArgs a) {
     constexpr int NP = HD / 32;  // 8-dim pieces per lane
@@ -443,6 +519,12 @@ attention_kernel(AttnArgs a) {
     const T* vp = static_cast<const T*>(a.v) + col;
     const T* qp = static_cast<const T*>(a.q) + static_cast<long long>(row) * a.ldq + col;
     T* op = static_cast<T*>(a.out) + static_cast<long long>(row) * a.ldo + col;
+    if constexpr (LONG) {
+        if (S > 17) {
+            attention_row_online<HD, T>(a, b, base, S, qp, kp, vp, op);
+            return;
+        }
+    }
 
     float q[NP][8];
 #pragma unroll
@@ -582,8 +664,9 @@ constexpr int kAttnMaxS = 17;
 // SMALL: S <= 8 tokens (40 % of the outfits at n ~ U{2..16}): only query rows 0..7 (h = 0) and the first
 // 8-key n-tile exist, so the second score MMA, half of the softmax and half of the output stores are skipped.
 // T: the 16-bit type of q / K / V, P and the output (__nv_bfloat16 or __half)
+// cap: rows reserved for each of q, K and V in shared memory (kAttnMaxS, or max_s in the long kernel)
 template <int HD, bool BIG, int NSPLIT, class T, bool SMALL = false>
-__device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* sm) {
+__device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* sm, int cap) {
     static_assert(!(BIG && SMALL), "one or the other");
     constexpr int MT = BIG ? 2 : 1, KT = BIG ? 2 : 1;
     constexpr int NH = SMALL ? 1 : 2;            // row halves (g, g + 8) in use
@@ -594,9 +677,9 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
     constexpr int STRIDE = (DM + 8) * 2;     // bytes per shared-memory row
     constexpr int KS = HD / 16;              // k-steps over the head dimension
     uint8_t* s_q = sm;
-    uint8_t* s_k = sm + kAttnMaxS * STRIDE;
-    uint8_t* s_v = s_k + kAttnMaxS * STRIDE;
-    uint8_t* s_z = s_v + kAttnMaxS * STRIDE;   // one zero row
+    uint8_t* s_k = sm + cap * STRIDE;
+    uint8_t* s_v = s_k + cap * STRIDE;
+    uint8_t* s_z = s_v + cap * STRIDE;   // one zero row
     const int b = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int base = a.batch + a.off[b];
@@ -785,9 +868,211 @@ attention_mma_kernel(const AttnArgs a) {
     extern __shared__ __align__(16) uint8_t attn_sm[];
     const int b = blockIdx.x;
     const int n_items = a.off[b + 1] - a.off[b];
-    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm);   // S = 1 + n <= 8
-    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm);         // S <= 16
-    else attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm);
+    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm, kAttnMaxS);   // S = 1 + n <= 8
+    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm, kAttnMaxS);         // S <= 16
+    else attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm, kAttnMaxS);
+}
+
+// ------------------------------------------------------------------ attention, bf16 / fp16, outfits of 17..64 items
+// S > 17 tokens (up to 65): the gather-once layout of attention_mma_body with max_s rows per region.  Each warp
+// walks the up to five 16-row query tiles of its heads one at a time; for each it scores all (up to five) 16-key
+// tiles into registers (10 n8-tiles), runs the masked warp-shuffle softmax over the whole row and accumulates
+// P.V through ldmatrix.trans.  Rows >= S read the zero row, so padded keys contribute exactly 0; under row0_only
+// only query tile 0 exists.
+constexpr int kAttnLongMaxS = 65;
+template <int HD, int NSPLIT, class T>
+__device__ __forceinline__ void attention_mma_long_body(const AttnArgs& a, uint8_t* sm, int cap) {
+    constexpr int KT = (kAttnLongMaxS + 15) / 16;   // 16-key tiles
+    constexpr int DM = 16 * HD / NSPLIT;
+    constexpr int HPW = 4 / NSPLIT;
+    constexpr int CPR = DM / 8;
+    constexpr int STRIDE = (DM + 8) * 2;
+    constexpr int KS = HD / 16;
+    uint8_t* s_q = sm;
+    uint8_t* s_k = sm + cap * STRIDE;
+    uint8_t* s_v = s_k + cap * STRIDE;
+    uint8_t* s_z = s_v + cap * STRIDE;
+    const int b = blockIdx.x;
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int base = a.batch + a.off[b];
+    const int S = min(1 + (a.off[b + 1] - a.off[b]), cap);
+    const int n_q = a.row0_only ? 1 : S;
+    const int gcol = static_cast<int>(blockIdx.y) * DM;
+    const T* gq = static_cast<const T*>(a.q) + gcol;
+    const T* gk = static_cast<const T*>(a.k) + gcol;
+    const T* gv = static_cast<const T*>(a.v) + gcol;
+
+    for (int i = tid; i < STRIDE / 16; i += 128) reinterpret_cast<uint4*>(s_z)[i] = make_uint4(0, 0, 0, 0);
+    auto load_rows = [&](const T* g, long long ld, uint8_t* dst, int n_rows) {
+        int j = tid / CPR, cc = tid - j * CPR;
+        while (j < n_rows) {
+            const long long row = j == 0 ? b : base + j - 1;
+            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(static_cast<uint32_t>(
+                             __cvta_generic_to_shared(dst + j * STRIDE + cc * 16))),
+                         "l"(g + row * ld + cc * 8)
+                         : "memory");
+            cc += 128;
+            while (cc >= CPR) { cc -= CPR; ++j; }
+        }
+    };
+    load_rows(gk, a.ldk, s_k, S);
+    load_rows(gv, a.ldv, s_v, S);
+    load_rows(gq, a.ldq, s_q, n_q);
+    asm volatile("cp.async.commit_group;" ::: "memory");
+    asm volatile("cp.async.wait_group 0;" ::: "memory");
+    __syncthreads();
+
+    const uint32_t q_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_q));
+    const uint32_t k_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_k));
+    const uint32_t v_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_v));
+    const uint32_t z_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_z));
+    const int n_mt = (n_q + 15) / 16;
+    const int n_kt = (S + 15) / 16;
+    const int g = lane >> 2, t4 = lane & 3;
+    const int a_row = (lane & 7) + 8 * ((lane >> 3) & 1), a_col = 8 * (lane >> 4);
+    const int b_row = (lane & 7) + 8 * (lane >> 4), b_col = 8 * ((lane >> 3) & 1);
+    const float sl2 = rsqrtf(static_cast<float>(HD)) * 1.4426950408889634f;
+    uint32_t kvalid = 0;      // bit nt*2+e: key nt*8 + 2*t4 + e exists
+#pragma unroll
+    for (int nt = 0; nt < 2 * KT; ++nt)
+#pragma unroll
+        for (int e = 0; e < 2; ++e) kvalid |= (nt * 8 + 2 * t4 + e < S ? 1u : 0u) << (nt * 2 + e);
+
+#pragma unroll 1
+    for (int hh = 0; hh < HPW; ++hh) {
+        const int col0 = (warp * HPW + hh) * HD;
+#pragma unroll 1
+        for (int mt = 0; mt < n_mt; ++mt) {
+            float sc[2 * KT][4];
+#pragma unroll
+            for (int nt = 0; nt < 2 * KT; ++nt)
+#pragma unroll
+                for (int e = 0; e < 4; ++e) sc[nt][e] = 0.f;
+#pragma unroll
+            for (int ks = 0; ks < KS; ++ks) {
+                uint32_t qa[4];
+                const int rq = mt * 16 + a_row;
+                ldsm_x4(qa, (rq < n_q ? q_s + rq * STRIDE : z_s) + (col0 + ks * 16 + a_col) * 2);
+#pragma unroll
+                for (int kt = 0; kt < KT; ++kt) {
+                    if (kt < n_kt) {
+                        uint32_t kb[4];
+                        const int r = kt * 16 + b_row;
+                        ldsm_x4(kb, (r < S ? k_s + r * STRIDE : z_s) + (col0 + ks * 16 + b_col) * 2);
+                        mma_16816<T>(sc[2 * kt], qa, kb[0], kb[1]);
+                        mma_16816<T>(sc[2 * kt + 1], qa, kb[2], kb[3]);
+                    }
+                }
+            }
+            // masked softmax over the whole row (rows g and g + 8 of the tile)
+            float inv[2];
+#pragma unroll
+            for (int h = 0; h < 2; ++h) {
+                float mx = -INFINITY;
+#pragma unroll
+                for (int nt = 0; nt < 2 * KT; ++nt)
+#pragma unroll
+                    for (int e = 0; e < 2; ++e) {
+                        const float v = (kvalid >> (nt * 2 + e)) & 1u ? sc[nt][2 * h + e] * sl2 : -INFINITY;
+                        sc[nt][2 * h + e] = v;
+                        mx = fmaxf(mx, v);
+                    }
+                mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
+                mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
+                float sum = 0.f;
+#pragma unroll
+                for (int nt = 0; nt < 2 * KT; ++nt)
+#pragma unroll
+                    for (int e = 0; e < 2; ++e) {
+                        const float pz = ex2_fast(sc[nt][2 * h + e] - mx);   // key 0 is always valid: mx finite
+                        sc[nt][2 * h + e] = pz;
+                        sum += pz;
+                    }
+                sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+                sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+                inv[h] = 1.f / sum;
+            }
+            uint32_t pa[KT][4];
+#pragma unroll
+            for (int kt = 0; kt < KT; ++kt) {
+                pa[kt][0] = pack2_16<T>(sc[2 * kt][0], sc[2 * kt][1]);
+                pa[kt][1] = pack2_16<T>(sc[2 * kt][2], sc[2 * kt][3]);
+                pa[kt][2] = pack2_16<T>(sc[2 * kt + 1][0], sc[2 * kt + 1][1]);
+                pa[kt][3] = pack2_16<T>(sc[2 * kt + 1][2], sc[2 * kt + 1][3]);
+            }
+            // out = P . V, 16 head dims at a time, into this tile's (dead) q rows of the head
+#pragma unroll
+            for (int dp = 0; dp < KS; ++dp) {
+                float o[2][4];
+#pragma unroll
+                for (int x = 0; x < 2; ++x)
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) o[x][e] = 0.f;
+#pragma unroll
+                for (int kt = 0; kt < KT; ++kt) {
+                    if (kt < n_kt) {
+                        uint32_t vb[4];
+                        const int r = kt * 16 + a_row;
+                        ldsm_x4_trans(vb, (r < S ? v_s + r * STRIDE : z_s) + (col0 + dp * 16 + a_col) * 2);
+                        mma_16816<T>(o[0], pa[kt], vb[0], vb[1]);
+                        mma_16816<T>(o[1], pa[kt], vb[2], vb[3]);
+                    }
+                }
+                __syncwarp();
+#pragma unroll
+                for (int h = 0; h < 2; ++h) {
+                    const int r = mt * 16 + g + 8 * h;
+                    if (r < n_q) {
+#pragma unroll
+                        for (int x = 0; x < 2; ++x)
+                            *reinterpret_cast<uint32_t*>(s_q + r * STRIDE + (col0 + dp * 16 + x * 8 + 2 * t4) * 2) =
+                                pack2_16<T>(o[x][2 * h] * inv[h], o[x][2 * h + 1] * inv[h]);
+                    }
+                }
+            }
+        }
+    }
+    __syncthreads();
+    T* go = static_cast<T*>(a.out) + gcol;
+    for (int c = tid; c < n_q * CPR; c += 128) {
+        const int r = c / CPR, cc = c - r * CPR;
+        const long long row = r == 0 ? b : base + r - 1;
+        *reinterpret_cast<uint4*>(go + row * a.ldo + cc * 8) = *reinterpret_cast<const uint4*>(s_q + r * STRIDE + cc * 16);
+    }
+}
+
+// max_s > 17: outfits of <= 16 items take the bodies of attention_mma_kernel (same arithmetic, rows at max_s
+// spacing), longer ones the long body
+template <int HD, int NSPLIT, class T>
+__global__ void __launch_bounds__(128)
+attention_mma_long_kernel(const AttnArgs a) {
+    extern __shared__ __align__(16) uint8_t attn_sm[];
+    const int b = blockIdx.x;
+    const int n_items = a.off[b + 1] - a.off[b];
+    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm, a.max_s);
+    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm, a.max_s);
+    else if (n_items == 16) attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm, a.max_s);
+    else attention_mma_long_body<HD, NSPLIT, T>(a, attn_sm, a.max_s);
+}
+
+// Shared memory is (3 max_s + 1) rows of (16 HD / NSPLIT + 8) x 2 bytes: at max_s = 65 the head split that keeps
+// two CTAs per SM is 2 at head_dim 32 (103 KB) and 4 at 64 (103 KB); at 96 a split of 4 (154 KB) is the least
+// that fits at all (2 needs 304 KB).
+template <int HD> constexpr int attn_long_split() { return HD == 32 ? 2 : 4; }
+template <int HD>
+constexpr int attn_long_smem(int max_s) { return (3 * max_s + 1) * (16 * HD / attn_long_split<HD>() + 8) * 2; }
+
+template <int HD, class T>
+static int launch_attention_mma_long(const AttnArgs& a, cudaStream_t stream) {
+    constexpr int kSplit = attn_long_split<HD>();
+    static DeviceOnce configured;
+    if (configured.need()) {
+        OFX_CUDA(cudaFuncSetAttribute(attention_mma_long_kernel<HD, kSplit, T>,
+                                      cudaFuncAttributeMaxDynamicSharedMemorySize, attn_long_smem<HD>(kAttnLongMaxS)));
+    }
+    attention_mma_long_kernel<HD, kSplit, T><<<dim3(a.batch, kSplit), 128, attn_long_smem<HD>(a.max_s), stream>>>(a);
+    OFX_LAUNCH_CHECK();
+    return OFX_OK;
 }
 
 // the 16 heads of an outfit split over two CTAs
@@ -808,8 +1093,18 @@ template <class T>
 int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     if (a.batch <= 0) return OFX_OK;
     if (a.n_head != 16) return fail(OFX_E_SHAPE, "attention: n_head %d != 16", a.n_head);
+    if (a.max_s < 2 || a.max_s > kAttnLongMaxS) return fail(OFX_E_SHAPE, "attention: max_s %d not in [2,%d]", a.max_s, kAttnLongMaxS);
+    const bool long_s = a.max_s > kAttnMaxS;     // some outfit may hold more than 16 items
     if constexpr (sizeof(T) == 2) {
         if ((a.ldq % 8 == 0) && (a.ldk % 8 == 0) && (a.ldv % 8 == 0) && (a.ldo % 8 == 0)) {
+            if (long_s) {
+                switch (head_dim) {
+                    case 32: return launch_attention_mma_long<32, T>(a, stream);
+                    case 64: return launch_attention_mma_long<64, T>(a, stream);
+                    case 96: return launch_attention_mma_long<96, T>(a, stream);
+                    default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
+                }
+            }
             switch (head_dim) {
                 case 32: return launch_attention_mma<32, T>(a, stream);
                 case 64: return launch_attention_mma<64, T>(a, stream);
@@ -820,11 +1115,19 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     }
     const int rows = a.row0_only ? a.batch : a.max_rows;
     const unsigned grid = static_cast<unsigned>((rows + 3) / 4);
-    switch (head_dim) {
-        case 32: attention_kernel<32, T><<<grid, 256, 0, stream>>>(a); break;
-        case 64: attention_kernel<64, T><<<grid, 256, 0, stream>>>(a); break;
-        case 96: attention_kernel<96, T><<<grid, 256, 0, stream>>>(a); break;
-        default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
+    if (head_dim != 32 && head_dim != 64 && head_dim != 96) return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
+    if (long_s) {
+        switch (head_dim) {
+            case 32: attention_kernel<32, T, true><<<grid, 256, 0, stream>>>(a); break;
+            case 64: attention_kernel<64, T, true><<<grid, 256, 0, stream>>>(a); break;
+            case 96: attention_kernel<96, T, true><<<grid, 256, 0, stream>>>(a); break;
+        }
+    } else {
+        switch (head_dim) {
+            case 32: attention_kernel<32, T, false><<<grid, 256, 0, stream>>>(a); break;
+            case 64: attention_kernel<64, T, false><<<grid, 256, 0, stream>>>(a); break;
+            case 96: attention_kernel<96, T, false><<<grid, 256, 0, stream>>>(a); break;
+        }
     }
     OFX_LAUNCH_CHECK();
     return OFX_OK;

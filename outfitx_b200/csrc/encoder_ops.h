@@ -5,11 +5,11 @@ namespace ofx {
 
 struct AssembleArgs {
     int task, batch, max_items;
-    const float* emb;      // (B,16,Dm) fused, or null
-    const float* img;      // (B,16,dpm)
+    const float* emb;      // (B,max_items,Dm) fused, or null
+    const float* img;      // (B,max_items,dpm)
     const float* txt;
     int dpm, fuse_mode, normalize;
-    const uint8_t* mask;   // (B,16) non-zero = pad
+    const uint8_t* mask;   // (B,max_items) non-zero = pad
     const int* off;        // (B+1) exclusive prefix of valid counts
     const float* outfit_token;  // (Dm)
     const float* target_img;    // (Dm/2)
@@ -23,7 +23,7 @@ struct AssembleArgs {
 
 struct AttnArgs {
     int batch, n_head, row0_only;
-    int max_s;             // upper bound of tokens per outfit (1 + max_items)
+    int max_s;             // upper bound of tokens per outfit (1 + max_items, <= 65)
     int max_rows;          // host upper bound of token rows
     const int* n_tok;      // device token-row count
     const int* owner;      // token row -> outfit (rows >= batch)

@@ -284,8 +284,8 @@ class OutfitX(nn.Module):
                 raise ValueError(f"outfit_embedding must be (B, L, {d}), got {tuple(emb.shape)}")
             B, n_items = emb.shape[0], emb.shape[1]
             dev = emb.device
-        if n_items < 1 or n_items > 16:
-            raise ValueError(f"outfits hold 1..16 item slots (max_length {self.cfg.max_length}), got {n_items}")
+        if n_items < 1 or n_items > 64:
+            raise ValueError(f"outfits hold 1..64 item slots (max_length {self.cfg.max_length}), got {n_items}")
         shape.max_items = n_items
         if mask is None or tuple(mask.shape) != (B, n_items):
             raise ValueError(f"outfit_mask must be (B, L) = ({B}, {n_items}), True = padding")

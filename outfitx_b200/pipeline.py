@@ -41,6 +41,7 @@ class HostScoringPipeline:
         self.use_graphs = use_graphs
         self.tail_min = chunk      # smallest chunk of a tapered tail (see _plan); = chunk: uniform chunks
         self._graphs = {}
+        self._graph_width = None   # max_items of the captured graphs: their staging buffers are sized by it
         if chunk < 1:
             raise ValueError("chunk must be >= 1")
         self.model, self.chunk = model, chunk
@@ -159,8 +160,11 @@ class HostScoringPipeline:
                      out: Optional[Dict[str, torch.Tensor]] = None, max_items: int = 16) -> Dict[str, torch.Tensor]:
         """As ``score`` for a HOST batch in the packed layout: ``image_rows`` / ``text_rows``
         ``(sum(lengths), dim_per_modality)`` hold the valid items of outfit 0, then outfit 1, ...;
-        ``lengths (B,)`` integers in ``[0, max_items]`` (a collate truncates to ``max_items`` = 16 first,
-        ``outfit_x_base_processor.py:57-81``).  Bit-identical to ``score`` on the padded tensors."""
+        ``lengths (B,)`` integers in ``[0, max_items]`` (a collate truncates to ``max_items`` first, 16 by default,
+        ``outfit_x_base_processor.py:57-81``); ``max_items`` lies in 1..64.  Bit-identical to ``score`` on the
+        padded tensors."""
+        if not 1 <= max_items <= 64:
+            raise ValueError(f"max_items must lie in 1..64, got {max_items}")
         lens = lengths.detach().to("cpu", torch.int64).flatten()
         B = lens.numel()
         if B and (int(lens.min()) < 0 or int(lens.max()) > max_items):
@@ -181,6 +185,10 @@ class HostScoringPipeline:
         ids_h = self._pinned("ids", (B, max_items), torch.int32)
         off = packed_layout(lens, plan, max_items, mask_h, ids_h)
         cap_rows = self.chunk * max_items
+        if max_items != self._graph_width:
+            # a new width reallocates the mask / ids / row staging buffers that the captured graphs read
+            self._graphs.clear()
+            self._graph_width = max_items
         cur = torch.cuda.current_stream(self.dev)
         self.copy_stream.wait_stream(cur)
         self.compute_stream.wait_stream(cur)

@@ -72,11 +72,11 @@ def _normalize(x: np.ndarray) -> np.ndarray:
 
 
 def make_modalities(batch: int, dim_per_modality: int = 512, seed: int = 1,
-                    normalized: bool = False) -> tuple[np.ndarray, np.ndarray]:
-    """Raw (un-normalised unless asked) image / text item embeddings, (B,16,dpm) fp32 each."""
+                    normalized: bool = False, max_items: int = MAX_ITEMS) -> tuple[np.ndarray, np.ndarray]:
+    """Raw (un-normalised unless asked) image / text item embeddings, (B,max_items,dpm) fp32 each."""
     g = _rng(seed)
-    img = g.standard_normal((batch, MAX_ITEMS, dim_per_modality), dtype=np.float32)
-    txt = g.standard_normal((batch, MAX_ITEMS, dim_per_modality), dtype=np.float32)
+    img = g.standard_normal((batch, max_items, dim_per_modality), dtype=np.float32)
+    txt = g.standard_normal((batch, max_items, dim_per_modality), dtype=np.float32)
     if normalized:
         img, txt = _normalize(img), _normalize(txt)
     return img, txt
@@ -87,9 +87,9 @@ def make_lengths(batch: int, seed: int = 2, lo: int = 2, hi: int = MAX_ITEMS) ->
     return _rng(seed).integers(lo, hi + 1, size=batch).astype(np.int32)
 
 
-def make_mask(lengths: np.ndarray) -> np.ndarray:
-    """(B,16) bool, True = pad; valid items left-aligned (reference collate contract)."""
-    return np.arange(MAX_ITEMS)[None, :] >= np.asarray(lengths)[:, None]
+def make_mask(lengths: np.ndarray, max_items: int = MAX_ITEMS) -> np.ndarray:
+    """(B,max_items) bool, True = pad; valid items left-aligned (reference collate contract)."""
+    return np.arange(max_items)[None, :] >= np.asarray(lengths)[:, None]
 
 
 def fuse(img: np.ndarray, txt: np.ndarray, method: str) -> np.ndarray:
@@ -107,12 +107,13 @@ def fuse(img: np.ndarray, txt: np.ndarray, method: str) -> np.ndarray:
 
 
 def make_outfits(batch: int, method: str = "concat", dim_per_modality: int = 512,
-                 seed: int = 1, fixed_len: int | None = None):
-    """Fused outfit embeddings + mask as the reference processors would emit them."""
-    img, txt = make_modalities(batch, dim_per_modality, seed)
+                 seed: int = 1, fixed_len: int | None = None, max_items: int = MAX_ITEMS):
+    """Fused outfit embeddings + mask as the reference processors would emit them, padded to
+    ``max_items`` slots with n ~ Uniform{2..max_items} valid items unless ``fixed_len`` is given."""
+    img, txt = make_modalities(batch, dim_per_modality, seed, max_items=max_items)
     lengths = (np.full(batch, fixed_len, np.int32) if fixed_len is not None
-               else make_lengths(batch, seed + 1))
-    mask = make_mask(lengths)
+               else make_lengths(batch, seed + 1, hi=max_items))
+    mask = make_mask(lengths, max_items)
     emb = fuse(img, txt, method)
     emb[mask] = 0.0  # reference pad rows are zeros
     return emb, mask, lengths
