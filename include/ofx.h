@@ -326,6 +326,26 @@ OFX_API int ofx_ffn_block_f16(float* x, int32_t rows, int32_t d_model, int32_t d
                       const void* w2, const float* b2, void* h_next, const float* next_ln_w,
                       const float* next_ln_b, void* workspace, size_t workspace_bytes, void* stream);
 
+/* ---- building block exported for tests / profiling: the masked multi-head self-attention of one encoder layer
+ * (softmax(q.K^T / sqrt(head_dim)) . V per outfit and head, padded slots dropped), launched exactly as
+ * ofx_encoder_forward launches it.
+ * Packed token layout: row b < batch is outfit b's prefix token; its items are rows batch + off[b] ..
+ * batch + off[b+1] - 1, and owner[r] is the outfit of item row r; *n_tok == batch + off[batch].  off (batch + 1),
+ * owner (at least *n_tok) and n_tok are int32 device arrays supplied by the caller.  An outfit attends over its
+ * S = 1 + off[b+1] - off[b] tokens.
+ * Elements are bf16, fp16 or fp32 after `precision` (OFX_PREC_*); 16 heads of d_model / 16 consecutive columns.
+ * q, k, v and out hold rows of pitch ldq, ldk, ldv, ldo elements; out receives every token row, or with
+ * row0_only = 1 (the pruned last layer) only rows 0 .. batch - 1, whose queries are then rows 0 .. batch - 1
+ * of q.  Nothing else of out is written.
+ * Refused before anything is launched: precision not an OFX_PREC_* (OFX_E_ARG); d_model not 512 / 1024 / 1536,
+ * max_items not in 1..64, batch < 0 or above the encoder's bound 2^26 / (max_items + 1) (OFX_E_SHAPE); a null or
+ * not 16-byte aligned pointer, row0_only not 0 / 1, a pitch below d_model or not a multiple of 8 elements for
+ * bf16 / fp16 or of 4 for fp32 (OFX_E_ARG). */
+OFX_API int ofx_attention(int32_t precision, int32_t d_model, int32_t batch, int32_t max_items,
+                          const int32_t* off, const int32_t* owner, const int32_t* n_tok, int32_t row0_only,
+                          const void* q, int64_t ldq, const void* k, int64_t ldk, const void* v, int64_t ldv,
+                          void* out, int64_t ldo, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

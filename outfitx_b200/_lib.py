@@ -114,6 +114,9 @@ _SIGNATURES = {
     "ofx_gemm_f32_tc": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int32, C.c_int32,
                                   C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_int64,
                                   C.c_void_p, C.c_int64, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "ofx_attention": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_int32, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                C.c_void_p, C.c_int64, C.c_void_p]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

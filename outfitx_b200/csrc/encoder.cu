@@ -1,5 +1,5 @@
 // Encoder forward of the outfit-scoring path behind the C ABI:
-//   ofx_pack_weights / ofx_encoder_forward / ofx_fuse / ofx_gemm_bf16 / ofx_gemm_f16.
+//   ofx_pack_weights / ofx_encoder_forward / ofx_fuse / ofx_gemm_bf16 / ofx_gemm_f16 / ofx_attention.
 // Mirrors OutfitX._cp_forward / _cir_forward (/root/reference/src/models/outfit_x.py:120-172)
 // with the exact simplifications of SURVEY.md App. A.4: padded tokens dropped, last layer
 // evaluated for the prefix-token query row only.
@@ -468,5 +468,39 @@ int ofx_ffn_block_f16(float* x, int32_t rows, int32_t d_model, int32_t d_ffn_pad
     fa.h_next = h_next; fa.lnn_w = next_ln_w; fa.lnn_b = next_ln_b;
     fa.workspace = workspace; fa.workspace_bytes = workspace_bytes;
     return ffn_block_f16(fa, static_cast<cudaStream_t>(stream));
+}
+
+int ofx_attention(int32_t precision, int32_t d_model, int32_t batch, int32_t max_items, const int32_t* off,
+                  const int32_t* owner, const int32_t* n_tok, int32_t row0_only, const void* q, int64_t ldq,
+                  const void* k, int64_t ldk, const void* v, int64_t ldv, void* out, int64_t ldo, void* stream) {
+    if (precision != OFX_PREC_BF16 && precision != OFX_PREC_FP32 && precision != OFX_PREC_FP16)
+        return fail(OFX_E_ARG, "ofx_attention: precision %d not in {0 (bf16), 1 (fp32), 2 (fp16)}", precision);
+    if (d_model != 512 && d_model != 1024 && d_model != 1536)
+        return fail(OFX_E_SHAPE, "ofx_attention: d_model %d not in {512,1024,1536}", d_model);
+    if (max_items < 1 || max_items > 64) return fail(OFX_E_SHAPE, "ofx_attention: max_items %d not in [1,64]", max_items);
+    if (batch < 0 || batch > (1 << 26) / (max_items + 1)) return fail(OFX_E_SHAPE, "ofx_attention: batch %d out of range", batch);
+    if (row0_only != 0 && row0_only != 1) return fail(OFX_E_ARG, "ofx_attention: row0_only %d not 0 / 1", row0_only);
+    const void* ptrs[] = {off, owner, n_tok, q, k, v, out};
+    for (const void* p : ptrs)
+        if (!p || reinterpret_cast<uintptr_t>(p) % 16)
+            return fail(OFX_E_ARG, "ofx_attention: null or not 16-byte aligned pointer");
+    // 16-byte rows: 8 elements of bf16 / fp16, 4 of fp32
+    const int64_t unit = precision == OFX_PREC_FP32 ? 4 : 8;
+    const int64_t lds[] = {ldq, ldk, ldv, ldo};
+    for (int64_t ld : lds)
+        if (ld < d_model || ld % unit)
+            return fail(OFX_E_ARG, "ofx_attention: pitch %lld below d_model %d or not a multiple of %lld", (long long)ld,
+                        d_model, (long long)unit);
+    OFX_TRY(require_sm100());
+    AttnArgs at{};
+    at.batch = batch; at.n_head = 16; at.row0_only = row0_only;
+    at.max_s = max_items + 1; at.max_rows = batch * (max_items + 1);
+    at.n_tok = n_tok; at.owner = owner; at.off = off;
+    at.q = q; at.ldq = ldq; at.k = k; at.ldk = ldk; at.v = v; at.ldv = ldv; at.out = out; at.ldo = ldo;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int hd = d_model / 16;
+    if (precision == OFX_PREC_BF16) return attention<__nv_bfloat16>(at, hd, st);
+    if (precision == OFX_PREC_FP16) return attention<__half>(at, hd, st);
+    return attention<float>(at, hd, st);
 }
 }

@@ -1096,41 +1096,44 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     if (a.max_s < 2 || a.max_s > kAttnLongMaxS) return fail(OFX_E_SHAPE, "attention: max_s %d not in [2,%d]", a.max_s, kAttnLongMaxS);
     const bool long_s = a.max_s > kAttnMaxS;     // some outfit may hold more than 16 items
     if constexpr (sizeof(T) == 2) {
-        if ((a.ldq % 8 == 0) && (a.ldk % 8 == 0) && (a.ldv % 8 == 0) && (a.ldo % 8 == 0)) {
-            if (long_s) {
-                switch (head_dim) {
-                    case 32: return launch_attention_mma_long<32, T>(a, stream);
-                    case 64: return launch_attention_mma_long<64, T>(a, stream);
-                    case 96: return launch_attention_mma_long<96, T>(a, stream);
-                    default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
-                }
-            }
+        // the mma kernels move 16-byte chunks of 8 elements: every row must start 16-byte aligned
+        if ((a.ldq % 8) || (a.ldk % 8) || (a.ldv % 8) || (a.ldo % 8))
+            return fail(OFX_E_ARG, "attention: 16-bit pitches must be multiples of 8 (q %lld, k %lld, v %lld, out %lld)",
+                        a.ldq, a.ldk, a.ldv, a.ldo);
+        if (long_s) {
             switch (head_dim) {
-                case 32: return launch_attention_mma<32, T>(a, stream);
-                case 64: return launch_attention_mma<64, T>(a, stream);
-                case 96: return launch_attention_mma<96, T>(a, stream);
+                case 32: return launch_attention_mma_long<32, T>(a, stream);
+                case 64: return launch_attention_mma_long<64, T>(a, stream);
+                case 96: return launch_attention_mma_long<96, T>(a, stream);
                 default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
             }
         }
-    }
-    const int rows = a.row0_only ? a.batch : a.max_rows;
-    const unsigned grid = static_cast<unsigned>((rows + 3) / 4);
-    if (head_dim != 32 && head_dim != 64 && head_dim != 96) return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
-    if (long_s) {
         switch (head_dim) {
-            case 32: attention_kernel<32, T, true><<<grid, 256, 0, stream>>>(a); break;
-            case 64: attention_kernel<64, T, true><<<grid, 256, 0, stream>>>(a); break;
-            case 96: attention_kernel<96, T, true><<<grid, 256, 0, stream>>>(a); break;
+            case 32: return launch_attention_mma<32, T>(a, stream);
+            case 64: return launch_attention_mma<64, T>(a, stream);
+            case 96: return launch_attention_mma<96, T>(a, stream);
+            default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
         }
     } else {
-        switch (head_dim) {
-            case 32: attention_kernel<32, T, false><<<grid, 256, 0, stream>>>(a); break;
-            case 64: attention_kernel<64, T, false><<<grid, 256, 0, stream>>>(a); break;
-            case 96: attention_kernel<96, T, false><<<grid, 256, 0, stream>>>(a); break;
+        const int rows = a.row0_only ? a.batch : a.max_rows;
+        const unsigned grid = static_cast<unsigned>((rows + 3) / 4);
+        if (head_dim != 32 && head_dim != 64 && head_dim != 96) return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
+        if (long_s) {
+            switch (head_dim) {
+                case 32: attention_kernel<32, T, true><<<grid, 256, 0, stream>>>(a); break;
+                case 64: attention_kernel<64, T, true><<<grid, 256, 0, stream>>>(a); break;
+                case 96: attention_kernel<96, T, true><<<grid, 256, 0, stream>>>(a); break;
+            }
+        } else {
+            switch (head_dim) {
+                case 32: attention_kernel<32, T, false><<<grid, 256, 0, stream>>>(a); break;
+                case 64: attention_kernel<64, T, false><<<grid, 256, 0, stream>>>(a); break;
+                case 96: attention_kernel<96, T, false><<<grid, 256, 0, stream>>>(a); break;
+            }
         }
+        OFX_LAUNCH_CHECK();
+        return OFX_OK;
     }
-    OFX_LAUNCH_CHECK();
-    return OFX_OK;
 }
 template int attention<float>(const AttnArgs&, int, cudaStream_t);
 template int attention<__nv_bfloat16>(const AttnArgs&, int, cudaStream_t);
