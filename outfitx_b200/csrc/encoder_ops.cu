@@ -418,6 +418,34 @@ template int cast_rows<__nv_bfloat16>(const float*, long long, __nv_bfloat16*, c
 template int cast_rows<__half>(const float*, long long, __half*, cudaStream_t);
 
 // ------------------------------------------------------------------ attention, CUDA cores
+// This lane's slice of the key (or value) rows j0 .. j0 + 3 of an outfit.  The four row loads are issued back to
+// back, so every thread keeps several independent 16-byte loads in flight; rows past S are clamped to key 0 (a valid,
+// cached address) and masked by the caller.
+template <int NP, class T>
+__device__ __forceinline__ void load_key_group(const T* src, long long ld, int b, int base, int S, int j0,
+                                               float (&t)[4][NP][8]) {
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+        const int j = j0 + u;
+        const long long r = (j == 0 || j >= S) ? b : base + j - 1;
+#pragma unroll
+        for (int p = 0; p < NP; ++p) load8(src + r * ld + 32 * p, t[u][p]);
+    }
+}
+
+// q . k over the head: each of the row's four lanes sums its 8 x NP dims, two xor-shuffles combine the partial sums
+template <int NP>
+__device__ __forceinline__ float dot_4lanes(const float (&q)[NP][8], const float (&k)[NP][8]) {
+    float acc = 0.f;
+#pragma unroll
+    for (int p = 0; p < NP; ++p)
+#pragma unroll
+        for (int e = 0; e < 8; ++e) acc = fmaf(q[p][e], k[p][e], acc);
+    acc += __shfl_xor_sync(0xffffffffu, acc, 1);
+    acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+    return acc;
+}
+
 // One (token row, head) of an outfit with S > 17 tokens: one pass over groups of 4 keys with a running
 // maximum and sum (online softmax); the output accumulator is rescaled whenever the maximum grows.
 template <int HD, class T>
@@ -437,23 +465,11 @@ __device__ __forceinline__ void attention_row_online(const AttnArgs& a, int b, i
 #pragma unroll 1
     for (int j0 = 0; j0 < S; j0 += 4) {
         float t[4][NP][8];
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int j = j0 + u;
-            const long long r = (j == 0 || j >= S) ? b : base + j - 1;
-#pragma unroll
-            for (int p = 0; p < NP; ++p) load8(kp + r * a.ldk + 32 * p, t[u][p]);
-        }
+        load_key_group<NP>(kp, a.ldk, b, base, S, j0, t);
         float sc[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
-            float acc = 0.f;
-#pragma unroll
-            for (int p = 0; p < NP; ++p)
-#pragma unroll
-                for (int e = 0; e < 8; ++e) acc = fmaf(q[p][e], t[u][p][e], acc);
-            acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-            acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+            const float acc = dot_4lanes<NP>(q, t[u]);
             sc[u] = j0 + u < S ? acc * scale : -INFINITY;
         }
         const float m_new = fmaxf(mx, fmaxf(fmaxf(sc[0], sc[1]), fmaxf(sc[2], sc[3])));   // finite: key 0 is valid
@@ -465,13 +481,7 @@ __device__ __forceinline__ void attention_row_online(const AttnArgs& a, int b, i
             sc[u] = sizeof(T) == 4 ? expf(sc[u] - mx) : __expf(sc[u] - mx);
             den += sc[u];
         }
-#pragma unroll
-        for (int u = 0; u < 4; ++u) {
-            const int j = j0 + u;
-            const long long r = (j == 0 || j >= S) ? b : base + j - 1;
-#pragma unroll
-            for (int p = 0; p < NP; ++p) load8(vp + r * a.ldv + 32 * p, t[u][p]);
-        }
+        load_key_group<NP>(vp, a.ldv, b, base, S, j0, t);
 #pragma unroll
         for (int p = 0; p < NP; ++p)
 #pragma unroll
@@ -529,9 +539,7 @@ attention_kernel(AttnArgs a) {
     float q[NP][8];
 #pragma unroll
     for (int p = 0; p < NP; ++p) load8(qp + 32 * p, q[p]);
-    // Keys are taken four at a time: the four row loads of a group are issued back to back
-    // (rows past S are clamped to key 0 -- a valid, cached address -- and masked afterwards), so
-    // every thread keeps several independent 16-byte loads in flight instead of one.
+    // keys are taken four at a time (load_key_group)
     constexpr int kGroups = 5;  // 5 x 4 >= 17
     float sc[kGroups * 4];
     const float scale = rsqrtf(static_cast<float>(HD));
@@ -541,22 +549,10 @@ attention_kernel(AttnArgs a) {
         for (int u = 0; u < 4; ++u) sc[4 * g + u] = -INFINITY;
         if (4 * g < S) {
             float t[4][NP][8];
+            load_key_group<NP>(kp, a.ldk, b, base, S, 4 * g, t);
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
-                const int j = 4 * g + u;
-                const long long r = (j == 0 || j >= S) ? b : base + j - 1;
-#pragma unroll
-                for (int p = 0; p < NP; ++p) load8(kp + r * a.ldk + 32 * p, t[u][p]);
-            }
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                float acc = 0.f;
-#pragma unroll
-                for (int p = 0; p < NP; ++p)
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) acc = fmaf(q[p][e], t[u][p][e], acc);
-                acc += __shfl_xor_sync(0xffffffffu, acc, 1);
-                acc += __shfl_xor_sync(0xffffffffu, acc, 2);
+                const float acc = dot_4lanes<NP>(q, t[u]);
                 if (4 * g + u < S) sc[4 * g + u] = acc * scale;
             }
         }
@@ -586,13 +582,7 @@ attention_kernel(AttnArgs a) {
     for (int g = 0; g < kGroups; ++g) {
         if (4 * g < S) {
             float t[4][NP][8];
-#pragma unroll
-            for (int u = 0; u < 4; ++u) {
-                const int j = 4 * g + u;
-                const long long r = (j == 0 || j >= S) ? b : base + j - 1;
-#pragma unroll
-                for (int p = 0; p < NP; ++p) load8(vp + r * a.ldv + 32 * p, t[u][p]);
-            }
+            load_key_group<NP>(vp, a.ldv, b, base, S, 4 * g, t);
 #pragma unroll
             for (int u = 0; u < 4; ++u) {
                 const float pj = sc[4 * g + u];
@@ -612,7 +602,7 @@ attention_kernel(AttnArgs a) {
 }
 
 // ------------------------------------------------------------------ attention, bf16 / fp16 path
-// One CTA (4 warps) per outfit.  The outfit's q / K / V rows (S <= 17 tokens x d_model) are
+// One CTA (4 warps) per outfit.  The outfit's q / K / V rows (S <= 65 tokens x d_model) are
 // gathered into shared memory once with 16-byte cp.async (row stride d_model + 8 elements, so
 // the ldmatrix row addresses of a fragment fall into distinct banks); every warp then serves 4
 // of the 16 heads with warp-level tensor-core MMAs (mma.sync m16n8k16, bf16 or fp16 in / fp32 out):
@@ -651,24 +641,30 @@ __device__ __forceinline__ float ex2_fast(float x) {
     return y;
 }
 
-constexpr int kAttnMaxS = 17;
+constexpr int kAttnMaxS = 17;       // tokens at up to 16 item slots
+constexpr int kAttnLongMaxS = 65;   // tokens at up to 64 item slots
 
-// BIG = false: this outfit has S <= 16 tokens (one 16-row query tile, one 16-key tile) -- 14 of 15
-// outfits when n ~ U{2..16}; BIG = true adds the second tiles for S = 17.  The kernel picks the
-// body per CTA, so the common case runs straight-line code without per-tile predicates.
+// The kernel picks the body per CTA from the outfit's item count, so the common cases run straight-line code
+// without per-tile predicates:
+//   SMALL (MT = KT = 1): S <= 8 tokens (40 % of the outfits at n ~ U{2..16}): only query rows 0..7 (h = 0) and the
+//     first 8-key n-tile exist, so the second score MMA, half of the softmax and half of the output stores are skipped.
+//   MT = KT = 1: S <= 16 tokens (one 16-row query tile, one 16-key tile) -- 14 of 15 outfits when n ~ U{2..16}.
+//   MT = KT = 2: adds the second tiles for S = 17.
+//   PASSES (MT = 1, KT = 5): S <= 65 tokens.  Each warp walks the up to five 16-row query tiles of its heads one
+//     pass at a time; per pass it scores all 16-key tiles in use into registers (10 n8-tiles) and runs the
+//     softmax over the whole row.  Under row0_only only query tile 0 exists.
 //
 // NSPLIT > 1 splits the 16 heads over NSPLIT CTAs (grid.y): each gathers only its DM / NSPLIT columns
 // (still >= 512 contiguous bytes per row), so a CTA needs 1 / NSPLIT of the shared memory and twice
 // as many CTAs are resident per SM -- the kernel is latency-bound (gather -> compute -> store with no
 // overlap inside a CTA), so residency is what hides the gather.
-// SMALL: S <= 8 tokens (40 % of the outfits at n ~ U{2..16}): only query rows 0..7 (h = 0) and the first
-// 8-key n-tile exist, so the second score MMA, half of the softmax and half of the output stores are skipped.
 // T: the 16-bit type of q / K / V, P and the output (__nv_bfloat16 or __half)
-// cap: rows reserved for each of q, K and V in shared memory (kAttnMaxS, or max_s in the long kernel)
-template <int HD, bool BIG, int NSPLIT, class T, bool SMALL = false>
+// MT, KT: 16-row query tiles per pass, 16-key tiles
+// cap: rows reserved for each of q, K and V in shared memory (kAttnMaxS, or max_s when max_s > 17)
+template <int HD, int NSPLIT, class T, int MT, int KT, bool SMALL, bool PASSES>
 __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* sm, int cap) {
-    static_assert(!(BIG && SMALL), "one or the other");
-    constexpr int MT = BIG ? 2 : 1, KT = BIG ? 2 : 1;
+    static_assert(PASSES ? MT == 1 : MT <= 2 && KT <= 2, "a pass is one query tile; without passes, two at most");
+    static_assert(!SMALL || (MT == 1 && KT == 1), "SMALL is one tile");
     constexpr int NH = SMALL ? 1 : 2;            // row halves (g, g + 8) in use
     constexpr int NNT = SMALL ? 1 : 2 * KT;      // 8-key n-tiles in use
     constexpr int DM = 16 * HD / NSPLIT;     // columns this CTA serves
@@ -683,7 +679,7 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
     const int b = blockIdx.x;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int base = a.batch + a.off[b];
-    const int S = min(1 + (a.off[b + 1] - a.off[b]), kAttnMaxS);
+    const int S = min(1 + (a.off[b + 1] - a.off[b]), PASSES ? cap : kAttnMaxS);
     const int n_q = a.row0_only ? 1 : S;
     const int gcol = NSPLIT > 1 ? static_cast<int>(blockIdx.y) * DM : 0;     // first global column of this CTA
     const T* gq = static_cast<const T*>(a.q) + gcol;
@@ -715,8 +711,9 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
     const uint32_t k_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_k));
     const uint32_t v_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_v));
     const uint32_t z_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_z));
-    const int n_mt = BIG && n_q > 16 ? 2 : 1;     // 16-row query tiles in use
-    const int n_kt = BIG && S > 16 ? 2 : 1;       // 16-key tiles in use
+    const int n_pass = PASSES ? (n_q + 15) / 16 : 1;
+    const int n_mt = MT > 1 && n_q > 16 ? 2 : 1;                              // 16-row query tiles in use per pass
+    const int n_kt = PASSES ? (S + 15) / 16 : KT > 1 && S > 16 ? 2 : 1;      // 16-key tiles in use
     const int g = lane >> 2, t4 = lane & 3;
     // ldmatrix row / column roles of this lane
     const int a_row = (lane & 7) + 8 * ((lane >> 3) & 1), a_col = 8 * (lane >> 4);     // A operand (q) and V^T
@@ -731,302 +728,127 @@ __device__ __forceinline__ void attention_mma_body(const AttnArgs& a, uint8_t* s
 #pragma unroll 1
     for (int hh = 0; hh < HPW; ++hh) {
         const int col0 = (warp * HPW + hh) * HD;   // first (CTA-local) column of this head
-        float sc[MT][2 * KT][4];                          // [query tile][8-key tile][fragment]
-#pragma unroll
-        for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-            for (int nt = 0; nt < 2 * KT; ++nt)
-#pragma unroll
-                for (int e = 0; e < 4; ++e) sc[mt][nt][e] = 0.f;
-#pragma unroll
-        for (int ks = 0; ks < KS; ++ks) {
-            uint32_t qa[MT][4];
-#pragma unroll
-            for (int mt = 0; mt < MT; ++mt) {
-                if (mt < n_mt) {
-                    const int r = mt * 16 + a_row;
-                    ldsm_x4(qa[mt], (r < n_q ? q_s + r * STRIDE : z_s) + (col0 + ks * 16 + a_col) * 2);
-                }
-            }
-#pragma unroll
-            for (int kt = 0; kt < KT; ++kt) {
-                if (kt < n_kt) {
-                    uint32_t kb[4];
-                    const int r = kt * 16 + b_row;
-                    ldsm_x4(kb, (r < S ? k_s + r * STRIDE : z_s) + (col0 + ks * 16 + b_col) * 2);
-#pragma unroll
-                    for (int mt = 0; mt < MT; ++mt) {
-                        if (mt < n_mt) {
-                            mma_16816<T>(sc[mt][2 * kt], qa[mt], kb[0], kb[1]);
-                            if constexpr (!SMALL) mma_16816<T>(sc[mt][2 * kt + 1], qa[mt], kb[2], kb[3]);
-                        }
-                    }
-                }
-            }
-        }
-        // masked softmax over the keys of each query row (rows g and g + 8 of every tile)
-        uint32_t pa[MT][KT][4];      // P as the A operand of P.V: [query tile][16-key tile]
-        float inv[MT][2];
-#pragma unroll
-        for (int mt = 0; mt < MT; ++mt) {
-            if (mt < n_mt) {
-#pragma unroll
-                for (int h = 0; h < NH; ++h) {      // h = 0: row g, h = 1: row g + 8
-                    float mx = -INFINITY;
-#pragma unroll
-                    for (int nt = 0; nt < NNT; ++nt)
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            float v = (kvalid >> (nt * 2 + e)) & 1u ? sc[mt][nt][2 * h + e] * sl2 : -INFINITY;
-                            sc[mt][nt][2 * h + e] = v;
-                            mx = fmaxf(mx, v);
-                        }
-                    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-                    mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-                    float sum = 0.f;
-#pragma unroll
-                    for (int nt = 0; nt < NNT; ++nt)
-#pragma unroll
-                        for (int e = 0; e < 2; ++e) {
-                            const float pz = ex2_fast(sc[mt][nt][2 * h + e] - mx);   // key 0 is always valid: mx finite
-                            sc[mt][nt][2 * h + e] = pz;
-                            sum += pz;
-                        }
-                    sum += __shfl_xor_sync(0xffffffffu, sum, 1);
-                    sum += __shfl_xor_sync(0xffffffffu, sum, 2);
-                    inv[mt][h] = 1.f / sum;
-                }
-#pragma unroll
-                for (int kt = 0; kt < KT; ++kt) {
-                    pa[mt][kt][0] = pack2_16<T>(sc[mt][2 * kt][0], sc[mt][2 * kt][1]);
-                    if constexpr (SMALL) {     // rows 8..15 and keys 8..15 do not exist
-                        pa[mt][kt][1] = pa[mt][kt][2] = pa[mt][kt][3] = 0u;
-                    } else {
-                        pa[mt][kt][1] = pack2_16<T>(sc[mt][2 * kt][2], sc[mt][2 * kt][3]);
-                        pa[mt][kt][2] = pack2_16<T>(sc[mt][2 * kt + 1][0], sc[mt][2 * kt + 1][1]);
-                        pa[mt][kt][3] = pack2_16<T>(sc[mt][2 * kt + 1][2], sc[mt][2 * kt + 1][3]);
-                    }
-                }
-            }
-        }
-        // out = P . V, 16 head dims at a time
-#pragma unroll
-        for (int dp = 0; dp < KS; ++dp) {
-            float o[MT][2][4];
+#pragma unroll 1
+        for (int pass = 0; pass < n_pass; ++pass) {
+            const int row0 = pass * 16 * MT;           // first query row of this pass
+            float sc[MT][2 * KT][4];                          // [query tile][8-key tile][fragment]
 #pragma unroll
             for (int mt = 0; mt < MT; ++mt)
 #pragma unroll
-                for (int x = 0; x < 2; ++x)
+                for (int nt = 0; nt < 2 * KT; ++nt)
 #pragma unroll
-                    for (int e = 0; e < 4; ++e) o[mt][x][e] = 0.f;
-#pragma unroll
-            for (int kt = 0; kt < KT; ++kt) {
-                if (kt < n_kt) {
-                    uint32_t vb[4];
-                    const int r = kt * 16 + a_row;
-                    ldsm_x4_trans(vb, (r < S ? v_s + r * STRIDE : z_s) + (col0 + dp * 16 + a_col) * 2);
-#pragma unroll
-                    for (int mt = 0; mt < MT; ++mt) {
-                        if (mt < n_mt) {
-                            mma_16816<T>(o[mt][0], pa[mt][kt], vb[0], vb[1]);
-                            mma_16816<T>(o[mt][1], pa[mt][kt], vb[2], vb[3]);
-                        }
-                    }
-                }
-            }
-            // the head's slice of the q rows is dead (fragments are in registers): reuse it for the output
-            __syncwarp();
-#pragma unroll
-            for (int mt = 0; mt < MT; ++mt) {
-                if (mt < n_mt) {
-#pragma unroll
-                    for (int h = 0; h < NH; ++h) {
-                        const int r = mt * 16 + g + 8 * h;
-                        if (r < n_q) {
-#pragma unroll
-                            for (int x = 0; x < 2; ++x)
-                                *reinterpret_cast<uint32_t*>(s_q + r * STRIDE + (col0 + dp * 16 + x * 8 + 2 * t4) * 2) =
-                                    pack2_16<T>(o[mt][x][2 * h] * inv[mt][h], o[mt][x][2 * h + 1] * inv[mt][h]);
-                        }
-                    }
-                }
-            }
-        }
-    }
-    __syncthreads();
-    T* go = static_cast<T*>(a.out) + gcol;
-    for (int c = tid; c < n_q * CPR; c += 128) {
-        const int r = c / CPR, cc = c - r * CPR;
-        const long long row = r == 0 ? b : base + r - 1;
-        *reinterpret_cast<uint4*>(go + row * a.ldo + cc * 8) = *reinterpret_cast<const uint4*>(s_q + r * STRIDE + cc * 16);
-    }
-}
-
-template <int HD, int NSPLIT, class T>
-__global__ void __launch_bounds__(128)
-attention_mma_kernel(const AttnArgs a) {
-    extern __shared__ __align__(16) uint8_t attn_sm[];
-    const int b = blockIdx.x;
-    const int n_items = a.off[b + 1] - a.off[b];
-    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm, kAttnMaxS);   // S = 1 + n <= 8
-    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm, kAttnMaxS);         // S <= 16
-    else attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm, kAttnMaxS);
-}
-
-// ------------------------------------------------------------------ attention, bf16 / fp16, outfits of 17..64 items
-// S > 17 tokens (up to 65): the gather-once layout of attention_mma_body with max_s rows per region.  Each warp
-// walks the up to five 16-row query tiles of its heads one at a time; for each it scores all (up to five) 16-key
-// tiles into registers (10 n8-tiles), runs the masked warp-shuffle softmax over the whole row and accumulates
-// P.V through ldmatrix.trans.  Rows >= S read the zero row, so padded keys contribute exactly 0; under row0_only
-// only query tile 0 exists.
-constexpr int kAttnLongMaxS = 65;
-template <int HD, int NSPLIT, class T>
-__device__ __forceinline__ void attention_mma_long_body(const AttnArgs& a, uint8_t* sm, int cap) {
-    constexpr int KT = (kAttnLongMaxS + 15) / 16;   // 16-key tiles
-    constexpr int DM = 16 * HD / NSPLIT;
-    constexpr int HPW = 4 / NSPLIT;
-    constexpr int CPR = DM / 8;
-    constexpr int STRIDE = (DM + 8) * 2;
-    constexpr int KS = HD / 16;
-    uint8_t* s_q = sm;
-    uint8_t* s_k = sm + cap * STRIDE;
-    uint8_t* s_v = s_k + cap * STRIDE;
-    uint8_t* s_z = s_v + cap * STRIDE;
-    const int b = blockIdx.x;
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int base = a.batch + a.off[b];
-    const int S = min(1 + (a.off[b + 1] - a.off[b]), cap);
-    const int n_q = a.row0_only ? 1 : S;
-    const int gcol = static_cast<int>(blockIdx.y) * DM;
-    const T* gq = static_cast<const T*>(a.q) + gcol;
-    const T* gk = static_cast<const T*>(a.k) + gcol;
-    const T* gv = static_cast<const T*>(a.v) + gcol;
-
-    for (int i = tid; i < STRIDE / 16; i += 128) reinterpret_cast<uint4*>(s_z)[i] = make_uint4(0, 0, 0, 0);
-    auto load_rows = [&](const T* g, long long ld, uint8_t* dst, int n_rows) {
-        int j = tid / CPR, cc = tid - j * CPR;
-        while (j < n_rows) {
-            const long long row = j == 0 ? b : base + j - 1;
-            asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(static_cast<uint32_t>(
-                             __cvta_generic_to_shared(dst + j * STRIDE + cc * 16))),
-                         "l"(g + row * ld + cc * 8)
-                         : "memory");
-            cc += 128;
-            while (cc >= CPR) { cc -= CPR; ++j; }
-        }
-    };
-    load_rows(gk, a.ldk, s_k, S);
-    load_rows(gv, a.ldv, s_v, S);
-    load_rows(gq, a.ldq, s_q, n_q);
-    asm volatile("cp.async.commit_group;" ::: "memory");
-    asm volatile("cp.async.wait_group 0;" ::: "memory");
-    __syncthreads();
-
-    const uint32_t q_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_q));
-    const uint32_t k_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_k));
-    const uint32_t v_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_v));
-    const uint32_t z_s = static_cast<uint32_t>(__cvta_generic_to_shared(s_z));
-    const int n_mt = (n_q + 15) / 16;
-    const int n_kt = (S + 15) / 16;
-    const int g = lane >> 2, t4 = lane & 3;
-    const int a_row = (lane & 7) + 8 * ((lane >> 3) & 1), a_col = 8 * (lane >> 4);
-    const int b_row = (lane & 7) + 8 * (lane >> 4), b_col = 8 * ((lane >> 3) & 1);
-    const float sl2 = rsqrtf(static_cast<float>(HD)) * 1.4426950408889634f;
-    uint32_t kvalid = 0;      // bit nt*2+e: key nt*8 + 2*t4 + e exists
-#pragma unroll
-    for (int nt = 0; nt < 2 * KT; ++nt)
-#pragma unroll
-        for (int e = 0; e < 2; ++e) kvalid |= (nt * 8 + 2 * t4 + e < S ? 1u : 0u) << (nt * 2 + e);
-
-#pragma unroll 1
-    for (int hh = 0; hh < HPW; ++hh) {
-        const int col0 = (warp * HPW + hh) * HD;
-#pragma unroll 1
-        for (int mt = 0; mt < n_mt; ++mt) {
-            float sc[2 * KT][4];
-#pragma unroll
-            for (int nt = 0; nt < 2 * KT; ++nt)
-#pragma unroll
-                for (int e = 0; e < 4; ++e) sc[nt][e] = 0.f;
+                    for (int e = 0; e < 4; ++e) sc[mt][nt][e] = 0.f;
 #pragma unroll
             for (int ks = 0; ks < KS; ++ks) {
-                uint32_t qa[4];
-                const int rq = mt * 16 + a_row;
-                ldsm_x4(qa, (rq < n_q ? q_s + rq * STRIDE : z_s) + (col0 + ks * 16 + a_col) * 2);
+                uint32_t qa[MT][4];
+#pragma unroll
+                for (int mt = 0; mt < MT; ++mt) {
+                    if (mt < n_mt) {
+                        const int r = row0 + mt * 16 + a_row;
+                        ldsm_x4(qa[mt], (r < n_q ? q_s + r * STRIDE : z_s) + (col0 + ks * 16 + a_col) * 2);
+                    }
+                }
 #pragma unroll
                 for (int kt = 0; kt < KT; ++kt) {
                     if (kt < n_kt) {
                         uint32_t kb[4];
                         const int r = kt * 16 + b_row;
                         ldsm_x4(kb, (r < S ? k_s + r * STRIDE : z_s) + (col0 + ks * 16 + b_col) * 2);
-                        mma_16816<T>(sc[2 * kt], qa, kb[0], kb[1]);
-                        mma_16816<T>(sc[2 * kt + 1], qa, kb[2], kb[3]);
+#pragma unroll
+                        for (int mt = 0; mt < MT; ++mt) {
+                            if (mt < n_mt) {
+                                mma_16816<T>(sc[mt][2 * kt], qa[mt], kb[0], kb[1]);
+                                if constexpr (!SMALL) mma_16816<T>(sc[mt][2 * kt + 1], qa[mt], kb[2], kb[3]);
+                            }
+                        }
                     }
                 }
             }
-            // masked softmax over the whole row (rows g and g + 8 of the tile)
-            float inv[2];
+            // masked softmax over the keys of each query row (rows g and g + 8 of every tile)
+            uint32_t pa[MT][KT][4];      // P as the A operand of P.V: [query tile][16-key tile]
+            float inv[MT][2];
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                float mx = -INFINITY;
+            for (int mt = 0; mt < MT; ++mt) {
+                if (mt < n_mt) {
 #pragma unroll
-                for (int nt = 0; nt < 2 * KT; ++nt)
+                    for (int h = 0; h < NH; ++h) {      // h = 0: row g, h = 1: row g + 8
+                        float mx = -INFINITY;
 #pragma unroll
-                    for (int e = 0; e < 2; ++e) {
-                        const float v = (kvalid >> (nt * 2 + e)) & 1u ? sc[nt][2 * h + e] * sl2 : -INFINITY;
-                        sc[nt][2 * h + e] = v;
-                        mx = fmaxf(mx, v);
+                        for (int nt = 0; nt < NNT; ++nt)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) {
+                                float v = (kvalid >> (nt * 2 + e)) & 1u ? sc[mt][nt][2 * h + e] * sl2 : -INFINITY;
+                                sc[mt][nt][2 * h + e] = v;
+                                mx = fmaxf(mx, v);
+                            }
+                        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
+                        mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
+                        float sum = 0.f;
+#pragma unroll
+                        for (int nt = 0; nt < NNT; ++nt)
+#pragma unroll
+                            for (int e = 0; e < 2; ++e) {
+                                const float pz = ex2_fast(sc[mt][nt][2 * h + e] - mx);   // key 0 is always valid: mx finite
+                                sc[mt][nt][2 * h + e] = pz;
+                                sum += pz;
+                            }
+                        sum += __shfl_xor_sync(0xffffffffu, sum, 1);
+                        sum += __shfl_xor_sync(0xffffffffu, sum, 2);
+                        inv[mt][h] = 1.f / sum;
                     }
-                mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
-                mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
-                float sum = 0.f;
 #pragma unroll
-                for (int nt = 0; nt < 2 * KT; ++nt)
-#pragma unroll
-                    for (int e = 0; e < 2; ++e) {
-                        const float pz = ex2_fast(sc[nt][2 * h + e] - mx);   // key 0 is always valid: mx finite
-                        sc[nt][2 * h + e] = pz;
-                        sum += pz;
+                    for (int kt = 0; kt < KT; ++kt) {
+                        pa[mt][kt][0] = pack2_16<T>(sc[mt][2 * kt][0], sc[mt][2 * kt][1]);
+                        if constexpr (SMALL) {     // rows 8..15 and keys 8..15 do not exist
+                            pa[mt][kt][1] = pa[mt][kt][2] = pa[mt][kt][3] = 0u;
+                        } else {
+                            pa[mt][kt][1] = pack2_16<T>(sc[mt][2 * kt][2], sc[mt][2 * kt][3]);
+                            pa[mt][kt][2] = pack2_16<T>(sc[mt][2 * kt + 1][0], sc[mt][2 * kt + 1][1]);
+                            pa[mt][kt][3] = pack2_16<T>(sc[mt][2 * kt + 1][2], sc[mt][2 * kt + 1][3]);
+                        }
                     }
-                sum += __shfl_xor_sync(0xffffffffu, sum, 1);
-                sum += __shfl_xor_sync(0xffffffffu, sum, 2);
-                inv[h] = 1.f / sum;
+                }
             }
-            uint32_t pa[KT][4];
-#pragma unroll
-            for (int kt = 0; kt < KT; ++kt) {
-                pa[kt][0] = pack2_16<T>(sc[2 * kt][0], sc[2 * kt][1]);
-                pa[kt][1] = pack2_16<T>(sc[2 * kt][2], sc[2 * kt][3]);
-                pa[kt][2] = pack2_16<T>(sc[2 * kt + 1][0], sc[2 * kt + 1][1]);
-                pa[kt][3] = pack2_16<T>(sc[2 * kt + 1][2], sc[2 * kt + 1][3]);
-            }
-            // out = P . V, 16 head dims at a time, into this tile's (dead) q rows of the head
+            // out = P . V, 16 head dims at a time
 #pragma unroll
             for (int dp = 0; dp < KS; ++dp) {
-                float o[2][4];
+                float o[MT][2][4];
 #pragma unroll
-                for (int x = 0; x < 2; ++x)
+                for (int mt = 0; mt < MT; ++mt)
 #pragma unroll
-                    for (int e = 0; e < 4; ++e) o[x][e] = 0.f;
+                    for (int x = 0; x < 2; ++x)
+#pragma unroll
+                        for (int e = 0; e < 4; ++e) o[mt][x][e] = 0.f;
 #pragma unroll
                 for (int kt = 0; kt < KT; ++kt) {
                     if (kt < n_kt) {
                         uint32_t vb[4];
                         const int r = kt * 16 + a_row;
                         ldsm_x4_trans(vb, (r < S ? v_s + r * STRIDE : z_s) + (col0 + dp * 16 + a_col) * 2);
-                        mma_16816<T>(o[0], pa[kt], vb[0], vb[1]);
-                        mma_16816<T>(o[1], pa[kt], vb[2], vb[3]);
+#pragma unroll
+                        for (int mt = 0; mt < MT; ++mt) {
+                            if (mt < n_mt) {
+                                mma_16816<T>(o[mt][0], pa[mt][kt], vb[0], vb[1]);
+                                mma_16816<T>(o[mt][1], pa[mt][kt], vb[2], vb[3]);
+                            }
+                        }
                     }
                 }
+                // the head's slice of the pass's q rows is dead (fragments are in registers): reuse it for the output
                 __syncwarp();
 #pragma unroll
-                for (int h = 0; h < 2; ++h) {
-                    const int r = mt * 16 + g + 8 * h;
-                    if (r < n_q) {
+                for (int mt = 0; mt < MT; ++mt) {
+                    if (mt < n_mt) {
 #pragma unroll
-                        for (int x = 0; x < 2; ++x)
-                            *reinterpret_cast<uint32_t*>(s_q + r * STRIDE + (col0 + dp * 16 + x * 8 + 2 * t4) * 2) =
-                                pack2_16<T>(o[x][2 * h] * inv[h], o[x][2 * h + 1] * inv[h]);
+                        for (int h = 0; h < NH; ++h) {
+                            const int r = row0 + mt * 16 + g + 8 * h;
+                            if (r < n_q) {
+#pragma unroll
+                                for (int x = 0; x < 2; ++x)
+                                    *reinterpret_cast<uint32_t*>(s_q + r * STRIDE + (col0 + dp * 16 + x * 8 + 2 * t4) * 2) =
+                                        pack2_16<T>(o[mt][x][2 * h] * inv[mt][h], o[mt][x][2 * h + 1] * inv[mt][h]);
+                            }
+                        }
                     }
                 }
             }
@@ -1041,52 +863,54 @@ __device__ __forceinline__ void attention_mma_long_body(const AttnArgs& a, uint8
     }
 }
 
-// max_s > 17: outfits of <= 16 items take the bodies of attention_mma_kernel (same arithmetic, rows at max_s
-// spacing), longer ones the long body
-template <int HD, int NSPLIT, class T>
+// LONG (max_s > 17): shared-memory rows are max_s apart, and outfits of more than 16 items take the PASSES body
+template <int HD, int NSPLIT, class T, bool LONG>
 __global__ void __launch_bounds__(128)
-attention_mma_long_kernel(const AttnArgs a) {
+attention_mma_kernel(const AttnArgs a) {
     extern __shared__ __align__(16) uint8_t attn_sm[];
+    const int cap = LONG ? a.max_s : kAttnMaxS;
     const int b = blockIdx.x;
     const int n_items = a.off[b + 1] - a.off[b];
-    if (n_items < 8) attention_mma_body<HD, false, NSPLIT, T, true>(a, attn_sm, a.max_s);
-    else if (n_items < 16) attention_mma_body<HD, false, NSPLIT, T>(a, attn_sm, a.max_s);
-    else if (n_items == 16) attention_mma_body<HD, true, NSPLIT, T>(a, attn_sm, a.max_s);
-    else attention_mma_long_body<HD, NSPLIT, T>(a, attn_sm, a.max_s);
+    if (n_items < 8) attention_mma_body<HD, NSPLIT, T, 1, 1, true, false>(a, attn_sm, cap);            // S = 1 + n <= 8
+    else if (n_items < 16) attention_mma_body<HD, NSPLIT, T, 1, 1, false, false>(a, attn_sm, cap);     // S <= 16
+    else if (!LONG || n_items == 16) attention_mma_body<HD, NSPLIT, T, 2, 2, false, false>(a, attn_sm, cap);
+    else attention_mma_body<HD, NSPLIT, T, 1, (kAttnLongMaxS + 15) / 16, false, true>(a, attn_sm, cap);
 }
 
-// Shared memory is (3 max_s + 1) rows of (16 HD / NSPLIT + 8) x 2 bytes: at max_s = 65 the head split that keeps
-// two CTAs per SM is 2 at head_dim 32 (103 KB) and 4 at 64 (103 KB); at 96 a split of 4 (154 KB) is the least
-// that fits at all (2 needs 304 KB).
+// Shared memory is (3 cap + 1) rows of (16 HD / NSPLIT + 8) x 2 bytes.  The 16 heads of an outfit split over NSPLIT
+// CTAs: 2 with max_s <= 17; at max_s = 65 the split that keeps two CTAs per SM is 2 at head_dim 32 (103 KB) and 4 at
+// 64 (103 KB); at 96 a split of 4 (154 KB) is the least that fits at all (2 needs 304 KB).
 template <int HD> constexpr int attn_long_split() { return HD == 32 ? 2 : 4; }
-template <int HD>
-constexpr int attn_long_smem(int max_s) { return (3 * max_s + 1) * (16 * HD / attn_long_split<HD>() + 8) * 2; }
+template <int HD, int NSPLIT> constexpr int attn_mma_smem(int cap) { return (3 * cap + 1) * (16 * HD / NSPLIT + 8) * 2; }
 
-template <int HD, class T>
-static int launch_attention_mma_long(const AttnArgs& a, cudaStream_t stream) {
-    constexpr int kSplit = attn_long_split<HD>();
+template <int HD, class T, bool LONG>
+static int launch_attention_mma(const AttnArgs& a, cudaStream_t stream) {
+    constexpr int kSplit = LONG ? attn_long_split<HD>() : 2;
+    constexpr int kMaxCap = LONG ? kAttnLongMaxS : kAttnMaxS;
+    const int cap = LONG ? a.max_s : kAttnMaxS;
     static DeviceOnce configured;
     if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(attention_mma_long_kernel<HD, kSplit, T>,
-                                      cudaFuncAttributeMaxDynamicSharedMemorySize, attn_long_smem<HD>(kAttnLongMaxS)));
+        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, kSplit, T, LONG>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      attn_mma_smem<HD, kSplit>(kMaxCap)));
     }
-    attention_mma_long_kernel<HD, kSplit, T><<<dim3(a.batch, kSplit), 128, attn_long_smem<HD>(a.max_s), stream>>>(a);
+    attention_mma_kernel<HD, kSplit, T, LONG><<<dim3(a.batch, kSplit), 128, attn_mma_smem<HD, kSplit>(cap), stream>>>(a);
     OFX_LAUNCH_CHECK();
     return OFX_OK;
 }
 
-// the 16 heads of an outfit split over two CTAs
 template <int HD, class T>
-static int launch_attention_mma(const AttnArgs& a, cudaStream_t stream) {
-    constexpr int kSplit = 2;
-    constexpr int smem = (3 * kAttnMaxS + 1) * (16 * HD / kSplit + 8) * 2;
-    static DeviceOnce configured;
-    if (configured.need()) {
-        OFX_CUDA(cudaFuncSetAttribute(attention_mma_kernel<HD, kSplit, T>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+static int launch_attention(const AttnArgs& a, cudaStream_t stream) {
+    const bool long_s = a.max_s > kAttnMaxS;     // some outfit may hold more than 16 items
+    if constexpr (sizeof(T) == 2) {
+        return long_s ? launch_attention_mma<HD, T, true>(a, stream) : launch_attention_mma<HD, T, false>(a, stream);
+    } else {
+        const int rows = a.row0_only ? a.batch : a.max_rows;
+        const unsigned grid = static_cast<unsigned>((rows + 3) / 4);
+        if (long_s) attention_kernel<HD, T, true><<<grid, 256, 0, stream>>>(a);
+        else attention_kernel<HD, T, false><<<grid, 256, 0, stream>>>(a);
+        OFX_LAUNCH_CHECK();
+        return OFX_OK;
     }
-    attention_mma_kernel<HD, kSplit, T><<<dim3(a.batch, kSplit), 128, smem, stream>>>(a);
-    OFX_LAUNCH_CHECK();
-    return OFX_OK;
 }
 
 template <class T>
@@ -1094,45 +918,15 @@ int attention(const AttnArgs& a, int head_dim, cudaStream_t stream) {
     if (a.batch <= 0) return OFX_OK;
     if (a.n_head != 16) return fail(OFX_E_SHAPE, "attention: n_head %d != 16", a.n_head);
     if (a.max_s < 2 || a.max_s > kAttnLongMaxS) return fail(OFX_E_SHAPE, "attention: max_s %d not in [2,%d]", a.max_s, kAttnLongMaxS);
-    const bool long_s = a.max_s > kAttnMaxS;     // some outfit may hold more than 16 items
-    if constexpr (sizeof(T) == 2) {
-        // the mma kernels move 16-byte chunks of 8 elements: every row must start 16-byte aligned
-        if ((a.ldq % 8) || (a.ldk % 8) || (a.ldv % 8) || (a.ldo % 8))
-            return fail(OFX_E_ARG, "attention: 16-bit pitches must be multiples of 8 (q %lld, k %lld, v %lld, out %lld)",
-                        a.ldq, a.ldk, a.ldv, a.ldo);
-        if (long_s) {
-            switch (head_dim) {
-                case 32: return launch_attention_mma_long<32, T>(a, stream);
-                case 64: return launch_attention_mma_long<64, T>(a, stream);
-                case 96: return launch_attention_mma_long<96, T>(a, stream);
-                default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
-            }
-        }
-        switch (head_dim) {
-            case 32: return launch_attention_mma<32, T>(a, stream);
-            case 64: return launch_attention_mma<64, T>(a, stream);
-            case 96: return launch_attention_mma<96, T>(a, stream);
-            default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
-        }
-    } else {
-        const int rows = a.row0_only ? a.batch : a.max_rows;
-        const unsigned grid = static_cast<unsigned>((rows + 3) / 4);
-        if (head_dim != 32 && head_dim != 64 && head_dim != 96) return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
-        if (long_s) {
-            switch (head_dim) {
-                case 32: attention_kernel<32, T, true><<<grid, 256, 0, stream>>>(a); break;
-                case 64: attention_kernel<64, T, true><<<grid, 256, 0, stream>>>(a); break;
-                case 96: attention_kernel<96, T, true><<<grid, 256, 0, stream>>>(a); break;
-            }
-        } else {
-            switch (head_dim) {
-                case 32: attention_kernel<32, T, false><<<grid, 256, 0, stream>>>(a); break;
-                case 64: attention_kernel<64, T, false><<<grid, 256, 0, stream>>>(a); break;
-                case 96: attention_kernel<96, T, false><<<grid, 256, 0, stream>>>(a); break;
-            }
-        }
-        OFX_LAUNCH_CHECK();
-        return OFX_OK;
+    // the mma kernels move 16-byte chunks of 8 elements: every row must start 16-byte aligned
+    if (sizeof(T) == 2 && ((a.ldq % 8) || (a.ldk % 8) || (a.ldv % 8) || (a.ldo % 8)))
+        return fail(OFX_E_ARG, "attention: 16-bit pitches must be multiples of 8 (q %lld, k %lld, v %lld, out %lld)",
+                    a.ldq, a.ldk, a.ldv, a.ldo);
+    switch (head_dim) {
+        case 32: return launch_attention<32, T>(a, stream);
+        case 64: return launch_attention<64, T>(a, stream);
+        case 96: return launch_attention<96, T>(a, stream);
+        default: return fail(OFX_E_SHAPE, "head_dim %d not in {32,64,96}", head_dim);
     }
 }
 template int attention<float>(const AttnArgs&, int, cudaStream_t);

@@ -1,7 +1,7 @@
 """GPU: the encoder's attention kernels (ofx_attention) against a plain fp64 reference (tests/attention_ref.py) at
 every precision, head size (d_model 512 / 1024 / 1536 = head_dim 32 / 64 / 96), outfit length, query set (all tokens,
 or the prefix rows of the pruned last layer) and both encoder layouts.  bf16 / fp16 run attention_mma_kernel
-(max_items <= 16) or attention_mma_long_kernel; fp32 runs the CUDA-core attention_kernel.
+(with LONG = true when max_items > 16); fp32 runs the CUDA-core attention_kernel.
 
 Exact routing tests hold a kernel to the bit (or one unit in the last place), so a wrong row, head, tile or key mask
 fails however small its effect on the result:
